@@ -14,7 +14,8 @@ unsharded single-GPU time measured in the same run.  `e2e` is the same metric th
 buffers: mesh upload (H2D) + trace! + segmentize! + download of every Segment record (D2H).  `parity`
 compares the GPU's segments of sampled uid blocks with the CPU oracle, bit for bit, in the same run.
 `--impl reference` times the reference's CPU algorithm (the oracle port: Julia is not installable here) on
-all host cores over a bounded uid sample of the same workload.
+all host cores over a bounded uid sample of the same workload.  `--dump-outputs DIR` writes what the last timed step
+computed as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -28,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 
 # segmentize!(tg; rtol): with the default rtol = sqrt(eps) the reference's own length check (src/track.jl:171-175) throws on 88
 # corner tracks of cfg3 (it drops a 2e-8 chord); 1e-6 -- the remedy its error message suggests -- lets every track complete.
@@ -161,6 +163,32 @@ class Compare:
         return {"checked_tracks": int(self.tracks), "checked_segments": int(self.segments), "mismatches": int(self.mismatches),
                 "ok": bool(self.mismatches == 0 and self.segments > 0), "first_mismatch": self.first,
                 "what": "GPU vs CPU oracle on sampled uid blocks: per-track counts and status, element ids and order, p/q/len bit for bit"}
+
+
+DUMP_CAP = 1 << 19  # elements per stored array: 13 arrays at most, 52 MiB in all
+
+
+def dump_outputs(tg, out_dir, suffix=""):
+    """What the last segmentize! handed its caller, as float64 .npy files in out_dir: the Segment columns of the resident batch
+    (px, py, qx, qy, len, element), segment_offsets, segment_status and the normalised volumes.  Every group is stored at the
+    positions <group>_index.npy names (segment positions count from the shard's first segment): all of them, or a sample of
+    DUMP_CAP positions seeded by nothing but the group's length when it is longer.  The volumes are summed with atomics: their
+    last bits differ from run to run, everything else is reproduced bit for bit."""
+    from raytracing_jl_b200 import _lib
+
+    # the step left the normalised volumes on the device (fetch_volumes=False): copy them, nothing is recomputed
+    _lib.check(tg._ctx, _lib.lib().rt_volumes(tg._ctx, _lib.ptr(tg.volumes)))
+    seg = tg.fetch_segments()
+    groups = [("segment", {k: seg[k] for k in SEG_KEYS}, tg.resident_batch()[2]),
+              ("segment_offsets", {"segment_offsets": tg.segment_offsets}, 0),
+              ("segment_status", {"segment_status": tg.segment_status}, 0), ("volumes", {"volumes": tg.volumes}, 0)]
+    os.makedirs(out_dir, exist_ok=True)
+    for group, cols, base in groups:
+        n = len(next(iter(cols.values())))
+        idx = np.arange(n) if n <= DUMP_CAP else np.unique(np.random.default_rng(n).integers(0, n, DUMP_CAP))
+        np.save(os.path.join(out_dir, f"{group}_index{suffix}.npy"), (idx + base).astype(np.float64))
+        for k, a in cols.items():
+            np.save(os.path.join(out_dir, f"{k}{suffix}.npy"), np.asarray(a)[idx].astype(np.float64))
 
 
 def estimate_segments(model, mesh, n_azim, delta):
@@ -325,6 +353,8 @@ def main():
     ap.add_argument("--clock-period-ms", type=float, default=20.0)
     ap.add_argument("--strong", action="store_true", help="N > 1: shard the named workload itself (fixed total work) instead of delta / N")
     ap.add_argument("--pipeline", type=int, default=None, help="rt_set_option('pipeline'): 0 hybrid, 1 sequential, 3 single-walk")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; one set per rank when N > 1)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
@@ -350,7 +380,6 @@ def main():
 
         bind_to_gpu_numa(local)  # pinned result buffers next to this rank's GPU: N downloads do not share one socket's memory
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    rt.build()
     model, n_azim, delta = load_workload(args.workload, world, args.strong)
     mesh = rt.Mesh(model)
     bcs = rt.BoundaryConditions(top=rt.Reflective, bottom=rt.Reflective, right=rt.Reflective, left=rt.Reflective)
@@ -396,6 +425,8 @@ def main():
     nseg_local = tg.n_segments
     st = tg.stats()
     tg.segment_offsets  # (also fetches tg.segment_status)
+    if args.dump_outputs:
+        dump_outputs(tg, args.dump_outputs, f"_rank{rank}" if world > 1 else "")
     if world > 1:
         print(f"[rank {rank}] ms/step {ms / args.steps:.3f} segments {nseg_local} phases "
               f"{ {k: round(float(np.mean([p[k] for p in phases])), 3) for k in phases[0]} }", file=sys.stderr)

@@ -86,13 +86,48 @@ def test_plot_views_match_the_recipes():
     assert np.array_equal(fx[[0, 1, 3, 4]], [0, 1, 1, 2]) and np.isnan(fx[2]) and fx.size == 5 and np.array_equal(fz[[0, 1, 3, 4]], [7, 7, 9, 9])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/demo"), reason="the reference tree only exists in the build container")
-def test_mesh_readers_on_the_reference_files():
-    """Both mesh files the reference ships for its quick start (demo/pincell.json: Gridap JSON, loaded by test/runtests.jl:5-6;
-    demo/pincell.msh: MSH 4.1) read into the same model, which is the committed fixture tests/golden/pincell.npz."""
+def _write_gridap_json(path, xy, ptrs, data):
+    import json
+
+    with open(path, "w") as fh:
+        json.dump({"grid": {"Dp": 2, "node_coordinates": xy.tolist(), "cell_node_ids": {"ptrs": ptrs.tolist(), "data": data.tolist()}}}, fh)
+
+
+def _write_msh41(path, xy, tri0, seed=7):
+    """MSH 4.1 ASCII laid out the way Gmsh writes a 2-D mesh: node blocks per geometric entity in no particular tag order, tags
+    with gaps, a node no triangle uses, point and line elements before the triangles, triangle nodes not in ascending order."""
+    rng = np.random.default_rng(seed)
+    tags = 2 * np.arange(xy.shape[0] + 1) + 2
+    coords = np.vstack([xy, [[0.123, 0.456]]])  # the last node is referenced by the point element only
+    tags[-1] = 1
+    blocks = np.array_split(rng.permutation(coords.shape[0]), 3)
+    out = ["$MeshFormat", "4.1 0 8", "$EndMeshFormat", "$Nodes", f"{len(blocks)} {coords.shape[0]} 1 {tags.max()}"]
+    for dim, b in enumerate(blocks):
+        out.append(f"{dim} {dim + 1} 0 {b.size}")
+        out += [str(tags[i]) for i in b] + [f"{float(coords[i, 0])!r} {float(coords[i, 1])!r} 0" for i in b]
+    out.append("$EndNodes")
+    rot = np.roll(tags[tri0], 1, axis=1)
+    halves = np.array_split(np.arange(rot.shape[0]), 2)
+    out += ["$Elements", f"{2 + len(halves)} {1 + 2 + rot.shape[0]} 1 {3 + rot.shape[0]}", "0 1 15 1", f"1 {tags[-1]}",
+            "1 1 1 2", f"2 {tags[tri0[0, 0]]} {tags[tri0[0, 1]]}", f"3 {tags[tri0[1, 0]]} {tags[tri0[1, 1]]}"]
+    for s, h in enumerate(halves):
+        out.append(f"2 {s + 1} 2 {h.size}")
+        out += [f"{4 + e} {a} {b} {c}" for e, (a, b, c) in zip(h, rot[h])]
+    out.append("$EndElements")
+    with open(path, "w") as fh:
+        fh.write("\n".join(out) + "\n")
+
+
+def test_mesh_readers_on_the_reference_files(tmp_path):
+    """The readers for the two formats the reference ships its quick-start mesh in (demo/pincell.json: Gridap JSON, loaded by
+    test/runtests.jl:5-6; demo/pincell.msh: MSH 4.1) give back the committed fixture tests/golden/pincell.npz, which was read
+    from those files.  The reference's files are not part of this repository: the fixture is written in both formats here."""
     import raytracing_jl_b200 as rt
 
     d = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pincell.npz"))
-    for m in (rt.DiscreteModelFromFile("/root/reference/demo/pincell.json"), rt.GmshDiscreteModel("/root/reference/demo/pincell.msh")):
-        assert np.array_equal(m.node_coordinates, d["node_coordinates"])
-        assert np.array_equal(m.cell_ptrs, d["cell_ptrs"]) and np.array_equal(m.cell_data, d["cell_data"])
+    xy, ptrs, data = d["node_coordinates"], d["cell_ptrs"], d["cell_data"]
+    _write_gridap_json(tmp_path / "pincell.json", xy, ptrs, data)
+    _write_msh41(tmp_path / "pincell.msh", xy, data.reshape(-1, 3).astype(np.int64) - 1)
+    for m in (rt.DiscreteModelFromFile(str(tmp_path / "pincell.json")), rt.GmshDiscreteModel(str(tmp_path / "pincell.msh"))):
+        assert np.array_equal(m.node_coordinates, xy)
+        assert np.array_equal(m.cell_ptrs, ptrs) and np.array_equal(m.cell_data, data)
