@@ -248,7 +248,7 @@ int rt_selftest_division(rt_ctx *ctx, int64_t n_threads, uint64_t seed, int32_t 
  * "pipeline" (3: ONE sign-test walk that counts and records every chunk + one lane per segment [default]; 0: sign-test count
  * walk + geometric fill walk; 1: sequential geometric walks only.  0 and 3 verify themselves and restart in mode 1 on any
  * disagreement; 3 restarts in mode 0 when its record
- * pool runs out), "march" (0: k_topo<2> instead of k_march in pipeline 3), "band_chunks" (0: uniform chunks also where a track
+ * pool runs out), "band_chunks" (0: uniform chunks also where a track
  * runs along the bounding box), "band_min" / "band_div" (a head or tail of a track that stays inside the boundary band for more
  * than band_min regular chunk lengths [0.0625] is cut into chunks band_div times shorter than the regular ones [8]), "pool_slots" / "pool_extra" (test hooks: chunk slots per count batch, spare record blocks),
  * "debug_verify_fail", "debug_clear_pool" (test hooks), "plan_cache" (0: rebuild the chunk plan in every call), "optimistic" (0: always read

@@ -1,10 +1,10 @@
 // march.cuh -- k_march: the count+record walk of the single-walk pipeline with a REGISTER-RESIDENT hot loop.
 //
-// Same walk, same decisions and same records as k_topo<2> (topo.cuh; the sign-test transitions of the half-edge graph with the
-// literal walk of the reference, src/track.jl:106-178, for everything the clearance test does not cover).  What differs is how
-// the code is laid out for the register allocator: in k_topo the literal path (point location, intersections(), 100+ live
-// values) is inlined next to the fast transition, ptxas runs out of the 64 registers that 8 resident blocks allow and keeps the
-// walker's state in local memory -- 17 local loads/stores per fast transition (profiles/r1_q).  Here
+// Same walk and same decisions as k_topo, the count walk of the hybrid pipeline (topo.cuh; the sign-test transitions of the
+// half-edge graph with the literal walk of the reference, src/track.jl:106-178, for everything the clearance test does not
+// cover), plus one record per accepted cell.  What differs is how the code is laid out for the register allocator: in k_topo
+// the literal path (point location, intersections(), 100+ live values) is inlined next to the fast transition, ptxas runs out
+// of the 64 registers that 8 resident blocks allow and keeps the walker's state in local memory -- 17 local loads/stores per fast transition (profiles/r1_q).  Here
 //   * the hot loop touches only scalars that fit the register file: track line (a, b, c, g), signed distances of the entry
 //     edge's end points (s1, s2), the encoded half-edge to enter next, clearances, counters;
 //   * everything the slow path needs beyond that lives in a MarchState record whose address is passed to ONE out-of-line

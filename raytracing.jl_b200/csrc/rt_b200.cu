@@ -124,8 +124,6 @@ struct rt_ctx {
     bool skip_optimistic_once = false;
     int optimistic_cancels = 0;        // calls whose optimistic evaluation the device-side guard cancelled (info)
     unsigned long long fit_gen = ~0ULL;  // trace generation whose previous call fitted the Segment columns and the pool in ONE batch
-    bool deferred_total = false;
-    bool redo_careful = false;         // the repeat asked for by the optimistic path (not a failed verification)
 
     int opt_band_chunks = 1;           // shorter chunks for tracks that run along the bounding box (walk.cuh k_plan_chunks)
     // ... when that stretch is longer than opt_band_min regular chunks, into chunks opt_band_div times shorter.  Both are relative to
@@ -135,13 +133,11 @@ struct rt_ctx {
     // (profiles/r2_chunk_band.txt: walk phase 0.70 -> 0.62 ms)
     double opt_band_min = 0.0625;
     double opt_band_div = 8.0;
-    int opt_march = 1;                 // single-walk pipeline: k_march (register-resident loop) instead of k_topo<2>
     long long opt_pool_slots = 0;      // test hook: at most this many chunk slots per count batch (0: as many as fit)
     double opt_pool_extra = 1.25;      // spare pool blocks, as a multiple of (expected segments / kRecBlock)
     int opt_pipeline = 3;              // 3: single walk (k_march counts AND records, k_eval3 evaluates) [default]; 0: hybrid (sign-test count walk +
                                        // geometric fill walk), 1: sequential (walk.cuh only); 3 falls back to 0 (pool exhausted) or 1, 0 falls back to 1
     int verify_fallbacks = 0;
-    int fallback_mode = 1;             // pipeline to repeat the call with after a failed verification
     int opt_debug_verify_fail = 0;     // test hook: make the verification of the two-stage pipeline fail
     double tau_ms = 0.0;
     cudaEvent_t ev2[2] = {nullptr, nullptr};
@@ -839,27 +835,238 @@ static double lmin_of(const DevMesh &m, double tiny_step) {
     return fmax(8.0 * tiny_step, kRtol * nb * (1.0 + 1e-6) + 1e-300);
 }
 
-// ---- single-walk pipeline (mode 3): k_topo<2> counts AND records every chunk in one walk, k_eval3 evaluates the records -------
+// ---- one attempt of rt_segmentize ----------------------------------------------------------------------------------------------
+// What rt_segmentize does after an attempt
+enum class Next {
+    Done,
+    RepeatCareful,  // the optimistic evaluation was cancelled on the device: the same pipeline, sized from the walk's result
+    Sequential,     // count and fill disagreed / a geometric fast-path condition failed: fall back to mode 1
+    Hybrid,         // the single walk's record pool ran out: fall back to mode 0
+};
+
+// One execution of a pipeline: its inputs, and what its driver leaves to the common tail of segmentize_attempt
+struct Attempt {
+    double rtol;
+    bool want_vol;
+    rt_batch_cb cb;
+    void *cb_user;
+    int index;                    // rt_batch::attempt
+    Next next = Next::Done;
+    double launches = 0;          // kernel launches (stats[0] when this attempt is the final one)
+    bool first_bad_scan = false;  // k_first_bad finds the first failing track (the single walk's k_track_status reports it itself)
+    bool defer_verify = false;    // the verification flag arrives with the final control read-back
+    bool defer_total = false;     // ... and so do the segment total and the guard of the optimistic evaluation
+};
+
+static double crossings_per_length(const rt_ctx *ctx) { return ctx->edge_sum / (kPi * ctx->area); }
+
+static void set_resident(rt_ctx *ctx, long long trk_begin, long long trk_end, long long off_base, long long nseg) {
+    ctx->res_trk_begin = trk_begin;
+    ctx->res_trk_end = trk_end;
+    ctx->res_off_base = off_base;
+    ctx->res_nseg = nseg;
+}
+
+// the Segment columns the fill / evaluation writes
+static void bind_columns(const rt_ctx *ctx, WalkParams &P) {
+    P.opx = ctx->s_px;
+    P.opy = ctx->s_py;
+    P.oqx = ctx->s_qx;
+    P.oqy = ctx->s_qy;
+    P.olen = ctx->s_len;
+    P.oelem = ctx->s_elem;
+}
+
+// Segment columns sized from free memory (0.92 x free / 44 bytes per segment, counting the columns held now) for `want` segments
+// (already limited by the capacity option): one batch takes what it needs if that fits, a walk in several batches everything that
+// fits.  *cap: the capacity to cut the batches with.
+static int size_columns(rt_ctx *ctx, long long want, bool take_all, size_t free_b, long long *cap) {
+    const long long fit = (long long)((double)(free_b + ctx->b_seg_d.bytes + ctx->b_seg_e.bytes) * 0.92 / 44.0);
+    *cap = take_all ? fit : std::min(want, fit);
+    if (ctx->cap_cfg > 0) *cap = std::min(*cap, (long long)ctx->cap_cfg);
+    return ensure_segment_buffers(ctx, *cap);
+}
+
+// The next batch of tracks, from track b on, whose segments fit `cap` (h_off: host copy of the offsets of the tracks from b0 on):
+// P takes its tracks, its offset base and the warp units of the 32-track blocks overlapping it, in identity order.
+static int cut_batch(rt_ctx *ctx, WalkParams &P, const std::vector<long long> &h_off, long long b0,
+                     const std::vector<long long> &h_unit_base, long long b, long long cap, long long *nseg) {
+    const long long lim = h_off[(size_t)(b - b0)] + cap;  // largest e with off[e] - off[b] <= cap
+    const long long e = b0 + (long long)(std::upper_bound(h_off.begin() + (b - b0), h_off.end(), lim) - h_off.begin()) - 1;
+    if (e <= b) return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: one track needs more than the segment capacity");
+    P.trk_begin = b;
+    P.trk_end = e;
+    P.offset_base = h_off[(size_t)(b - b0)];
+    P.ch.order = nullptr;
+    P.unit_begin = h_unit_base[(size_t)(b >> 5)];
+    P.unit_end = h_unit_base[(size_t)((e - 1) >> 5) + 1];
+    *nseg = h_off[(size_t)(e - b0)] - P.offset_base;
+    return RT_OK;
+}
+
+// the reference's length check (src/track.jl:171-175) of the batch P describes, on the segment lengths it accumulated
+static void launch_track_status(rt_ctx *ctx, const WalkParams &P, double rtol, const int *cancel, unsigned long long *bad) {
+    if (P.trk_end <= P.trk_begin) return;
+    EvalParams E{};
+    E.t = ctx->t;
+    E.offsets = P.offsets;
+    E.trk_begin = P.trk_begin;
+    E.trk_end = P.trk_end;
+    E.offset_base = P.offset_base;
+    E.olen = P.olen;
+    E.status = P.status;
+    E.tsum = P.tsum;
+    E.rtol = rtol;
+    E.cancel = cancel;
+    E.bad = bad;
+    k_track_status<<<blocks_for(P.trk_end - P.trk_begin, 128), 128, 0, ctx->stream>>>(E);
+}
+
+// waits for the batch and reads its verification flag
+static int read_verify(rt_ctx *ctx, bool *failed) {
+    ctx->h_pin[2] = 0;
+    CK(cudaMemcpyAsync(&ctx->h_pin[2], d_verify(ctx), sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    *failed = (int)ctx->h_pin[2] != 0;
+    return RT_OK;
+}
+
+// the resident batch (rt_segments_device) to the caller's batch callback, if there is one
+static int deliver_batch(rt_ctx *ctx, const Attempt &a) {
+    if (!a.cb) return RT_OK;
+    rt_batch bt;
+    int rc = rt_segments_device(ctx, &bt);
+    if (rc) return rc;
+    bt.attempt = a.index;
+    if (a.cb(&bt, a.cb_user)) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
+    return RT_OK;
+}
+
+// ---- chunk plan: cut tracks so that ~target_walkers independent walkers exist, >= chunk_segments segments each (n > 0) ----------
+static int plan_chunks(rt_ctx *ctx, WalkParams &P, uint32_t flags, double *launches) {
+    cudaStream_t st = ctx->stream;
+    const long long n = ctx->n_shard;
+    const DevMesh &m = ctx->m;
+    const long long n_blocks = (n + 31) / 32;
+    double rho = crossings_per_length(ctx);  // expected cell crossings per unit track length
+    double est_total = ctx->sum_len * rho;
+    double seg_target = fmax(ctx->opt_chunk_segments, est_total / ctx->opt_target_walkers);
+    double chunk_len = (flags & RT_SEG_NO_CHUNKS) || !(rho > 0.0) ? INFINITY : seg_target / rho;
+    rt_ctx::PlanKey key;
+    key.gen = ctx->trace_gen;
+    key.chunk_len = chunk_len;
+    key.band = ctx->opt_band_chunks;
+    key.band_min = ctx->opt_band_min;
+    key.band_div = ctx->opt_band_div;
+    key.order_grid = ctx->opt_order_grid + 1000 * ctx->opt_order_classes;
+    key.n = n;
+    const bool reuse = ctx->opt_plan_cache && key == ctx->plan_key && ctx->n_units > 0;
+    ChunkPlan &ch = P.ch;
+    if (!reuse) {
+        ctx->plan_key = rt_ctx::PlanKey{};
+        CK(ensure(ctx->b_nch, sizeof(int) * (size_t)n));
+        CK(ensure(ctx->b_blk_chunks, sizeof(int) * (size_t)n_blocks));
+        CK(ensure(ctx->b_unit_base, sizeof(long long) * ((size_t)n_blocks + 1)));
+        PlanGeom pg{ctx->t.px, ctx->t.py, ctx->t.qx, ctx->t.qy, {m.bbmin[0], m.bbmin[1]}, {m.bbmax[0], m.bbmax[1]},
+                    ctx->opt_band_chunks ? ctx->lmax : 0.0, ctx->opt_band_min * chunk_len, chunk_len / ctx->opt_band_div};
+        CK(ensure(ctx->b_layout, sizeof(ChunkLayout) * (size_t)n));
+        k_plan_chunks<<<blocks_for(n_blocks * 32, 128), 128, 0, st>>>(n, ctx->t.len, chunk_len, pg, (int *)ctx->b_nch.p,
+                                                                     (ChunkLayout *)ctx->b_layout.p, (int *)ctx->b_blk_chunks.p);
+        CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_blk_chunks.p, (long long *)ctx->b_unit_base.p, n_blocks)));
+        CK(cudaMemcpyAsync(&ctx->h_pin[0], (long long *)ctx->b_unit_base.p + n_blocks, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        ctx->n_units = ctx->h_pin[0];
+        *launches += 5;
+    }
+    const long long n_units = ctx->n_units;
+    size_t nc = (size_t)n_units * 32;
+    CK(ensure(ctx->b_unit_block, sizeof(int) * (size_t)n_units));
+    CK(ensure(ctx->b_ch_i, sizeof(int) * 5 * nc));
+    CK(ensure(ctx->b_ch_d, sizeof(double) * 3 * nc));
+    if (!reuse) {  // (slots no track owns are never written by the kernels, but the evaluation requests them before it knows that)
+        CK(cudaMemsetAsync(ctx->b_ch_i.p, 0, sizeof(int) * 5 * nc, st));
+        CK(cudaMemsetAsync(ctx->b_ch_d.p, 0, sizeof(double) * 3 * nc, st));
+    }
+    if (!reuse)
+        k_fill_units<<<blocks_for(n_blocks, 128), 128, 0, st>>>(n_blocks, (const long long *)ctx->b_unit_base.p,
+                                                                 (int *)ctx->b_unit_block.p);
+    ch.nch = (int *)ctx->b_nch.p;
+    ch.layout = (const ChunkLayout *)ctx->b_layout.p;
+    ch.unit_block = (int *)ctx->b_unit_block.p;
+    ch.unit_base = (long long *)ctx->b_unit_base.p;
+    ch.n_units = n_units;
+    int *ci = (int *)ctx->b_ch_i.p;
+    ch.seed_cell = ci;
+    ch.seed_kexit = ci + nc;
+    ch.count = ci + 2 * nc;
+    ch.endcode = ci + 3 * nc;
+    ch.prefix = ci + 4 * nc;
+    double *cd = (double *)ctx->b_ch_d.p;
+    ch.seed_qx = cd;
+    ch.seed_qy = cd + nc;
+    ch.sum = cd + 2 * nc;
+    P.unit_begin = 0;
+    P.unit_end = n_units;
+    // ---- execution orders (counting sorts of the units): the walk launches the units that start a track first and the short
+    // ones last, in Morton order of their tiles inside each class; the evaluation, whose warps live for microseconds, keeps
+    // the plain Morton order
+    ch.order = nullptr;
+    ctx->order_eval = nullptr;
+    if (ctx->opt_order_grid > 0 && n_units < (1LL << 31)) {
+        const bool two = ctx->opt_order_classes != 0;
+        if (!reuse) {
+            int G = std::min(ctx->opt_order_grid, 256);
+            int gp = 1;
+            while (gp < G) gp <<= 1;
+            CK(ensure(ctx->b_order, sizeof(int) * (size_t)n_units * (two ? 2 : 1)));
+            CK(ensure(ctx->b_okeys, sizeof(int) * (size_t)n_units));
+            for (int pass = 0; pass < (two ? 2 : 1); ++pass) {
+                const int classes = (two && pass == 0 && isfinite(chunk_len)) ? ctx->opt_order_classes : 1;
+                size_t n_keys = (size_t)gp * gp * classes;
+                CK(ensure(ctx->b_ohist, sizeof(int) * (3 * n_keys + 1)));
+                int *hist = (int *)ctx->b_ohist.p, *ptrs = hist + n_keys, *cursor = ptrs + n_keys + 1;
+                CK(cudaMemsetAsync(hist, 0, sizeof(int) * (3 * n_keys + 1), st));
+                k_unit_keys<<<blocks_for(n_units, 256), 256, 0, st>>>(P, G, classes, gp * gp, chunk_len, chunk_len / ctx->opt_band_div, (int *)ctx->b_okeys.p, hist);
+                CK((exclusive_scan<int, int>(ctx, hist, ptrs, (long long)n_keys)));
+                k_unit_scatter<<<blocks_for(n_units, 256), 256, 0, st>>>(n_units, (const int *)ctx->b_okeys.p, ptrs, cursor,
+                                                                        (int *)ctx->b_order.p + (size_t)pass * n_units);
+                *launches += 5;
+            }
+        }
+        ch.order = (const int *)ctx->b_order.p;
+        ctx->order_eval = two ? (const int *)ctx->b_order.p + n_units : ch.order;
+    }
+    if (!reuse) ctx->plan_key = key;
+    CK(cudaGetLastError());
+    return RT_OK;
+}
+
+// ---- single-walk pipeline (mode 3): k_march counts AND records every chunk in one walk, k_eval3 evaluates the records -------
 // The records live in a pool of kRecBlock-record blocks: block i < slots is the first block of chunk slot i of the batch, the
 // blocks behind are claimed by the walkers as they need them.  Shards whose pool would not fit next to the Segment columns are
 // processed in uid batches (whole 32-track blocks): count+record a batch, scan its offsets (carrying the running total), then
-// evaluate it -- in sub-batches when its segments exceed the resident capacity.  *next_mode = 0 asks the caller to repeat the
-// call with the hybrid pipeline (pool exhausted: the mesh is far denser along some chunks than the Cauchy-Crofton estimate).
-static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_vol, rt_batch_cb cb, void *cb_user, int attempt,
-                             bool *verify_failed, int *next_mode, double *launches_io, double est_total, bool *deferred_verify) {
-    *deferred_verify = false;
+// evaluate it -- in sub-batches when its segments exceed the resident capacity.  Next::Hybrid asks for the call to be repeated
+// with the hybrid pipeline (pool exhausted: the mesh is far denser along some chunks than the Cauchy-Crofton estimate).
+static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
     cudaStream_t st = ctx->stream;
     const long long n = ctx->n_shard;
     const long long n_blocks = (n + 31) / 32;
     const long long n_units = P.ch.n_units;
     const size_t nn = (size_t)std::max<long long>(n, 1);
-    double launches = 0;
     const int *order_all = P.ch.order;
     CK(ensure(ctx->b_tsum, sizeof(double) * nn));  // (cleared per batch by k_seed, like the pool cursor and the volume accumulator)
     CK(ensure(ctx->b_pool_cursor, sizeof(int)));
     P.tsum = (double *)ctx->b_tsum.p;
     P.pool_cursor = (int *)ctx->b_pool_cursor.p;
     const double lmin_eval = ctx->opt_debug_verify_fail ? INFINITY : P.lmin;
+    // the evaluation of the records of the tracks and units P describes (cancel: the guard of the optimistic evaluation)
+    auto launch_eval = [&](const int *cancel) {
+        WalkParams PE = P;
+        PE.lmin = lmin_eval;
+        PE.cancel = cancel;
+        if (PE.ch.order) PE.ch.order = ctx->order_eval;
+        k_eval3<<<blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads), kEval3Threads, 0, st>>>(PE);
+    };
 
     // ---- memory plan
     size_t free_b = 0, total_b = 0;
@@ -870,6 +1077,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_
         return cudaMemGetInfo(&free_b, &total_b);
     };
     const long long slots_all = n_units * 32;
+    const double est_total = ctx->sum_len * crossings_per_length(ctx);
     const double extra_per_slot = est_total * ctx->opt_pool_extra / kRecBlock / (double)std::max<long long>(slots_all, 1);
     const size_t block_bytes = sizeof(int) * (kRecBlock + 1);  // records + chain entry
     const long long spare = ctx->opt_pool_extra > 0.0 ? 4096 : 0;
@@ -887,8 +1095,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_
         }
         const long long pb = blocks_for_slots(std::min(max_slots, slots_all));
         if (max_slots < 32 || pb >= (1LL << 31)) {
-            *next_mode = 0;
-            *verify_failed = true;
+            a.next = Next::Hybrid;
             return RT_OK;
         }
         if ((size_t)pb > pool_have) {
@@ -948,73 +1155,40 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_
         P.vol = nullptr;
         P.offset_base = 0;
         P.cursor_init = (int)slots;
-        P.zero_vol = (want_vol && B0 == 0) ? ctx->vol_acc : nullptr;  // (+1: the failed-rank flag of rt_volumes)
+        P.zero_vol = (a.want_vol && B0 == 0) ? ctx->vol_acc : nullptr;  // (+1: the failed-rank flag of rt_volumes)
         P.zero_vol_n = (long long)P.m.n_cells + 1;
         if (ctx->opt_debug_clear_pool) CK(cudaMemsetAsync(ctx->b_pool.p, 0, ctx->b_pool.bytes, st));
         if (B0 > 0) tic(ctx, 2);  // (the first batch's count phase started with the chunk plan)
         k_seed<<<blocks_for(slots, 128), 128, 0, st>>>(P);
-        if (ctx->opt_march)
-            k_march<<<blocks_for(slots, kMarchThreads), kMarchThreads, 0, st>>>(P);
-        else
-            k_topo<2><<<blocks_for(slots, kTopoThreads), kTopoThreads, 0, st>>>(P);
+        k_march<<<blocks_for(slots, kMarchThreads), kMarchThreads, 0, st>>>(P);
         k_fixup_tracks<<<blocks_for(e - b, 128), 128, 0, st>>>(P);
         CK(cudaGetLastError());
         toc(ctx, 2);
         tic(ctx, 3);
-        const bool optimistic = !multi && !cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
+        const bool optimistic = !multi && !a.cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
                                 ctx->fit_gen == ctx->trace_gen && ctx->b_seg_d.p && ctx->cap > 0;
         ScanGuard guard{};
         if (optimistic) guard = ScanGuard{d_guard(ctx), base, ctx->cap, P.pool_cursor, P.pool_blocks};
         CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p + b, (long long *)ctx->b_offsets.p + b, e - b, base, guard)));
         toc(ctx, 3);
-        launches += 6;
+        a.launches += 6;
         CK(cudaMemcpyAsync(&ctx->h_pin[1], (long long *)ctx->b_offsets.p + e, sizeof(long long), cudaMemcpyDeviceToHost, st));
         if (!optimistic) CK(cudaMemcpyAsync(&ctx->h_pin[9], P.pool_cursor, sizeof(int), cudaMemcpyDeviceToHost, st));
         if (optimistic) {
             // ---- optimistic evaluation: no host round trip between the walk and the evaluation (see rt_ctx::opt_optimistic);
             // the guard (does the batch fit the Segment columns, did the pool hold every record?) is evaluated by the scan
-            P.opx = ctx->s_px;
-            P.opy = ctx->s_py;
-            P.oqx = ctx->s_qx;
-            P.oqy = ctx->s_qy;
-            P.olen = ctx->s_len;
-            P.oelem = ctx->s_elem;
-            P.vol = want_vol ? ctx->vol_acc : nullptr;
-            P.trk_begin = b;
-            P.trk_end = e;
             P.offset_base = base;
-            WalkParams PE = P;
-            PE.lmin = lmin_eval;
-            PE.cancel = d_guard(ctx);
-            if (PE.ch.order) PE.ch.order = ctx->order_eval;
+            bind_columns(ctx, P);
+            P.vol = a.want_vol ? ctx->vol_acc : nullptr;
             tic(ctx, 4);
-            k_eval3<<<blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads), kEval3Threads, 0, st>>>(PE);
-            EvalParams E{};
-            E.m = P.m;
-            E.t = ctx->t;
-            E.ang = P.ang;
-            E.offsets = P.offsets;
-            E.n_tracks = n;
-            E.olen = P.olen;
-            E.status = P.status;
-            E.tsum = P.tsum;
-            E.rtol = rtol;
-            E.trk_begin = b;
-            E.trk_end = e;
-            E.offset_base = base;
-            E.cancel = PE.cancel;
-            E.bad = d_bad(ctx);
-            k_track_status<<<blocks_for(e - b, 128), 128, 0, st>>>(E);
-            launches += 2;
+            launch_eval(d_guard(ctx));
+            launch_track_status(ctx, P, a.rtol, d_guard(ctx), d_bad(ctx));
+            a.launches += 2;
             CK(cudaGetLastError());
             toc(ctx, 4);
-            // (verification and guard flags come back with the control block at the end of the call, segmentize_once)
-            ctx->res_trk_begin = b;
-            ctx->res_trk_end = e;
-            ctx->res_off_base = base;
-            ctx->deferred_total = true;  // total / resident count are filled in by segmentize_once after its final read-back
-            *deferred_verify = true;
-            *launches_io += launches;
+            // (the total, the resident count and the verification and guard flags come with the final read-back of the attempt)
+            set_resident(ctx, b, e, base, 0);
+            a.defer_total = a.defer_verify = true;
             return RT_OK;
         }
         CK(cudaStreamSynchronize(st));
@@ -1022,42 +1196,23 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_
         take(3);
         const long long batch_total = ctx->h_pin[1] - base;
         if ((long long)*(int *)&ctx->h_pin[9] > (long long)P.pool_blocks) {  // some walker found the pool empty
-            *next_mode = 0;
-            *verify_failed = true;
+            a.next = Next::Hybrid;
             return RT_OK;
         }
         ctx->total_segments = base + batch_total;
         // ---- Segment columns: everything of this batch if it fits, else as much as fits
-        long long want = batch_total;
-        if (ctx->cap_cfg > 0) want = std::min(want, (long long)ctx->cap_cfg);
+        const long long want = ctx->cap_cfg > 0 ? std::min(batch_total, (long long)ctx->cap_cfg) : batch_total;
         if (want > ctx->cap || !ctx->b_seg_d.p) {
             CK(query_mem());
-            const long long fit = (long long)((double)(free_b + ctx->b_seg_d.bytes + ctx->b_seg_e.bytes) * 0.92 / 44.0);
-            long long cap = std::min(multi ? std::max(want, fit) : want, fit);
-            if (ctx->cap_cfg > 0) cap = std::min(cap, (long long)ctx->cap_cfg);
-            int rc = ensure_segment_buffers(ctx, cap);
+            long long fitted = 0;
+            int rc = size_columns(ctx, want, multi, free_b, &fitted);
             if (rc) return rc;
             have_mem = false;
         }
         const long long cap = ctx->cap_cfg > 0 ? std::min(ctx->cap, (long long)ctx->cap_cfg) : ctx->cap;
-        P.opx = ctx->s_px;
-        P.opy = ctx->s_py;
-        P.oqx = ctx->s_qx;
-        P.oqy = ctx->s_qy;
-        P.olen = ctx->s_len;
-        P.oelem = ctx->s_elem;
-        P.vol = want_vol ? ctx->vol_acc : nullptr;
-        EvalParams E{};
-        E.m = P.m;
-        E.t = ctx->t;
-        E.ang = P.ang;
-        E.offsets = P.offsets;
-        E.n_tracks = n;
-        E.olen = P.olen;
-        E.status = P.status;
-        E.tsum = P.tsum;
-        E.rtol = rtol;
-        E.bad = d_bad(ctx);
+        P.offset_base = base;
+        bind_columns(ctx, P);
+        P.vol = a.want_vol ? ctx->vol_acc : nullptr;
         const bool split = batch_total > cap;
         ctx->fit_gen = (!multi && !split) ? ctx->trace_gen : ~0ULL;  // (the next call with these tracks may skip this round trip)
         if (split) {
@@ -1069,104 +1224,163 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, double rtol, bool want_
             CK(cudaMemcpyAsync(h_off.data(), (long long *)ctx->b_offsets.p + b, sizeof(long long) * h_off.size(), cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
         }
-        long long sb = b;
-        while (sb < e) {
-            long long se = e;
+        for (long long sb = b; sb < e; sb = P.trk_end) {
+            long long nseg = batch_total;
             if (split) {
-                const long long lim = h_off[(size_t)(sb - b)] + cap;
-                se = b + (long long)(std::upper_bound(h_off.begin() + (sb - b), h_off.end(), lim) - h_off.begin()) - 1;
-                if (se <= sb) return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: one track needs more than the segment capacity");
+                int rc = cut_batch(ctx, P, h_off, b, h_unit_base, sb, cap, &nseg);
+                if (rc) return rc;
             }
-            const long long off_b = split ? h_off[(size_t)(sb - b)] : base;
-            const long long nseg_b = (split ? h_off[(size_t)(se - b)] : base + batch_total) - off_b;
-            P.trk_begin = sb;
-            P.trk_end = se;
-            P.offset_base = off_b;
-            if (split) {  // the warp units of the 32-track blocks overlapping [sb, se), in identity order
-                P.ch.order = nullptr;
-                P.unit_begin = h_unit_base[(size_t)(sb >> 5)];
-                P.unit_end = h_unit_base[(size_t)((se - 1) >> 5) + 1];
-            }
-            WalkParams PE = P;
-            PE.lmin = lmin_eval;
-            if (PE.ch.order) PE.ch.order = ctx->order_eval;
             tic(ctx, 4);
-            if (nseg_b > 0)
-                k_eval3<<<blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads), kEval3Threads, 0, st>>>(PE);
-            E.trk_begin = sb;
-            E.trk_end = se;
-            E.offset_base = off_b;
-            E.n_seg = nseg_b;
-            if (se > sb) k_track_status<<<blocks_for(se - sb, 128), 128, 0, st>>>(E);
-            launches += 2;
+            if (nseg > 0) launch_eval(nullptr);
+            launch_track_status(ctx, P, a.rtol, nullptr, d_bad(ctx));
+            a.launches += 2;
             CK(cudaGetLastError());
-            ctx->res_trk_begin = sb;
-            ctx->res_trk_end = se;
-            ctx->res_off_base = off_b;
-            ctx->res_nseg = nseg_b;
+            set_resident(ctx, P.trk_begin, P.trk_end, P.offset_base, nseg);
             toc(ctx, 4);
-            ctx->h_pin[2] = 0;
-            CK(cudaMemcpyAsync(&ctx->h_pin[2], d_verify(ctx), sizeof(int), cudaMemcpyDeviceToHost, st));
-            if (!cb && !multi && !split) {
-                // one batch, nobody waits for it: the verification flag is read with the final read-back of the call
-                // (segmentize_once), which saves one host synchronisation per call; the fill time is collected lazily
-                *deferred_verify = true;
+            if (!a.cb && !multi && !split) {
+                // one batch, nobody waits for it: the verification flag is read with the final read-back of the attempt, which
+                // saves one host synchronisation per call; the fill time is collected lazily
+                a.defer_verify = true;
                 ctx->phase_ms[2] = acc[2];
                 ctx->phase_ms[3] = acc[3];
-                *launches_io += launches;
                 return RT_OK;
             }
-            CK(cudaStreamSynchronize(st));
+            bool failed = false;
+            int rc = read_verify(ctx, &failed);
+            if (rc) return rc;
             take(4);
-            if ((int)ctx->h_pin[2]) {
-                *verify_failed = true;
+            if (failed) {
+                a.next = Next::Sequential;
                 return RT_OK;
             }
-            if (cb) {
-                rt_batch bt;
-                int rcb = rt_segments_device(ctx, &bt);
-                if (rcb) return rcb;
-                bt.attempt = attempt;
-                if (cb(&bt, cb_user)) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
-            }
-            sb = se;
+            rc = deliver_batch(ctx, a);
+            if (rc) return rc;
         }
         base += batch_total;
         B0 = B1;
     }
     for (int ph = 2; ph <= 4; ++ph) ctx->phase_ms[ph] = acc[ph];
-    *launches_io += launches;
     return RT_OK;
 }
 
-// One complete count -> scan -> fill execution.
+// ---- two-pass pipelines: count -> scan -> fill (possibly in uid batches over a recycled buffer)
 //   mode 1 (sequential): k_walk<false> counts, k_walk<true> fills (walk.cuh);
-//   mode 0 (hybrid):     k_topo<0> counts by sign tests (topo.cuh), k_walk<true> fills and re-derives the same decisions
-//                        from the exact geometry;
-//   mode 3 (single walk): segmentize_single above.
-// In modes 0 and 3 the length check (src/track.jl:171-175) runs after the fill (k_track_status).  *verify_failed reports that
-// the fill disagreed with the count (mode 0) or that a segment broke a geometric fast-path condition (mode 3): the caller then
-// repeats the call in mode 1.
-static int segmentize_once(rt_ctx *ctx, double tiny_step, int32_t k, double rtol, int32_t max_iter, uint32_t flags, rt_batch_cb cb,
-                           void *cb_user, int mode, int attempt, bool *verify_failed, unsigned long long *bad_out) {
-    const bool topo_count = mode != 1;
+//   mode 0 (hybrid):     k_topo counts by sign tests (topo.cuh), k_walk<true> fills and re-derives the same decisions from the
+//                        exact geometry, k_track_status runs the length check (src/track.jl:171-175) after the fill.  A fill
+//                        that disagrees with the count fails the verification: Next::Sequential.
+static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool hybrid, Attempt &a) {
     cudaStream_t st = ctx->stream;
     const long long n = ctx->n_shard;
-    const bool single = mode == 3 && n > 0;
-    double est_total_segments = 0.0;
-    bool deferred_verify = false;
+    const size_t nn = (size_t)std::max<long long>(n, 1);
+    // (+1: the failed-rank flag of rt_volumes)
+    if (a.want_vol) CK(cudaMemsetAsync(ctx->vol_acc, 0, sizeof(double) * ((size_t)ctx->m.n_cells + 1), st));
+    // ---- seeds, count pass, per-track fix-up
+    if (n > 0) {
+        const long long n_units = P.ch.n_units;
+        k_seed<<<blocks_for(n_units * 32, 128), 128, 0, st>>>(P);
+        if (hybrid) {
+            k_topo<<<blocks_for(n_units * 32, kTopoThreads), kTopoThreads, 0, st>>>(P);
+        } else {
+            P.vol = (a.want_vol && (flags & RT_SEG_COUNT_ONLY)) ? ctx->vol_acc : nullptr;
+            if (ctx->mixed)
+                k_walk<false, true><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+            else
+                k_walk<false><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        }
+        k_fixup_tracks<<<blocks_for(n, 128), 128, 0, st>>>(P);
+        a.launches += 3;
+        a.first_bad_scan = true;
+    }
+    CK(cudaGetLastError());
+    toc(ctx, 2);
+    // ---- scan
+    tic(ctx, 3);
+    long long total = 0;
+    if (n > 0) {
+        CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p, (long long *)ctx->b_offsets.p, n)));
+        a.launches += 3;
+        CK(cudaMemcpyAsync(&ctx->h_pin[1], (long long *)ctx->b_offsets.p + n, sizeof(long long), cudaMemcpyDeviceToHost, st));
+    }
+    toc(ctx, 3);
+    CK(cudaStreamSynchronize(st));
+    if (n > 0) total = ctx->h_pin[1];
+    ctx->total_segments = total;
+    ctx->phase_ms[4] = 0.0;
+    ctx->pev_dirty[4] = false;
+    if ((flags & RT_SEG_COUNT_ONLY) || n == 0) return RT_OK;
+
+    // ---- fill pass
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    long long cap = 0;
+    int rc = size_columns(ctx, ctx->cap_cfg > 0 ? std::min(total, (long long)ctx->cap_cfg) : total, false, free_b, &cap);
+    if (rc) return rc;
+    if (hybrid) {
+        CK(ensure(ctx->b_tsum, sizeof(double) * nn));
+        CK(cudaMemsetAsync(ctx->b_tsum.p, 0, sizeof(double) * nn, st));
+    }
+    bind_columns(ctx, P);
+    P.tsum = hybrid ? (double *)ctx->b_tsum.p : nullptr;
+    P.vol = a.want_vol ? ctx->vol_acc : nullptr;
+    P.counters = nullptr;
+    if (ctx->opt_debug_verify_fail && hybrid) CK(cudaMemsetAsync(d_verify(ctx), 1, 1, st));
+    const bool split = total > cap;
+    std::vector<long long> h_off, h_unit_base;
+    if (split) {
+        h_off.resize((size_t)n + 1);
+        CK(cudaMemcpy(h_off.data(), ctx->b_offsets.p, sizeof(long long) * ((size_t)n + 1), cudaMemcpyDeviceToHost));
+        h_unit_base.resize((size_t)((n + 31) / 32) + 1);
+        CK(cudaMemcpy(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost));
+    }
+    tic(ctx, 4);
+    for (long long b = 0; b < n; b = P.trk_end) {
+        long long nseg = total;
+        if (split) {
+            rc = cut_batch(ctx, P, h_off, 0, h_unit_base, b, cap, &nseg);
+            if (rc) return rc;
+        }
+        if (ctx->mixed)
+            k_walk<true, true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        else
+            k_walk<true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        a.launches += 1;
+        if (hybrid) {
+            launch_track_status(ctx, P, a.rtol, nullptr, nullptr);
+            a.launches += 1;
+        }
+        CK(cudaGetLastError());
+        set_resident(ctx, P.trk_begin, P.trk_end, P.offset_base, nseg);
+        if (hybrid) {
+            bool failed = false;
+            rc = read_verify(ctx, &failed);
+            if (rc) return rc;
+            if (failed) {
+                a.next = Next::Sequential;
+                toc(ctx, 4);
+                return RT_OK;
+            }
+        }
+        rc = deliver_batch(ctx, a);
+        if (rc) return rc;
+    }
+    toc(ctx, 4);
+    return RT_OK;
+}
+
+// One attempt of rt_segmentize in pipeline `mode` (segmentize_single or segmentize_two_pass); a.next says whether it stands.
+static int segmentize_attempt(rt_ctx *ctx, double tiny_step, int32_t k, int32_t max_iter, uint32_t flags, int mode, Attempt &a,
+                              unsigned long long *bad_out) {
+    cudaStream_t st = ctx->stream;
+    const long long n = ctx->n_shard;
     const int n2 = ctx->n2;
-    DevMesh &m = ctx->m;
-    const bool want_vol = !(flags & RT_SEG_NO_VOLUMES);
-    *verify_failed = false;
+    const DevMesh &m = ctx->m;
     *bad_out = ~0ULL;
-    // (+1: the failed-rank flag of rt_volumes; the single-walk pipeline clears the accumulator in its first k_seed)
-    if (want_vol && !(mode == 3 && n > 0)) CK(cudaMemsetAsync(ctx->vol_acc, 0, sizeof(double) * ((size_t)m.n_cells + 1), st));
-    size_t nn = (size_t)std::max<long long>(n, 1);
+    // ---- control block: counters, "no bad track", flags
     for (int q = 0; q < 8; ++q) ctx->h_pin[kPinCtrlInit + q] = 0;
-    ctx->h_pin[kPinCtrlInit + 4] = -1LL;  // "no bad track"
+    ctx->h_pin[kPinCtrlInit + 4] = -1LL;
     CK(cudaMemcpyAsync(ctx->b_ctrl.p, &ctx->h_pin[kPinCtrlInit], 64, cudaMemcpyHostToDevice, st));
-    if (n == 0) CK(cudaMemsetAsync(ctx->b_offsets.p, 0, sizeof(long long) * (nn + 1), st));  // (otherwise the scan writes all n + 1 entries)
+    if (n == 0) CK(cudaMemsetAsync(ctx->b_offsets.p, 0, sizeof(long long) * 2, st));  // (otherwise the scan writes all n + 1 entries)
+    set_resident(ctx, 0, 0, 0, 0);
 
     WalkParams P{};
     P.m = m;
@@ -1177,7 +1391,7 @@ static int segmentize_once(rt_ctx *ctx, double tiny_step, int32_t k, double rtol
     P.ang.cosp = ad + 2 * n2;
     P.ang.delta_eff = ad + 6 * n2;
     P.tiny = tiny_step;
-    P.rtol = topo_count ? -1.0 : rtol;  // sign-test count: the length check runs after the fill (k_track_status)
+    P.rtol = mode == 1 ? a.rtol : -1.0;  // sign-test count: the length check runs after the fill (k_track_status)
     P.k = k;
     P.max_iter = max_iter;
     P.flags = flags;
@@ -1189,276 +1403,20 @@ static int segmentize_once(rt_ctx *ctx, double tiny_step, int32_t k, double rtol
     P.offsets = (const long long *)ctx->b_offsets.p;
     P.counters = d_counters(ctx);
     P.verify_fail = d_verify(ctx);
-    const bool count_only = (flags & RT_SEG_COUNT_ONLY) != 0;
-    double launches = 0;
-
-    // ---- chunk plan: cut tracks so that ~target_walkers independent walkers exist, >= chunk_segments segments each
-    tic(ctx, 2);
     P.n_tracks = n;
     P.trk_begin = 0;
     P.trk_end = n;
-    std::vector<long long> h_unit_base;
-    if (n > 0) {
-        const long long n_blocks = (n + 31) / 32;
-        double rho = ctx->edge_sum / (kPi * ctx->area);  // expected cell crossings per unit track length
-        double est_total = ctx->sum_len * rho;
-        est_total_segments = est_total;
-        double seg_target = fmax(ctx->opt_chunk_segments, est_total / ctx->opt_target_walkers);
-        double chunk_len = (flags & RT_SEG_NO_CHUNKS) || !(rho > 0.0) ? INFINITY : seg_target / rho;
-        rt_ctx::PlanKey key;
-        key.gen = ctx->trace_gen;
-        key.chunk_len = chunk_len;
-        key.band = ctx->opt_band_chunks;
-        key.band_min = ctx->opt_band_min;
-        key.band_div = ctx->opt_band_div;
-        key.order_grid = ctx->opt_order_grid + 1000 * ctx->opt_order_classes;
-        key.n = n;
-        const bool reuse = ctx->opt_plan_cache && key == ctx->plan_key && ctx->n_units > 0;
-        ChunkPlan &ch = P.ch;
-        if (!reuse) {
-            ctx->plan_key = rt_ctx::PlanKey{};
-            CK(ensure(ctx->b_nch, sizeof(int) * (size_t)n));
-            CK(ensure(ctx->b_blk_chunks, sizeof(int) * (size_t)n_blocks));
-            CK(ensure(ctx->b_unit_base, sizeof(long long) * ((size_t)n_blocks + 1)));
-            PlanGeom pg{ctx->t.px, ctx->t.py, ctx->t.qx, ctx->t.qy, {m.bbmin[0], m.bbmin[1]}, {m.bbmax[0], m.bbmax[1]},
-                        ctx->opt_band_chunks ? ctx->lmax : 0.0, ctx->opt_band_min * chunk_len, chunk_len / ctx->opt_band_div};
-            CK(ensure(ctx->b_layout, sizeof(ChunkLayout) * (size_t)n));
-            k_plan_chunks<<<blocks_for(n_blocks * 32, 128), 128, 0, st>>>(n, ctx->t.len, chunk_len, pg, (int *)ctx->b_nch.p,
-                                                                         (ChunkLayout *)ctx->b_layout.p, (int *)ctx->b_blk_chunks.p);
-            CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_blk_chunks.p, (long long *)ctx->b_unit_base.p, n_blocks)));
-            CK(cudaMemcpyAsync(&ctx->h_pin[0], (long long *)ctx->b_unit_base.p + n_blocks, sizeof(long long), cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            ctx->n_units = ctx->h_pin[0];
-            launches += 5;
-        }
-        const long long n_units = ctx->n_units;
-        size_t nc = (size_t)n_units * 32;
-        CK(ensure(ctx->b_unit_block, sizeof(int) * (size_t)n_units));
-        CK(ensure(ctx->b_ch_i, sizeof(int) * 5 * nc));
-        CK(ensure(ctx->b_ch_d, sizeof(double) * 3 * nc));
-        if (!reuse) {  // (slots no track owns are never written by the kernels, but the evaluation requests them before it knows that)
-            CK(cudaMemsetAsync(ctx->b_ch_i.p, 0, sizeof(int) * 5 * nc, st));
-            CK(cudaMemsetAsync(ctx->b_ch_d.p, 0, sizeof(double) * 3 * nc, st));
-        }
-        if (!reuse)
-            k_fill_units<<<blocks_for(n_blocks, 128), 128, 0, st>>>(n_blocks, (const long long *)ctx->b_unit_base.p,
-                                                                     (int *)ctx->b_unit_block.p);
-        ch.nch = (int *)ctx->b_nch.p;
-        ch.layout = (const ChunkLayout *)ctx->b_layout.p;
-        ch.unit_block = (int *)ctx->b_unit_block.p;
-        ch.unit_base = (long long *)ctx->b_unit_base.p;
-        ch.n_units = n_units;
-        int *ci = (int *)ctx->b_ch_i.p;
-        ch.seed_cell = ci;
-        ch.seed_kexit = ci + nc;
-        ch.count = ci + 2 * nc;
-        ch.endcode = ci + 3 * nc;
-        ch.prefix = ci + 4 * nc;
-        double *cd = (double *)ctx->b_ch_d.p;
-        ch.seed_qx = cd;
-        ch.seed_qy = cd + nc;
-        ch.sum = cd + 2 * nc;
-        P.unit_begin = 0;
-        P.unit_end = n_units;
-        // ---- execution orders (counting sorts of the units): the walk launches the units that start a track first and the short
-        // ones last, in Morton order of their tiles inside each class; the evaluation, whose warps live for microseconds, keeps
-        // the plain Morton order
-        ch.order = nullptr;
-        ctx->order_eval = nullptr;
-        if (ctx->opt_order_grid > 0 && n_units < (1LL << 31)) {
-            const bool two = ctx->opt_order_classes != 0;
-            if (!reuse) {
-                int G = std::min(ctx->opt_order_grid, 256);
-                int gp = 1;
-                while (gp < G) gp <<= 1;
-                CK(ensure(ctx->b_order, sizeof(int) * (size_t)n_units * (two ? 2 : 1)));
-                CK(ensure(ctx->b_okeys, sizeof(int) * (size_t)n_units));
-                for (int pass = 0; pass < (two ? 2 : 1); ++pass) {
-                    const int classes = (two && pass == 0 && isfinite(chunk_len)) ? ctx->opt_order_classes : 1;
-                    size_t n_keys = (size_t)gp * gp * classes;
-                    CK(ensure(ctx->b_ohist, sizeof(int) * (3 * n_keys + 1)));
-                    int *hist = (int *)ctx->b_ohist.p, *ptrs = hist + n_keys, *cursor = ptrs + n_keys + 1;
-                    CK(cudaMemsetAsync(hist, 0, sizeof(int) * (3 * n_keys + 1), st));
-                    k_unit_keys<<<blocks_for(n_units, 256), 256, 0, st>>>(P, G, classes, gp * gp, chunk_len, chunk_len / ctx->opt_band_div, (int *)ctx->b_okeys.p, hist);
-                    CK((exclusive_scan<int, int>(ctx, hist, ptrs, (long long)n_keys)));
-                    k_unit_scatter<<<blocks_for(n_units, 256), 256, 0, st>>>(n_units, (const int *)ctx->b_okeys.p, ptrs, cursor,
-                                                                            (int *)ctx->b_order.p + (size_t)pass * n_units);
-                    launches += 5;
-                }
-            }
-            ch.order = (const int *)ctx->b_order.p;
-            ctx->order_eval = two ? (const int *)ctx->b_order.p + n_units : ch.order;
-        }
-        if (!reuse) ctx->plan_key = key;
-        // ---- seeds, count pass, per-track fix-up
-        P.vol = nullptr;
-        if (single) {
-            // (the single-walk pipeline runs them per uid batch, see segmentize_single)
-        } else {
-        k_seed<<<blocks_for(n_units * 32, 128), 128, 0, st>>>(P);
-        if (topo_count) {
-            k_topo<0><<<blocks_for(n_units * 32, kTopoThreads), kTopoThreads, 0, st>>>(P);
-        } else {
-            P.vol = (want_vol && count_only) ? ctx->vol_acc : nullptr;
-            if (ctx->mixed)
-                k_walk<false, true><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-            else
-                k_walk<false><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-        }
-        k_fixup_tracks<<<blocks_for(n, 128), 128, 0, st>>>(P);
-        launches += 3;
-        }
-    }
-    CK(cudaGetLastError());
-    if (single) {
-        ctx->res_trk_begin = ctx->res_trk_end = 0;
-        ctx->res_off_base = 0;
-        ctx->res_nseg = 0;
-        P.counters = d_counters(ctx);
-        int next_mode = 1;
-        int rc = segmentize_single(ctx, P, rtol, want_vol, cb, cb_user, attempt, verify_failed, &next_mode, &launches, est_total_segments,
-                                   &deferred_verify);
-        if (rc) return rc;
-        if (*verify_failed) {
-            ctx->fallback_mode = next_mode;
-            return RT_OK;
-        }
-    }
-    if (!single) toc(ctx, 2);
-    // ---- scan
-    if (!single) tic(ctx, 3);
-    long long total = 0;
-    if (n > 0 && !single) {
-        CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p, (long long *)ctx->b_offsets.p, n)));
-        launches += 3;
-        CK(cudaMemcpyAsync(&ctx->h_pin[1], (long long *)ctx->b_offsets.p + n, sizeof(long long), cudaMemcpyDeviceToHost, st));
-    }
-    if (!single) {
-        toc(ctx, 3);
-        CK(cudaStreamSynchronize(st));
-        if (n > 0) total = ctx->h_pin[1];
-        ctx->total_segments = total;
-    }
 
-    // ---- fill pass (possibly in uid batches over a recycled buffer)
-    if (!single) {
-        ctx->phase_ms[4] = 0.0;
-        ctx->pev_dirty[4] = false;
-        ctx->res_trk_begin = ctx->res_trk_end = 0;
-        ctx->res_off_base = 0;
-        ctx->res_nseg = 0;
-    }
-    if (!count_only && n > 0 && !single) {
-        long long cap = total;
-        size_t free_b = 0, total_b = 0;
-        CK(cudaMemGetInfo(&free_b, &total_b));
-        long long fit = (long long)((double)(free_b + ctx->b_seg_d.bytes + ctx->b_seg_e.bytes) * 0.92 / 44.0);
-        if (ctx->cap_cfg > 0) cap = std::min(cap, (long long)ctx->cap_cfg);
-        cap = std::min(cap, fit);
-        int rc = ensure_segment_buffers(ctx, cap);
+    tic(ctx, 2);  // (the count phase of the first batch includes the chunk plan)
+    if (n > 0) {
+        int rc = plan_chunks(ctx, P, flags, &a.launches);
         if (rc) return rc;
-        if (topo_count) {
-            CK(ensure(ctx->b_tsum, sizeof(double) * nn));
-            CK(cudaMemsetAsync(ctx->b_tsum.p, 0, sizeof(double) * nn, st));
-        }
-        P.opx = ctx->s_px;
-        P.opy = ctx->s_py;
-        P.oqx = ctx->s_qx;
-        P.oqy = ctx->s_qy;
-        P.olen = ctx->s_len;
-        P.oelem = ctx->s_elem;
-        P.tsum = topo_count ? (double *)ctx->b_tsum.p : nullptr;
-        P.vol = want_vol ? ctx->vol_acc : nullptr;
-        P.counters = nullptr;
-        EvalParams E{};
-        E.m = m;
-        E.t = ctx->t;
-        E.ang = P.ang;
-        E.offsets = P.offsets;
-        E.n_tracks = n;
-        E.opx = P.opx;
-        E.opy = P.opy;
-        E.oqx = P.oqx;
-        E.oqy = P.oqy;
-        E.olen = P.olen;
-        E.oelem = P.oelem;
-        E.vol = P.vol;
-        E.lmin = ctx->opt_debug_verify_fail ? INFINITY : P.lmin;
-        if (ctx->opt_debug_verify_fail && topo_count) CK(cudaMemsetAsync(d_verify(ctx), 1, 1, st));
-        E.verify_fail = P.verify_fail;
-        E.status = P.status;
-        E.tsum = P.tsum;
-        E.rtol = rtol;
-        std::vector<long long> h_off;
-        if (total > cap) {
-            h_off.resize((size_t)n + 1);
-            CK(cudaMemcpy(h_off.data(), ctx->b_offsets.p, sizeof(long long) * ((size_t)n + 1), cudaMemcpyDeviceToHost));
-            h_unit_base.resize((size_t)((n + 31) / 32) + 1);
-            CK(cudaMemcpy(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost));
-        }
-        tic(ctx, 4);
-        long long b = 0;
-        while (b < n) {
-            long long e = n;
-            if (total > cap) {
-                // largest e with off[e] - off[b] <= cap
-                long long lim = h_off[b] + cap;
-                e = (long long)(std::upper_bound(h_off.begin() + b, h_off.end(), lim) - h_off.begin()) - 1;
-                if (e <= b) return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: one track needs more than the segment capacity");
-            }
-            P.trk_begin = b;
-            P.trk_end = e;
-            P.offset_base = total > cap ? h_off[b] : 0;
-            if (total > cap) {  // the warp units of the 32-track blocks overlapping [b, e), in identity order
-                P.ch.order = nullptr;
-                P.unit_begin = h_unit_base[(size_t)(b >> 5)];
-                P.unit_end = h_unit_base[(size_t)((e - 1) >> 5) + 1];
-            }
-            const long long nseg_b = (total > cap ? h_off[e] : total) - P.offset_base;
-            {
-                if (ctx->mixed)
-                    k_walk<true, true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-                else
-                    k_walk<true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-                launches += 1;
-                if (topo_count) {
-                    E.trk_begin = b;
-                    E.trk_end = e;
-                    E.offset_base = P.offset_base;
-                    E.n_seg = nseg_b;
-                    k_track_status<<<blocks_for(e - b, 128), 128, 0, st>>>(E);
-                    launches += 1;
-                }
-            }
-            CK(cudaGetLastError());
-            ctx->res_trk_begin = b;
-            ctx->res_trk_end = e;
-            ctx->res_off_base = P.offset_base;
-            ctx->res_nseg = nseg_b;
-            if (topo_count) {
-                ctx->h_pin[2] = 0;
-                CK(cudaMemcpyAsync(&ctx->h_pin[2], d_verify(ctx), sizeof(int), cudaMemcpyDeviceToHost, st));
-                CK(cudaStreamSynchronize(st));
-                const int vf = (int)ctx->h_pin[2];
-                if (vf) {
-                    *verify_failed = true;
-                    toc(ctx, 4);
-                    return RT_OK;
-                }
-            }
-            if (cb) {
-                rt_batch bt;
-                int rcb = rt_segments_device(ctx, &bt);
-                if (rcb) return rcb;
-                bt.attempt = attempt;
-                if (cb(&bt, cb_user)) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
-            }
-            b = e;
-        }
-        toc(ctx, 4);
     }
+    int rc = mode == 3 && n > 0 ? segmentize_single(ctx, P, a) : segmentize_two_pass(ctx, P, flags, mode == 0, a);
+    if (rc || a.next != Next::Done) return rc;
+
     ctx->voln_done = false;
-    if (want_vol && m.n_cells > 0 && ctx->vol_acc && !(ctx->comm && ctx->coll_stream)) {
+    if (a.want_vol && m.n_cells > 0 && ctx->vol_acc && !(ctx->comm && ctx->coll_stream)) {
         // volumes ./= n_azim_2 right behind the evaluation (rt_volumes would launch it after the host has seen the call return:
         // one more host round trip with the GPU idle); with a communicator the all-reduce comes first and rt_volumes does both
         CK(ensure(ctx->b_voln, sizeof(double) * ((size_t)m.n_cells + 1)));
@@ -1467,39 +1425,33 @@ static int segmentize_once(rt_ctx *ctx, double tiny_step, int32_t k, double rtol
         CK(cudaGetLastError());
         toc(ctx, 5);
         ctx->voln_done = true;
-        launches += 1;
+        a.launches += 1;
     }
-    unsigned long long bad = ~0ULL;
-    if (n > 0 && !single) {  // (the single-walk pipeline's k_track_status reports the failing tracks itself)
+    if (a.first_bad_scan) {
         k_first_bad<<<blocks_for(n, 256), 256, 0, st>>>((const int *)ctx->b_status.p, n, d_bad(ctx));
-        launches += 1;
+        a.launches += 1;
     }
     CK(cudaMemcpyAsync(&ctx->h_pin[kPinCtrl], ctx->b_ctrl.p, 64, cudaMemcpyDeviceToHost, st));  // counters, first bad track, flags: one copy
     CK(cudaStreamSynchronize(st));
     const int flag_verify = (int)(ctx->h_pin[kPinCtrl + 5] & 0xffffffffLL), flag_guard = (int)((unsigned long long)ctx->h_pin[kPinCtrl + 5] >> 32);
-    if (ctx->deferred_total) {  // optimistic evaluation: the total arrives only now
-        ctx->deferred_total = false;
+    if (a.defer_total) {  // optimistic evaluation: the total arrives only now
         if (flag_guard) {  // cancelled on the device (Segment columns or record pool too small): repeat on the careful path
             ctx->skip_optimistic_once = true;
             ctx->optimistic_cancels += 1;
             ctx->fit_gen = ~0ULL;
-            ctx->redo_careful = true;
-            *verify_failed = true;
+            a.next = Next::RepeatCareful;
             return RT_OK;
         }
         ctx->total_segments = ctx->h_pin[1];
         ctx->res_nseg = ctx->h_pin[1];
     }
-    if (deferred_verify && flag_verify) {
-        *verify_failed = true;
+    if (a.defer_verify && flag_verify) {
+        a.next = Next::Sequential;
         return RT_OK;
     }
-    if (n > 0) bad = (unsigned long long)ctx->h_pin[kPinCtrl + 4];
-    unsigned long long hc[4];
-    for (int q = 0; q < 4; ++q) hc[q] = (unsigned long long)ctx->h_pin[kPinCtrl + q];
-    ctx->stats[0] += launches;
-    for (int q = 0; q < 4; ++q) ctx->stats[1 + q] = (double)hc[q];
-    *bad_out = bad;
+    if (n > 0) *bad_out = (unsigned long long)ctx->h_pin[kPinCtrl + 4];
+    ctx->stats[0] += a.launches;
+    for (int q = 0; q < 4; ++q) ctx->stats[1 + q] = (double)(unsigned long long)ctx->h_pin[kPinCtrl + q];
     return RT_OK;
 }
 
@@ -1565,18 +1517,12 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
     unsigned long long bad = ~0ULL;
     if (mode == 3 && (flags & RT_SEG_LITERAL)) mode = 1;  // (literal-only walks have nothing to gain from per-segment evaluation)
     for (int attempt = 0; attempt < 4; ++attempt) {
-        bool vf = false;
-        ctx->fallback_mode = 1;
-        int rc = segmentize_once(ctx, tiny_step, k, rtol, max_iter, flags, cb, cb_user, mode, attempt, &vf, &bad);
+        Attempt a{rtol, want_vol, cb, cb_user, attempt};
+        int rc = segmentize_attempt(ctx, tiny_step, k, max_iter, flags, mode, a, &bad);
         if (rc) return rc;
-        if (!vf) break;
-        if (ctx->redo_careful) {  // the optimistic evaluation did not fit: same pipeline, sized from the walk's result this time
-            ctx->redo_careful = false;
-            continue;
-        }
-        // count and fill disagreed / a geometric fast-path condition failed: redo everything sequentially (the single-walk
-        // pipeline asks for the hybrid one when its record pool ran out)
-        mode = ctx->fallback_mode;
+        if (a.next == Next::Done) break;
+        if (a.next == Next::RepeatCareful) continue;  // the optimistic evaluation did not fit: sized from the walk's result this time
+        mode = a.next == Next::Hybrid ? 0 : 1;
         ctx->verify_fallbacks += 1;
     }
     ctx->skip_optimistic_once = false;
@@ -2117,8 +2063,6 @@ extern "C" int rt_set_option(rt_ctx *ctx, const char *name, double value) {
         ctx->opt_order_grid = (int)value;
     else if (n == "pipeline" && (value == 0.0 || value == 1.0 || value == 3.0))
         ctx->opt_pipeline = (int)value;
-    else if (n == "march")
-        ctx->opt_march = value != 0.0;
     else if (n == "debug_clear_pool")
         ctx->opt_debug_clear_pool = value != 0.0;
     else if (n == "band_cost" && value >= 0.0)

@@ -4,13 +4,11 @@
 // (src/intersection.jl:60).  So the serial part of _segmentize_track! (src/track.jl:106-178) is only the ORDER in which
 // cells are accepted; the geometry of every accepted cell can be evaluated independently afterwards.
 //
-//   k_topo<0>  count pass of the hybrid pipeline: walks the half-edge graph deciding each transition from the SIGNS of the
+//   k_topo     count pass of the hybrid pipeline: walks the half-edge graph deciding each transition from the SIGNS of the
 //                  signed distances of the cell's vertices from the track line (two multiply-adds per step, no division, no
 //                  square root), under the same clearance test as the sequential fast path (walk.cuh); everything that test
-//                  does not cover runs the literal walk of the reference, exactly as in walk.cuh.
-//   k_topo<2>  count AND record in one walk (the reference form of k_march, march.cuh): one 4-byte record per segment
-//                  fast:  (h << 2) | (exit1 << 1)   h = entry half-edge 3*cell + k, exit1: leaves through edge k+1 (else k+2)
-//                  literal: (cell << 2) | 1
+//                  does not cover runs the literal walk of the reference, exactly as in walk.cuh.  (k_march, march.cuh, is the
+//                  same walk for the single-walk pipeline: it also records every accepted cell.)
 //   k_track_status per track: the reference's length check (src/track.jl:171-175) on the accumulated segment lengths.
 #pragma once
 #include "walk.cuh"
@@ -28,30 +26,6 @@ __device__ __forceinline__ void stg256_plain_i(void *p, const int *v) {
                  "r"(v[5]), "r"(v[6]), "r"(v[7])
                  : "memory");
 }
-__device__ __forceinline__ void stg256_stream_i(void *p, unsigned long long pol, const int *v) {
-    asm volatile("st.global.L2::cache_hint.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8}, %9;" ::"l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]),
-                 "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "l"(pol)
-                 : "memory");
-}
-
-// scalar loads / stores with L2 eviction policies (see walk.cuh): the node and cell tables are re-read by every segment
-// (evict_last), the per-segment records and the Segment columns pass through once (evict_first)
-__device__ __forceinline__ int ldg_i32_pol(const int *p, unsigned long long pol) {
-    int v;
-    asm volatile("ld.global.nc.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    return v;
-}
-__device__ __forceinline__ double2 ldg_f64x2_pol(const double2 *p, unsigned long long pol) {
-    double2 v;
-    asm volatile("ld.global.nc.L2::cache_hint.v2.f64 {%0,%1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol));
-    return v;
-}
-__device__ __forceinline__ void stg_f64_pol(double *p, double v, unsigned long long pol) {
-    asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(p), "d"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void stg_i32_pol(int *p, int v, unsigned long long pol) {
-    asm volatile("st.global.L2::cache_hint.b32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-}
 
 // exit point of cell `c` through its local edge k: the reference's intersection() with that edge's line
 __device__ __forceinline__ P2 exit_point(const DevMesh &m, const Line &trk, int c, int k) {
@@ -61,17 +35,10 @@ __device__ __forceinline__ P2 exit_point(const DevMesh &m, const Line &trk, int 
     return X;
 }
 
-// MODE 0: count only; MODE 2: count AND record in one walk -- the records go to a pool of kRecBlock-record blocks (the chunk's first block
-// is implicit, further blocks are claimed with one atomic each and chained through pool_next), from where k_eval3 (eval3.cuh)
-// evaluates them once the scan has fixed the final positions.
-template <int MODE>
+// the count pass of the hybrid pipeline (see the top of this file)
 __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const __grid_constant__ WalkParams P) {
-    static_assert(MODE == 0 || MODE == 2, "k_topo: count (0) or count+record (2)");
-    constexpr bool REC = MODE == 2;
     const unsigned FULL = 0xffffffffu;
     const DevMesh &m = P.m;
-    __shared__ int s_rec[REC ? 8 * kTopoThreads : 1];  // 8 records per thread = one 32-byte sector
-    const int tid = threadIdx.x;
     long long gw = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
     int lane = threadIdx.x & 31;
     long long slot = P.unit_begin + gw;
@@ -96,8 +63,6 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
     const bool literal_only = (P.flags & 1u) != 0;
     bool active = false;
     const unsigned long long pol_keep = l2_policy_keep();
-    int pb = REC ? (int)(cidx - P.pool_slot_base) : 0;  // MODE 2: block of the pool that is being filled
-    bool recording = REC;
     constexpr double kKappa = 1.0 / RT_KAPPA_INV;  // smallest sine of a crossing angle the cheap filter accepts
     bool cheap_ok = false;                 // x-ordering of entry/exit is decided by the track direction, beyond rounding
     double ang_thr = 0.0;
@@ -160,28 +125,7 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
         }
     }
 
-    auto push = [&](int e, int rec) {
-        if (REC && recording) {
-            if (nseg > 0 && (nseg & (kRecBlock - 1)) == 0) {  // the current block is full: claim the next one
-                const int nb = atomicAdd(P.pool_cursor, 1);
-                if (nb >= P.pool_blocks) {
-                    recording = false;  // pool exhausted (the host sees pool_cursor > pool_blocks and repeats the call with another pipeline)
-                } else {
-                    P.pool_next[pb] = nb;
-                    pb = nb;
-                }
-            }
-            if (recording) {
-                const int k = nseg & 7;
-                s_rec[k * kTopoThreads + tid] = rec;
-                if (k == 7) {
-                    int v[8];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) v[q] = s_rec[q * kTopoThreads + tid];
-                    stg256_plain_i(P.pool + (long long)pb * kRecBlock + ((nseg & (kRecBlock - 1)) - 7), v);
-                }
-            }
-        }
+    auto push = [&](int e) {
         nseg += 1;
         if (nseg >= limit) {  // while i < MAX_ITER (src/track.jl:119)
             endcode = END_CAP;
@@ -246,7 +190,7 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
                         enc = nenc;
                         clearA = clearB;
                         ok = true;
-                        push(cur, (h << 2) | (exit1 ? 2 : 0));
+                        push(cur);
                     }
                 }
             }
@@ -270,7 +214,7 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
             }
             if (o.code == 0) {
                 n_litpush++;
-                push(o.e, (o.e << 2) | 1);
+                push(o.e);
                 cur = o.e;
                 cur_kout = o.e_q;
                 qx = o.qx;
@@ -287,17 +231,10 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
         }
     }
 
-    if (REC && recording && (nseg & 7)) {  // the incomplete last sector of this chunk's records
-        const int rem = nseg & 7;
-        int *dst = P.pool + (long long)pb * kRecBlock + (((nseg - 1) & (kRecBlock - 1)) - (rem - 1));
-        for (int kk = 0; kk < rem; ++kk) dst[kk] = s_rec[kk * kTopoThreads + tid];
-    }
     if (t < P.n_tracks && j < P.ch.nch[t]) {
         P.ch.count[cidx] = active ? nseg : 0;
         P.ch.sum[cidx] = 0.0;
         P.ch.endcode[cidx] = active ? (endcode | (status << 8)) : (END_HANDOFF | (0 << 8));
-    } else if (REC) {
-        P.ch.count[cidx] = 0;  // (a slot no track owns: the evaluation requests its count before it knows that)
     }
     if (P.counters) {
         unsigned long long v = active ? (unsigned long long)(nseg - n_litpush) : 0ull;
@@ -308,19 +245,11 @@ __global__ void __launch_bounds__(kTopoThreads, RT_TOPO_MIN_BLOCKS) k_topo(const
 
 // ---- per-track length check after the fill --------------------------------------------------------------------------------
 struct EvalParams {
-    DevMesh m;
     TrackSoA t;
-    AngleTabs ang;
-    const long long *offsets;  // shard-local exclusive scan of the per-track counts (n_tracks + 1)
-    long long n_tracks;
+    const long long *offsets;      // shard-local exclusive scan of the per-track counts (n_tracks + 1)
     long long trk_begin, trk_end;  // tracks of this batch
     long long offset_base;         // offsets[trk_begin]
-    long long n_seg;               // segments of this batch
-    double *opx, *opy, *oqx, *oqy, *olen;
-    int *oelem;
-    double *vol;
-    double lmin;
-    int *verify_fail;
+    const double *olen;            // segment lengths of this batch
     int *status;   // per track
     double *tsum;  // per track: sum of segment lengths (atomics)
     double rtol;

@@ -74,7 +74,7 @@ struct WalkParams {
     int *verify_fail;
     const int *cancel;             // optimistic evaluation: set by the scan (ScanGuard) when the batch does not fit (nullptr: not used)
     double *tsum;                  // self-verifying pipelines: per-track sum of segment lengths
-    // single-walk pipeline (k_topo<2> + k_eval3): pool of record blocks
+    // single-walk pipeline (k_march + k_eval3): pool of record blocks
     int *pool;                     // pool_blocks * kRecBlock records
     int *pool_next;                // per block: the chunk's next block
     int *pool_cursor;              // next unclaimed block

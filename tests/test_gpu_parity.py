@@ -725,7 +725,7 @@ def test_self_verifying_pipelines_fall_back_to_sequential(pincell_model):
 
 
 def test_single_walk_pipeline_batches_and_pool_exhaustion():
-    """pipeline 3 (k_topo<2> + k_eval3): uid batches of the count walk when the record pool is small, sub-batches of the
+    """pipeline 3 (k_march + k_eval3): uid batches of the count walk when the record pool is small, sub-batches of the
     evaluation when the Segment columns are small, chunks longer than one pool block, and the fall-back to the hybrid pipeline
     when the pool runs out -- always the oracle's bits."""
     model = rt.synth.jittered_triangle_mesh(130, 130, seed=21)

@@ -1,4 +1,4 @@
-"""GPU experiment: the single-walk pipeline (3) against the hybrid one (0), k_march against k_topo<2>; chunk size / order sweeps."""
+"""GPU experiment: the single-walk pipeline (3) against the hybrid one (0); chunk size / order sweeps."""
 import os
 import sys
 
@@ -27,7 +27,6 @@ def run(label, flags=0, reps=4, chk=False, **opts):
     tg.set_option("chunk_segments", opts.get("chunk_segments", 128))
     tg.set_option("order_grid", opts.get("order_grid", 32))
     tg.set_option("pipeline", opts.get("pipeline", 0))
-    tg.set_option("march", opts.get("march", 1))
     best = None
     for _ in range(reps):
         tg.timer_start()
@@ -47,9 +46,6 @@ c3 = run("single-walk (3)", pipeline=3, chk=small)
 print("chunk stats:", tg.chunk_stats(), flush=True)
 if small:
     print("checksums equal:", c0 == c3, flush=True)
-c3t = run("single-walk (3), k_topo<2>", pipeline=3, march=0, chk=small)
-if small:
-    print("checksums equal:", c0 == c3t, flush=True)
 for cs in (64, 96, 192, 256):
     run(f"single-walk chunk={cs}", pipeline=3, chunk_segments=cs)
 for og in (0, 16, 64):
