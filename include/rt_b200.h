@@ -58,7 +58,9 @@ enum {
     RT_SEG_DEFAULT = 0,
     RT_SEG_LITERAL = 1,     /* disable the adjacency fast path: every step re-locates like src/track.jl:122 */
     RT_SEG_NO_VOLUMES = 2,  /* skip the fused fill_volumes accumulation */
-    RT_SEG_COUNT_ONLY = 4,  /* count + scan only (no segment buffers are written) */
+    RT_SEG_COUNT_ONLY = 4,  /* count + scan only (no segment buffers are written).  Without RT_SEG_NO_VOLUMES the volumes are
+                               those of exactly the segments a full call produces (max_iter cap and failing tracks included):
+                               they are summed by the count walk, which then runs one walker per track (as RT_SEG_NO_CHUNKS) */
     RT_SEG_NO_CHUNKS = 8,   /* one walker per track (no sub-track chunks) */
     RT_SEG_SEQUENTIAL = 16  /* sequential walk kernels only (the self-verifying pipelines fall back to them by themselves) */
 };

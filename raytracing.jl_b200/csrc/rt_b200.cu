@@ -1478,6 +1478,10 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
     ctx->vol_valid = false;
 
     if (ctx->mixed) flags |= RT_SEG_LITERAL | RT_SEG_NO_CHUNKS | RT_SEG_SEQUENTIAL;  // quadrilaterals: the reference's walk, step by step
+    // count-only with volumes: the volumes are summed by the count walk itself, where every chunk runs on its own (its own max_iter
+    // cap, blind to an error or the track end in an earlier chunk) and the fix-up cannot take back what a dropped chunk added.
+    // One walker per track stops exactly where the reference loop does.
+    if ((flags & RT_SEG_COUNT_ONLY) && want_vol) flags |= RT_SEG_NO_CHUNKS;
     if (!ctx->mixed && ctx->clear_tiny != tiny_step) {
         k_finalize_clear<<<blocks_for(m.n_cells, 128), 128, 0, st>>>(m, (CellRec *)ctx->b_cells.p, (HalfEdge *)ctx->b_he.p,
                                                                      (const float *)ctx->b_qual.p, (const float *)ctx->b_bdist.p,
