@@ -124,7 +124,9 @@ int rt_plan_shards(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x, con
  * larger values are rejected with RT_ERR_ARG instead of being clamped silently (the reference has no limit).
  * delta_eff: tg.azimuthal_quadrature.deltas (n_azim_2 values) or NULL with RT_SEG_NO_VOLUMES.
  * If the shard's segments exceed the context's segment capacity (rt_set_segment_capacity) the fill runs
- * in uid batches over a recycled buffer and `cb` (may be NULL) is called once per batch.
+ * in uid batches over a recycled buffer and `cb` (may be NULL) is called once per batch.  While `cb` runs, the batch it receives
+ * is the resident batch: rt_segments_download, rt_segments_download_compact, rt_optical_lengths and rt_correct_volumes may be called
+ * from inside it and act on that batch (outside a callback they need a completed rt_segmentize).  `cb` must not call rt_segmentize.
  * Returns RT_ERR_TRACK if any track failed (first_bad_uid, bad_status say which, like the reference's
  * first thrown error); the other tracks are still segmentized. */
 typedef struct rt_batch {
@@ -146,7 +148,7 @@ int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rtol, int32_t
 /* per-track segment counts / offsets / status of the shard after rt_segmentize (host copies) */
 int rt_segment_offsets(rt_ctx *ctx, int64_t *offsets /* n_shard+1 */, int32_t *status /* n_shard or NULL */);
 /* Segment(p, q, len, element) records (src/segment.jl:23-33) of the resident batch (the whole shard when
- * it fitted), SoA, in uid order then walk order. Any pointer may be NULL. */
+ * it fitted), SoA, in uid order then walk order. Any pointer may be NULL.  Also valid inside the batch callback of rt_segmentize. */
 int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double *qy, double *len,
                          int32_t *element);
 /* The same records over a thinner wire: 28 instead of 44 bytes per segment cross the bus.  Inside a track, `p` of a segment is
@@ -155,7 +157,8 @@ int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double
  * literal walk produced -- come as an unordered exception list (index into the resident batch, px, py).  The caller rebuilds
  * p[i] = q[i-1] and patches the listed positions: the result is bit-identical to rt_segments_download (tests/test_gpu_parity.py).
  * *n_exceptions receives the number of exceptions found; if it exceeds max_exceptions the call returns RT_ERR_NOMEM after the
- * columns have been copied, and can be repeated with larger buffers.  Column pointers may be NULL. */
+ * columns have been copied, and can be repeated with larger buffers.  Column pointers may be NULL.  Also valid inside the batch
+ * callback of rt_segmentize. */
 int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy, double *len, int32_t *element, int64_t max_exceptions,
                                  int64_t *exc_index, double *exc_px, double *exc_py, int64_t *n_exceptions);
 /* device-resident view of the resident batch for on-GPU consumers (transport sweeps) */
@@ -189,7 +192,7 @@ int rt_quadrature_device(rt_ctx *ctx, rt_quad_view *view, double *omega_host);
  * (src/segment.jl:27), which the reference leaves empty for the transport code.  sigma_t: HOST array, n_cells x n_groups
  * (element-major).  layout 0: tau[s*n_groups + g] (the reference's per-segment vectors, concatenated); layout 1:
  * tau[g*n_segments + s].  *d_tau receives the device buffer (owned by the context, valid until the next call);
- * tau_host, when not NULL, receives a copy. */
+ * tau_host, when not NULL, receives a copy.  Inside the batch callback of rt_segmentize: tau of the batch the callback received. */
 int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
                        double *tau_host);
 
@@ -200,8 +203,12 @@ int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int
  * src/trackgenerator.jl:388-397, flag `volume_correction` :48): after rt_segmentize + rt_volumes, every resident segment length
  * is multiplied by factor[element] = area[element] / volumes[element] (1 where no track crosses the element), so that the
  * traced volumes of the corrected lengths equal the exact areas.  p and q are left untouched.  `factors` / *d_factors: the
- * n_cells factors (host copy / device buffer; either may be NULL).  With batched segments call it from the batch callback of
- * a SECOND rt_segmentize (the factors need the volumes of all tracks). */
+ * n_cells factors (host copy / device buffer; either may be NULL).  With batched segments the factors need the volumes of all
+ * tracks: run one rt_segmentize with volumes (+ rt_volumes), then a SECOND rt_segmentize whose batch callback calls
+ * rt_correct_volumes for every batch.  Inside a callback the factors come from the normalised volumes of the previous completed
+ * rt_segmentize (RT_ERR_ARG if that call had none, e.g. RT_SEG_NO_VOLUMES); the correcting call itself may run with or without
+ * RT_SEG_NO_VOLUMES, and its own traced volumes are those of the lengths BEFORE correction (they are summed before the callback
+ * runs). */
 int rt_element_volumes(rt_ctx *ctx, double *areas, const double **d_areas);
 int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d_factors);
 

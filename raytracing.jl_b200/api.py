@@ -377,6 +377,8 @@ class TrackGenerator(TrackLayout):
         self._segments = None
         self._offsets = None
         self._resident = None
+        self._in_batch = False  # inside the on_batch of segmentize_: the batch it received is resident
+        self.volume_factors = None
         self.n_segments = 0
 
     def _mesh_arrays(self):
@@ -438,6 +440,10 @@ class TrackGenerator(TrackLayout):
         return ms.value
 
     # ---- lazily fetched device results -------------------------------------------------------------
+    def _resident_valid(self):
+        """a Segment batch is resident: after segmentize_, or inside its on_batch"""
+        return self._segmented or self._in_batch
+
     @property
     def track_data(self):
         if self._track_data is None:
@@ -480,7 +486,7 @@ class TrackGenerator(TrackLayout):
         """(uid_begin, uid_end, offset_base, n_segments) of the Segment batch the device holds (``rt_segments_device``), read
         when first needed after a segmentize_ and dropped whenever the segments are invalidated."""
         if self._resident is None:
-            if not self._segmented:
+            if not self._resident_valid():
                 raise RuntimeError("call segmentize_ first")
             view = _lib.rt_batch()
             _lib.check(self._ctx, _lib.lib().rt_segments_device(self._ctx, C.byref(view)))
@@ -495,8 +501,9 @@ class TrackGenerator(TrackLayout):
         ``compact=True`` moves 28 instead of 44 bytes per segment (rt_segments_download_compact): q, len, element plus the list of
         positions where p is not the preceding q; ``px`` / ``py`` are rebuilt on the host on first use (SegmentColumns).
         ``compact="q"`` leaves ``len`` on the device as well (20 bytes per segment): it is rebuilt as norm(p - q) with the same
-        IEEE operations (not after ``correct_volumes``, which rescales the resident lengths)."""
-        if not self._segmented:
+        IEEE operations (not after ``correct_volumes``, which rescales the resident lengths).
+        Inside ``on_batch`` of segmentize_ it copies the batch the callback received."""
+        if not self._resident_valid():
             raise RuntimeError("call segmentize_ first")
         L = _lib.lib()
         n = self.resident_batch()[3]
@@ -563,7 +570,8 @@ class TrackGenerator(TrackLayout):
 
     def optical_lengths(self, sigma_t, layout: int = 0, fetch: bool = True):
         """tau[s][g] = sigma_t[element(s)][g] * len(s) on the device for the resident segments (Segment.tau, src/segment.jl:27).
-        ``sigma_t``: (n_cells, n_groups).  Returns (numpy copy or None, DeviceColumn)."""
+        ``sigma_t``: (n_cells, n_groups).  Returns (numpy copy or None, DeviceColumn); the device buffer is reused by the next call.
+        Inside ``on_batch`` of segmentize_: tau of the batch the callback received."""
         sig = np.ascontiguousarray(sigma_t, dtype=np.float64)
         if sig.ndim != 2 or sig.shape[0] != self.mesh.num_cells:
             raise ValueError("sigma_t must have shape (n_cells, n_groups)")
@@ -584,7 +592,9 @@ class TrackGenerator(TrackLayout):
 
     def correct_volumes(self):
         """The reference's announced volume correction (src/trackgenerator.jl:388): resident segment lengths are scaled by
-        area[element] / volumes[element].  Returns the per-element factors; ``tg.segments`` is re-read afterwards."""
+        area[element] / volumes[element].  Returns the per-element factors; ``tg.segments`` is re-read afterwards.
+        Inside ``on_batch`` of segmentize_ it corrects the batch the callback received with the volumes of the segmentize_ before
+        the running one (see segmentize_)."""
         f = np.zeros(self.mesh.num_cells)
         _lib.check(self._ctx, _lib.lib().rt_correct_volumes(self._ctx, _lib.ptr(f), None))
         self._segments = None
@@ -713,23 +723,36 @@ class SegmentBatch:
 def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flags: int = 0, max_iter: int = MAX_ITER,
                 check: bool = True, fetch_volumes: bool = True, on_batch=None) -> TrackGenerator:
     """segmentize!(tg; k, rtol): count pass -> scan -> fill pass (+ fused fill_volumes) on the device.
-    ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits)."""
+    ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits).  Inside it
+    ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()`` and ``tg.correct_volumes()`` act
+    on that batch.
+
+    ``tg.volume_correction`` corrects the segments (``tg.volume_factors``) only when they all stay resident; otherwise, and with
+    ``on_batch`` or RT_SEG_COUNT_ONLY, ``tg.volume_factors`` is None.  Batched segments are corrected by a second segmentize_
+    whose ``on_batch`` calls ``tg.correct_volumes()`` for every batch: the factors come from the volumes of the call before it,
+    which must have run with volumes, and the correcting call may use RT_SEG_NO_VOLUMES (its own volumes would be those of the
+    lengths before correction)."""
     L = _lib.lib()
     cb = None
     if on_batch is not None:
         def _cb(bptr, _user):
+            tg._in_batch = True
             try:
                 on_batch(SegmentBatch(bptr.contents))
                 return 0
             except Exception as e:  # noqa: BLE001 -- reported through the return code
                 tg._batch_error = e
                 return 1
+            finally:
+                tg._in_batch = False
+                tg._segments = tg._resident = None  # (read again from the device if needed: a later batch replaces this one)
 
         cb = _lib.BATCH_CB(_cb)
     if not tg._traced:
         raise RuntimeError("Segmentation is intended after tracing. Please, call `trace!` first!")
     tg._segmented = False
     tg._segments = tg._offsets = tg._resident = None
+    tg.volume_factors = None
     nseg, bad_uid, bad_status = C.c_int64(0), C.c_int64(0), C.c_int32(0)
     delta = tg.azimuthal_quadrature.deltas
     rc = L.rt_segmentize(tg._ctx, tg.tiny_step, int(k), float(rtol), int(max_iter), _lib.ptr(delta), int(flags),
@@ -759,7 +782,8 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
             raise err  # (after the collective: the peers of this rank are not left inside ncclAllReduce)
         _lib.check(tg._ctx, rcv)
         # volume_correction = true: the reference's TODO (src/trackgenerator.jl:388), applied when every segment is resident
-        if tg.volume_correction and on_batch is None and not (flags & _lib.RT_SEG_COUNT_ONLY) and tg.info("segment_capacity") >= tg.n_segments:
+        # (the resident batch, not the allocated capacity: columns sized by an earlier call can be larger than the batches)
+        if tg.volume_correction and on_batch is None and not (flags & _lib.RT_SEG_COUNT_ONLY) and tg.resident_batch()[3] == tg.n_segments:
             tg.volume_factors = tg.correct_volumes()
     elif err is not None:
         raise err

@@ -159,6 +159,11 @@ struct rt_ctx {
     int *s_elem = nullptr;
     long long res_trk_begin = 0, res_trk_end = 0, res_off_base = 0, res_nseg = 0;  // resident batch (shard-local)
     bool vol_valid = false;
+    // Inside the batch callback of rt_segmentize the resident batch is valid although the call has not finished (`segmented` is
+    // false until it returns); the volume correction then uses the normalised volumes of the PREVIOUS call, which the current one
+    // overwrites only after its last callback (k_normalise, rt_volumes).
+    bool in_batch_cb = false;
+    bool prev_vol_valid = false;  // the call before the current rt_segmentize left volumes in b_voln
 
     double phase_ms[6] = {0, 0, 0, 0, 0, 0};
     double stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -931,6 +936,9 @@ static int read_verify(rt_ctx *ctx, bool *failed) {
     return RT_OK;
 }
 
+// the resident batch may be read: after a completed rt_segmentize, or from inside its batch callback
+static bool resident_valid(const rt_ctx *ctx) { return ctx && (ctx->segmented || ctx->in_batch_cb); }
+
 // the resident batch (rt_segments_device) to the caller's batch callback, if there is one
 static int deliver_batch(rt_ctx *ctx, const Attempt &a) {
     if (!a.cb) return RT_OK;
@@ -938,7 +946,10 @@ static int deliver_batch(rt_ctx *ctx, const Attempt &a) {
     int rc = rt_segments_device(ctx, &bt);
     if (rc) return rc;
     bt.attempt = a.index;
-    if (a.cb(&bt, a.cb_user)) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
+    ctx->in_batch_cb = true;  // (the resident-batch calls accept the batch while the callback runs)
+    const int stop = a.cb(&bt, a.cb_user);
+    ctx->in_batch_cb = false;
+    if (stop) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
     return RT_OK;
 }
 
@@ -1459,6 +1470,9 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
                              uint32_t flags, rt_batch_cb cb, void *cb_user, int64_t *n_segments_total, int64_t *first_bad_uid,
                              int32_t *bad_status) {
     if (!ctx) return RT_ERR_ARG;
+    if (ctx->in_batch_cb) return fail(ctx, RT_ERR_ARG, "rt_segmentize: called from inside a batch callback");
+    // (what rt_correct_volumes may use inside this call's batch callback)
+    ctx->prev_vol_valid = ctx->segmented && ctx->vol_valid && ctx->b_voln.p;
     // (whatever goes wrong below, the results of an earlier call are no longer "the last segmentize!": rt_volumes must see that)
     ctx->segmented = false;
     ctx->vol_valid = false;
@@ -1559,7 +1573,7 @@ extern "C" int rt_segment_offsets(rt_ctx *ctx, int64_t *offsets, int32_t *status
 }
 
 extern "C" int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double *qy, double *len, int32_t *element) {
-    if (!ctx || !ctx->segmented) return fail(ctx, RT_ERR_ARG, "rt_segments_download: call rt_segmentize first");
+    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_segments_download: call rt_segmentize first");
     CK(cudaSetDevice(ctx->device));
     size_t n = (size_t)ctx->res_nseg;
     if (n == 0) return RT_OK;
@@ -1576,7 +1590,7 @@ extern "C" int rt_segments_download(rt_ctx *ctx, double *px, double *py, double 
 
 extern "C" int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy, double *len, int32_t *element, int64_t max_exceptions,
                                             int64_t *exc_index, double *exc_px, double *exc_py, int64_t *n_exceptions) {
-    if (!ctx || !ctx->segmented) return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: call rt_segmentize first");
+    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: call rt_segmentize first");
     if (max_exceptions < 0 || !n_exceptions || (max_exceptions > 0 && (!exc_index || !exc_px || !exc_py)))
         return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: bad exception buffers");
     CK(cudaSetDevice(ctx->device));
@@ -1691,7 +1705,7 @@ extern "C" int rt_quadrature_device(rt_ctx *ctx, rt_quad_view *v, double *omega_
 extern "C" int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
                                   double *tau_host) {
     if (!ctx || n_groups < 1 || !sigma_t || (layout != 0 && layout != 1)) return fail(ctx, RT_ERR_ARG, "rt_optical_lengths: bad arguments");
-    if (!ctx->segmented) return fail(ctx, RT_ERR_ARG, "rt_optical_lengths: call rt_segmentize first");
+    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_optical_lengths: call rt_segmentize first");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const long long n_seg = ctx->res_nseg;
@@ -1741,8 +1755,12 @@ extern "C" int rt_element_volumes(rt_ctx *ctx, double *areas, const double **d_a
 }
 
 extern "C" int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d_factors) {
-    if (!ctx || !ctx->segmented || !ctx->vol_valid || !ctx->b_voln.p)
-        return fail(ctx, RT_ERR_ARG, "rt_correct_volumes: run rt_segmentize with volumes enabled and rt_volumes first");
+    // inside a batch callback: the volumes of the call before the running one (its own are summed only as far as its batches go)
+    const bool have_vol = ctx && (ctx->in_batch_cb ? ctx->prev_vol_valid : ctx->segmented && ctx->vol_valid && ctx->b_voln.p);
+    if (!have_vol)
+        return fail(ctx, RT_ERR_ARG, ctx && ctx->in_batch_cb
+                                         ? "rt_correct_volumes: inside a batch callback it needs an earlier rt_segmentize with volumes"
+                                         : "rt_correct_volumes: run rt_segmentize with volumes enabled and rt_volumes first");
     CK(cudaSetDevice(ctx->device));
     int rc = ensure_areas(ctx);
     if (rc) return rc;
