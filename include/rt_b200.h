@@ -236,7 +236,9 @@ int rt_stats(rt_ctx *ctx, double stats[8]);
 /* named scalars: "verify_fallbacks", "n_units", "segment_capacity", "count_batches"
  * (uid batches of the single-walk pipeline's count walk) of the last rt_segmentize; "optimistic_cancels" (calls of this context
  * whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
- * repeated); "rho", "band_cost" (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths */
+ * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose
+ * rt_segmentize failed: the ranks of a communicator that call rt_volumes as documented below agree on it); "rho", "band_cost"
+ * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths */
 int rt_info(rt_ctx *ctx, const char *key, double *value);
 /* CUDA-event time (ms) of the last call's device work, by phase: 0 upload+prep, 1 trace, 2 count,
  * 3 scan, 4 fill, 5 volumes(+allreduce) */

@@ -725,7 +725,9 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
     """segmentize!(tg; k, rtol): count pass -> scan -> fill pass (+ fused fill_volumes) on the device.
     ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits).  Inside it
     ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()`` and ``tg.correct_volumes()`` act
-    on that batch.
+    on that batch.  An exception raised by ``on_batch`` stops the call and is re-raised here -- on a TrackGenerator with a
+    communicator only after this rank has joined the call's all-reduce of the volumes (as after any other failure), so that its
+    peers are not left waiting inside it.
 
     ``tg.volume_correction`` corrects the segments (``tg.volume_factors``) only when they all stay resident; otherwise, and with
     ``on_batch`` or RT_SEG_COUNT_ONLY, ``tg.volume_factors`` is None.  Batched segments are corrected by a second segmentize_
@@ -758,18 +760,19 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
     rc = L.rt_segmentize(tg._ctx, tg.tiny_step, int(k), float(rtol), int(max_iter), _lib.ptr(delta), int(flags),
                          C.cast(cb, C.c_void_p) if cb is not None else None, None,
                          C.byref(nseg), C.byref(bad_uid), C.byref(bad_status))
-    if on_batch is not None and getattr(tg, "_batch_error", None) is not None:
-        err, tg._batch_error = tg._batch_error, None
-        raise err
+    batch_error, tg._batch_error = getattr(tg, "_batch_error", None), None
     tg.n_segments = int(nseg.value)
     tg.first_bad_uid, tg.bad_status = int(bad_uid.value), int(bad_status.value)
     want_vol = not (flags & _lib.RT_SEG_NO_VOLUMES)
     if rc not in (0, -8):
-        # every rank of a communicator has to enter the all-reduce once per segmentize! -- a rank that failed joins it with a
-        # zero contribution and the failed-rank flag (rt_volumes), so that its peers are not left waiting; then the error is raised
+        # every rank of a communicator has to enter the all-reduce once per segmentize! -- a rank that failed (also because its
+        # on_batch raised: the call then stops with RT_ERR_ARG) joins it with a zero contribution and the failed-rank flag
+        # (rt_volumes), so that its peers are not left waiting; then the error is raised, the exception of on_batch if there is one
         msg = L.rt_last_error(tg._ctx)
         if want_vol and getattr(tg, "_has_comm", False):
             L.rt_volumes(tg._ctx, None)
+        if batch_error is not None:
+            raise batch_error
         raise _lib.RTError(rc, msg.decode() if msg else "")
     tg._segmented = True
     err = None

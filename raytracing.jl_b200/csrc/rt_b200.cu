@@ -183,6 +183,7 @@ struct rt_ctx {
     bool ev_vol_used[2] = {false, false};
     bool voln_done = false;                                 // b_voln already holds the normalised volumes of the last rt_segmentize (no communicator)
     int voln_ready = -1;                                    // index of the event that marks b_voln complete (-1: main stream)
+    long long collectives = 0;                              // ncclAllReduce calls issued by rt_volumes, failed-rank joins included (info)
 };
 
 static inline unsigned long long *d_counters(rt_ctx *c) { return (unsigned long long *)c->b_ctrl.p; }
@@ -1862,6 +1863,7 @@ extern "C" int rt_volumes(rt_ctx *ctx, double *volumes) {
         CK(cudaEventRecord(ctx->pev[5][0], cs));
         ncclResult_t r = ctx->nccl.AllReduce(src, ctx->b_voln.p, (size_t)nc + 1, ncclFloat64, ncclSum, ctx->comm, cs);
         if (r != 0) return fail(ctx, RT_ERR_NCCL, "ncclAllReduce: %s", ctx->nccl.GetErrorString ? ctx->nccl.GetErrorString(r) : "?");
+        ctx->collectives += 1;
         k_normalise<<<blocks_for(nc, 256), 256, 0, cs>>>((const double *)ctx->b_voln.p, (double *)ctx->b_voln.p, nc, (double)ctx->n2);
         CK(cudaGetLastError());
         CK(cudaEventRecord(ctx->pev[5][1], cs));
@@ -1981,6 +1983,8 @@ extern "C" int rt_info(rt_ctx *ctx, const char *key, double *value) {
         *value = (double)ctx->count_batches;
     else if (k == "optimistic_cancels")
         *value = (double)ctx->optimistic_cancels;
+    else if (k == "collectives")
+        *value = (double)ctx->collectives;
     else
         return fail(ctx, RT_ERR_ARG, "rt_info: unknown key %s", key);
     return RT_OK;
