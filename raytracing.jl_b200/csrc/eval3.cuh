@@ -19,7 +19,7 @@
 // gathers ONE 32-byte sector (the EdgeRec), executes ~45 FP64 instructions (one shared reciprocal, one square root) and
 // writes 44 bytes: the HBM write stream of the Segment columns is its roofline.
 #pragma once
-#include "topo.cuh"
+#include "walk.cuh"
 
 namespace rt {
 

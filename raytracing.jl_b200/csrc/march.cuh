@@ -1,10 +1,17 @@
-// march.cuh -- k_march: the count+record walk of the single-walk pipeline with a REGISTER-RESIDENT hot loop.
+// march.cuh -- k_march: the sign-test walk of the half-edge graph, with a REGISTER-RESIDENT hot loop.
 //
-// Same walk and same decisions as k_topo, the count walk of the hybrid pipeline (topo.cuh; the sign-test transitions of the
-// half-edge graph with the literal walk of the reference, src/track.jl:106-178, for everything the clearance test does not
-// cover), plus one record per accepted cell.  What differs is how the code is laid out for the register allocator: in k_topo
-// the literal path (point location, intersections(), 100+ live values) is inlined next to the fast transition, ptxas runs out
-// of the 64 registers that 8 resident blocks allow and keeps the walker's state in local memory -- 17 local loads/stores per fast transition (profiles/r1_q).  Here
+// A Segment(p, q, l, element) depends only on (track, cell): intersections() uses the track's infinite line
+// (src/intersection.jl:60).  So the serial part of _segmentize_track! (src/track.jl:106-178) is only the ORDER in which cells
+// are accepted; the geometry of every accepted cell can be evaluated independently afterwards.  k_march walks each chunk
+// deciding every transition from the SIGNS of the signed distances of the cell's vertices from the track line (two
+// multiply-adds per step, no division, no square root), under the same clearance test as the sequential fast path (walk.cuh);
+// everything that test does not cover runs the literal walk of the reference, exactly as in walk.cuh.  It counts the accepted
+// cells of every chunk and, when it is given a record pool (single-walk pipeline), records each of them for k_eval3; without a
+// pool (the count pass of the hybrid pipeline) it only counts.
+//
+// The code is laid out for the register allocator: with the literal path (point location, intersections(), 100+ live values)
+// inlined next to the fast transition, ptxas runs out of the 64 registers that 8 resident blocks allow and keeps the walker's
+// state in local memory -- 17 local loads/stores per fast transition (profiles/r1_q).  Here
 //   * the hot loop touches only scalars that fit the register file: track line (a, b, c, g), signed distances of the entry
 //     edge's end points (s1, s2), the encoded half-edge to enter next, clearances, counters;
 //   * everything the slow path needs beyond that lives in a MarchState record whose address is passed to ONE out-of-line
@@ -12,7 +19,7 @@
 //     across the call and the callee's register appetite cannot leak into the loop;
 //   * the last accepted cell / exit edge are recovered from the last record instead of being carried.
 #pragma once
-#include "topo.cuh"
+#include "walk.cuh"
 
 namespace rt {
 
@@ -52,6 +59,21 @@ struct MarchState {
     unsigned lit_iters, nn_q, knn_q;
     unsigned s_rec;  // shared-space address of this thread's column of the staging tile (stride kMarchThreads words)
 };
+
+// (the pool records are read back by k_eval3 within the same call: no eviction hint, they should stay in L2 if they fit)
+__device__ __forceinline__ void stg256_plain_i(void *p, const int *v) {
+    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]),
+                 "r"(v[5]), "r"(v[6]), "r"(v[7])
+                 : "memory");
+}
+
+// exit point of cell `c` through its local edge k: the reference's intersection() with that edge's line
+__device__ __forceinline__ P2 exit_point(const DevMesh &m, const Line &trk, int c, int k) {
+    const EdgeRec e = m.edges[3 * c + k];
+    P2 X;
+    intersection(trk, Line{e.a, e.b, e.c}, X);
+    return X;
+}
 
 // MODE_RETRY: the hot loop gave up on the transition through `enc`; march_slow re-examines it exactly before going literal
 enum { MODE_RETRY = 3 };
@@ -136,7 +158,7 @@ __device__ __forceinline__ bool march_exact(const WalkParams &P, double ta, doub
 }
 
 // The slow side of the walk, out of line: (1) the transition the hot loop could not decide with the cheap filter is re-examined
-// with the exact chord (same tests as k_topo); (2) if it is not a fast transition, the literal walk of the reference runs until
+// with the exact chord (march_exact); (2) if it is not a fast transition, the literal walk of the reference runs until
 // it pushes one segment, and the fast path is re-armed from there.
 __device__ __noinline__ void march_slow(const WalkParams &P, MarchState &s) {
     const DevMesh &m = P.m;
@@ -232,7 +254,7 @@ __device__ __noinline__ void march_init(const WalkParams &P, MarchState &s, int 
     s.stop_cell = -1;
     s.limit = P.max_iter;
     s.pb = (int)(s.cidx - P.pool_slot_base);
-    s.recording = 1;
+    s.recording = P.pool != nullptr;  // (the count pass of the hybrid pipeline records nothing)
     s.ta = s.tb = s.tc = s.g = s.ang_thr = s.s1 = s.s2 = s.qx = s.qy = 0.0;
     s.clearA = INFINITY;
     s.f = 0;
@@ -350,22 +372,15 @@ __global__ void __launch_bounds__(kMarchThreads, RT_MARCH_MIN_BLOCKS) k_march(co
             const int nenc = exit1 ? __double2loint(rw0) : __double2hiint(rw0);
             const float clearf = __int_as_float(__double2loint(rw1));
             const float clear2 = __int_as_float(__double2hiint(rw1));
-#ifndef RT_MARCH_LATE_LOAD
             if (nenc >= 0) ldg256_keep(m.he + (nenc >> 3), pol_keep, rax, ray, rw0, rw1);  // (speculative: the tests below may still say no)
-#endif
             const float clearB = fabsf(clearf);
             const double thr = g * (double)fmaxf(clearA, clearB);
             const double ks = opp1 ? s1 : s2;  // ... which is the only vertex on its side of the track line
             // clearance test + cheap filter (DESIGN.md): the geometric fast-path conditions hold without evaluating the chord;
             // transitions it cannot decide (and every cell of the bounding-box band) are re-examined exactly by march_slow -- not
             // here: any call or any larger body inside this loop makes ptxas keep the walker's state in local memory
-#ifdef RT_MARCH_BRANCHY
-            const bool accept = (fabs(sa) >= thr) && (fabs(s1) >= thr) && (fabs(s2) >= thr) && cheap_ok && (clearf >= 0.0f) &&
-                                (fabs(ks) >= g * (double)clear2) && (fabs(ks) + fabs(sa) >= ang_thr) && (fabs(s1) + fabs(s2) >= ang_thr);
-#else
             const bool accept = (fabs(sa) >= thr) & (fabs(s1) >= thr) & (fabs(s2) >= thr) & cheap_ok & (clearf >= 0.0f) &
                                 (fabs(ks) >= g * (double)clear2) & (fabs(ks) + fabs(sa) >= ang_thr) & (fabs(s1) + fabs(s2) >= ang_thr);
-#endif
             if (!accept) {
                 mode = MODE_RETRY;  // (the record in flight belongs to a half-edge that is not entered: march_slow re-arms)
                 continue;
@@ -380,9 +395,6 @@ __global__ void __launch_bounds__(kMarchThreads, RT_MARCH_MIN_BLOCKS) k_march(co
             // (cell of h == stop_cell) without dividing: h in [3*stop_cell, 3*stop_cell + 2]; stop_cell = -1: never
             const bool at_stop = (unsigned)(h - 3 * stop_cell) < 3u;
             march_push(P, at_stop, last_rec, nseg, pb, recording, mode, endcode, limit, my_rec);
-#ifdef RT_MARCH_LATE_LOAD
-            if (mode == MODE_FAST && enc >= 0) ldg256_keep(m.he + (enc >> 3), pol_keep, rax, ray, rw0, rw1);
-#endif
         }
         // ------------------------------------------------------------------ SLOW phase (out of line)
         if (mode == MODE_SLOW || mode == MODE_RETRY) {

@@ -291,7 +291,7 @@ __global__ void k_finalize_clear(DevMesh m, CellRec *cells, HalfEdge *he, const 
     else if (boundary)
         cf = -cf;
     cells[c].clear = cf;
-    // chord >= d * sin(gamma) >= d * sigma for a lone vertex at distance d from the track line (topo.cuh)
+    // chord >= d * sin(gamma) >= d * sigma for a lone vertex at distance d from the track line (the cheap filter of k_march, march.cuh)
     double c2 = lmin * 1.001 * (double)qual[c];
     float c2f = (float)c2;
     if (!(c2f >= c2)) c2f = nextafterf(c2f, INFINITY);

@@ -17,7 +17,6 @@
 #include "sweep.cuh"
 #include "eval3.cuh"
 #include "march.cuh"
-#include "topo.cuh"
 #include "trace.cuh"
 
 using namespace rt;
@@ -135,8 +134,8 @@ struct rt_ctx {
     double opt_band_div = 8.0;
     long long opt_pool_slots = 0;      // test hook: at most this many chunk slots per count batch (0: as many as fit)
     double opt_pool_extra = 1.25;      // spare pool blocks, as a multiple of (expected segments / kRecBlock)
-    int opt_pipeline = 3;              // 3: single walk (k_march counts AND records, k_eval3 evaluates) [default]; 0: hybrid (sign-test count walk +
-                                       // geometric fill walk), 1: sequential (walk.cuh only); 3 falls back to 0 (pool exhausted) or 1, 0 falls back to 1
+    int opt_pipeline = 3;              // 3: single walk (k_march counts AND records, k_eval3 evaluates) [default]; 0: hybrid (k_march without records
+                                       // counts, geometric fill walk), 1: sequential (walk.cuh only); 3 falls back to 0 (pool exhausted) or 1, 0 falls back to 1
     int verify_fallbacks = 0;
     int opt_debug_verify_fail = 0;     // test hook: make the verification of the two-stage pipeline fail
     double tau_ms = 0.0;
@@ -1277,9 +1276,10 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
 
 // ---- two-pass pipelines: count -> scan -> fill (possibly in uid batches over a recycled buffer)
 //   mode 1 (sequential): k_walk<false> counts, k_walk<true> fills (walk.cuh);
-//   mode 0 (hybrid):     k_topo counts by sign tests (topo.cuh), k_walk<true> fills and re-derives the same decisions from the
-//                        exact geometry, k_track_status runs the length check (src/track.jl:171-175) after the fill.  A fill
-//                        that disagrees with the count fails the verification: Next::Sequential.
+//   mode 0 (hybrid):     k_march counts by sign tests (march.cuh; no record pool, so it records nothing), k_walk<true> fills
+//                        and re-derives the same decisions from the exact geometry, k_track_status runs the length check
+//                        (src/track.jl:171-175) after the fill.  A fill that disagrees with the count fails the verification:
+//                        Next::Sequential.
 static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool hybrid, Attempt &a) {
     cudaStream_t st = ctx->stream;
     const long long n = ctx->n_shard;
@@ -1291,7 +1291,7 @@ static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool 
         const long long n_units = P.ch.n_units;
         k_seed<<<blocks_for(n_units * 32, 128), 128, 0, st>>>(P);
         if (hybrid) {
-            k_topo<<<blocks_for(n_units * 32, kTopoThreads), kTopoThreads, 0, st>>>(P);
+            k_march<<<blocks_for(n_units * 32, kMarchThreads), kMarchThreads, 0, st>>>(P);
         } else {
             P.vol = (a.want_vol && (flags & RT_SEG_COUNT_ONLY)) ? ctx->vol_acc : nullptr;
             if (ctx->mixed)

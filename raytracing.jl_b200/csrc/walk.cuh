@@ -728,7 +728,7 @@ __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const
         P.ch.sum[cidx] = sum;
         P.ch.endcode[cidx] = active ? (endcode | (status << 8)) : (END_HANDOFF | (0 << 8));
     }
-    if (FILL && active && P.tsum) {  // hybrid pipeline: the counts came from the sign-test walk (topo.cuh)
+    if (FILL && active && P.tsum) {  // hybrid pipeline: the counts came from the sign-test walk (k_march, march.cuh)
         atomicAdd(&P.tsum[t], sum);
         if (nseg != limit) atomicExch(P.verify_fail, 1);  // this walk ended before producing the counted segments
     }
@@ -783,6 +783,47 @@ __global__ void k_fixup_tracks(const __grid_constant__ WalkParams P) {
     if (P.rtol >= 0.0 && status == 0 && (truncated || !isapprox(P.t.len[t], sum, 0.0, P.rtol))) status = 2;
     P.count[t] = total;
     P.status[t] = status;
+}
+
+// ---- per-track length check after the fill --------------------------------------------------------------------------------
+struct EvalParams {
+    TrackSoA t;
+    const long long *offsets;      // shard-local exclusive scan of the per-track counts (n_tracks + 1)
+    long long trk_begin, trk_end;  // tracks of this batch
+    long long offset_base;         // offsets[trk_begin]
+    const double *olen;            // segment lengths of this batch
+    int *status;   // per track
+    double *tsum;  // per track: sum of segment lengths (atomics)
+    double rtol;
+    const int *cancel;  // optimistic evaluation cancelled (scan.cuh ScanGuard): nothing to check
+    unsigned long long *bad;  // min over the failing tracks of (track << 4 | status), or nullptr
+};
+
+// isapprox(track.l, sum(l.(segments)); rtol)  src/track.jl:171-175.  The atomically accumulated sum differs from the
+// reference's left-to-right sum by at most ~n*eps relative; only when the comparison is that close to its threshold is the
+// track re-summed left to right from the segment records.
+__global__ void k_track_status(const __grid_constant__ EvalParams P) {
+    long long t = P.trk_begin + blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (t >= P.trk_end) return;
+    if (P.cancel && *P.cancel) return;
+    const int st0 = P.status[t];
+    if (st0 != 0) {  // (failed in the walk)
+        if (P.bad) atomicMin(P.bad, ((unsigned long long)t << 4) | (unsigned long long)(st0 & 15));
+        return;
+    }
+    const double len = P.t.len[t];
+    double sum = P.tsum[t];
+    const double tol = P.rtol * fmax(fabs(len), fabs(sum));
+    const double slack = 1e-10 * fmax(fabs(len), fabs(sum));
+    if (fabs(fabs(len - sum) - tol) <= slack) {
+        long long b = P.offsets[t] - P.offset_base, e = P.offsets[t + 1] - P.offset_base;
+        sum = 0.0;
+        for (long long s = b; s < e; ++s) sum += P.olen[s];
+    }
+    if (!isapprox(len, sum, 0.0, P.rtol)) {
+        P.status[t] = 2;
+        if (P.bad) atomicMin(P.bad, ((unsigned long long)t << 4) | 2ull);
+    }
 }
 
 }  // namespace rt

@@ -166,11 +166,16 @@ def test_jittered_mesh_matches_oracle(seed, n, n_azim, delta):
     otg, tg = run_both(model, n_azim, delta, flags=SEQ, chunk_segments=5)  # the sequential kernels on the same input
     assert_segments_equal(otg, tg)
     assert_volumes_close(otg, tg)
+    walk_counters = ("fast_transitions", "literal_iterations", "nn_queries", "knn_queries")
+    counters = {(3, None): [st[c] for c in walk_counters]}
     for pipeline, chunk in ((0, 5), (0, None), (3, 5), (3, 600)):  # hybrid pipeline; single walk with tiny / with multi-block chunks
         otg, tg = run_both(model, n_azim, delta, chunk_segments=chunk, pipeline=pipeline)
         assert_segments_equal(otg, tg)
         assert_volumes_close(otg, tg)
         assert tg.info("verify_fallbacks") == 0
+        counters[pipeline, chunk] = [tg.stats()[c] for c in walk_counters]
+    for chunk in (5, None):  # the count pass of the hybrid pipeline is the single walk's walk: same decisions, same counters
+        assert counters[0, chunk] == counters[3, chunk]
 
 
 def test_offset_domain_and_rectangle():
