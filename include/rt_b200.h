@@ -212,6 +212,17 @@ int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int
 int rt_element_volumes(rt_ctx *ctx, double *areas, const double **d_areas);
 int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d_factors);
 
+/* ---- point location: find_element(mesh, x, k) (src/mesh.jl:103-146) outside the walk ---------------------------------------
+ * For n points: xy = x0,y0,x1,y1,... (HOST), element[i] = 1-based cell or -1 (no cell passes the tolerant test, like the reference).
+ * The answer is the walk's own find_element: the first passing cell around the nearest node in Gridap's order, then around the k
+ * nearest other nodes.  Needs rt_mesh_upload only.  1 <= k <= RT_MAX_K.  Non-finite coordinates are rejected (RT_ERR_ARG, the
+ * message names the first such point).  Triangle and mixed meshes.  Nearest-node distance ties go to the lowest node id (the
+ * oracle's choice; NearestNeighbors.jl documents none).  n = 0 launches nothing.  element (may be NULL) receives a host copy;
+ * *d_element (may be NULL) the device buffer (owned by the context, valid until the next call).  Runs on the context's stream and
+ * leaves what rt_segmentize produced untouched (resident batch, offsets, volumes, rt_stats, rt_phase_ms): it may also be called
+ * inside the batch callback of rt_segmentize.  rt_info "locate_knn" / "locate_ms" describe the last call. */
+int rt_find_elements(rt_ctx *ctx, int64_t n, const double *xy, int32_t k, int32_t *element, const int32_t **d_element);
+
 /* ---- volumes: replaces the tail of fill_volumes (src/trackgenerator.jl:378-386) -----------------------
  * volumes[e] = (sum over this context's segments of delta_eff[azim]*len) / n_azim_2, after an NCCL
  * all-reduce across the communicator set up with rt_comm_init (skipped when there is none).  With a communicator the
@@ -238,7 +249,8 @@ int rt_stats(rt_ctx *ctx, double stats[8]);
  * whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
  * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose
  * rt_segmentize failed: the ranks of a communicator that call rt_volumes as documented below agree on it); "rho", "band_cost"
- * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths */
+ * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths; "locate_knn" (points that entered the k-nearest-node
+ * branch of find_element) and "locate_ms" (k_find_elements alone) of the last rt_find_elements */
 int rt_info(rt_ctx *ctx, const char *key, double *value);
 /* CUDA-event time (ms) of the last call's device work, by phase: 0 upload+prep, 1 trace, 2 count,
  * 3 scan, 4 fill, 5 volumes(+allreduce) */

@@ -278,3 +278,32 @@ function b200_mesh_upload_device_ingest(ctx::Ptr{Cvoid}, model)
     _b200_check(ctx, ccall((:rt_mesh_bbox, LIBRT_B200), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}), ctx, lo, hi))
     return Point2D(lo[1], lo[2]), Point2D(hi[1], hi[2])
 end
+
+# ---- point location outside the walk (include/rt_b200.h: rt_find_elements) ------------------------------------------------
+
+"""
+    b200_find_elements(t::TrackGenerator, xs::AbstractVector; k=2) -> Vector{Int32}
+
+`find_element(t.mesh, x, k)` (src/mesh.jl:103-146) for every point `x` of `xs` (anything indexable as `x[1]`, `x[2]`: `Point2D`,
+`VectorValue`, a 2-vector) in one device call, instead of one KD-tree query per point: the cell of each point, or -1 like the
+reference when no cell passes.  Nearest-node distance ties go to the lowest node id.  Needs only the uploaded mesh (no `trace!`).
+"""
+function b200_find_elements(t::TrackGenerator, xs::AbstractVector; k::Integer=2)
+    ctx = _b200_context(t)
+    n = length(xs)
+    xy = Vector{Float64}(undef, 2n)
+    for (i, x) in enumerate(xs)
+        xy[2i-1] = x[1]; xy[2i] = x[2]
+    end
+    element = Vector{Int32}(undef, n)
+    _b200_check(ctx, ccall((:rt_find_elements, LIBRT_B200), Cint,
+        (Ptr{Cvoid}, Int64, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Ptr{Int32}}), ctx, Int64(n), xy, Int32(k), element, C_NULL))
+    return element
+end
+
+"""
+    b200_find_element(t::TrackGenerator, x; k=2) -> Int32
+
+`find_element(t.mesh, x, k)` (src/mesh.jl:103-146) for one point, with the reference's return value.
+"""
+b200_find_element(t::TrackGenerator, x; k::Integer=2) = b200_find_elements(t, [x]; k=k)[1]

@@ -97,6 +97,7 @@ SYMBOLS = {
     "rt_optical_lengths": (C.c_int, [_vp, C.c_int32, _f64, C.c_int32, C.POINTER(_vp), _vp]),
     "rt_element_volumes": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
     "rt_correct_volumes": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
+    "rt_find_elements": (C.c_int, [_vp, C.c_int64, _f64, C.c_int32, _vp, C.POINTER(_vp)]),
     "rt_comm_unique_id": (C.c_int, [_vp, C.c_char_p]),
     "rt_comm_init": (C.c_int, [_vp, C.c_int32, C.c_int32, C.c_char_p]),
     "rt_stats": (C.c_int, [_vp, _f64]),

@@ -584,6 +584,20 @@ class TrackGenerator(TrackLayout):
         _lib.check(self._ctx, _lib.lib().rt_optical_lengths(self._ctx, G, sig.reshape(-1), int(layout), C.byref(d), _lib.ptr(host)))
         return host, DeviceColumn(d.value, n * G, "<f8")
 
+    def find_elements(self, xy, k: int = 2, fetch: bool = True):
+        """find_element(mesh, x, k) (src/mesh.jl:103-146) for every row of ``xy`` (n, 2) in one device call (rt_find_elements): the
+        1-based cell of each point, -1 where no cell passes.  Returns (int32 ids or None, DeviceColumn); the device buffer is reused
+        by the next call.  Needs only the uploaded mesh; it leaves the segments, volumes and stats of segmentize_ as they are and may
+        be called inside its ``on_batch``."""
+        pts = np.ascontiguousarray(xy, dtype=np.float64)
+        if pts.ndim != 2 or pts.shape[1] != 2:
+            raise ValueError("xy must have shape (n, 2)")
+        n = pts.shape[0]
+        ids = np.empty(n, np.int32) if fetch else None
+        d = C.c_void_p()
+        _lib.check(self._ctx, _lib.lib().rt_find_elements(self._ctx, n, pts.reshape(-1), int(k), _lib.ptr(ids), C.byref(d)))
+        return ids, DeviceColumn(d.value, n, "<i4")
+
     def element_volumes(self):
         """element_volume of every cell (src/trackgenerator.jl:402-411: the `volumes2` the reference computes and discards)."""
         a = np.zeros(self.mesh.num_cells)
@@ -648,6 +662,13 @@ class TrackGenerator(TrackLayout):
                 "  Effective azimuthal spacings: %s\n  Total tracks: %d\n  Correct volumes: %s" %
                 (nazim2(aq), np.round(np.degrees(aq.phis), 2), np.round(aq.deltas, 3), self.n_total_tracks,
                  str(self.volume_correction).lower()))
+
+
+def find_element(tg: TrackGenerator, x, k: int = 2) -> int:
+    """find_element(mesh, x, k=2) (src/mesh.jl:103-146) for one point ``x`` = (x, y) on the mesh of ``tg``: the 1-based cell, or -1
+    like the reference when no cell passes.  For many points use ``tg.find_elements``."""
+    ids, _ = tg.find_elements(np.asarray(x, dtype=np.float64).reshape(1, 2), k)
+    return int(ids[0])
 
 
 def _angle_tables(tg: TrackLayout):

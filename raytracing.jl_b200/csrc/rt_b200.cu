@@ -7,6 +7,7 @@
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -18,6 +19,7 @@
 #include "eval3.cuh"
 #include "march.cuh"
 #include "trace.cuh"
+#include "locate.cuh"
 
 using namespace rt;
 
@@ -139,7 +141,9 @@ struct rt_ctx {
     int verify_fallbacks = 0;
     int opt_debug_verify_fail = 0;     // test hook: make the verification of the two-stage pipeline fail
     double tau_ms = 0.0;
-    cudaEvent_t ev2[2] = {nullptr, nullptr};
+    cudaEvent_t ev2[2] = {nullptr, nullptr};  // kernel stopwatch of the synchronous exports (rt_optical_lengths, rt_find_elements)
+    DevBuf b_loc_xy, b_loc_elem, b_loc_knn;   // rt_find_elements: points, element ids, k-nearest branch counter
+    double locate_knn = 0.0, locate_ms = 0.0;
     int opt_order_grid = 32;           // G x G tiles (0: identity order)
     const int *order_eval = nullptr;   // execution order of the evaluation (plain Morton order)
     int opt_order_classes = 3;         // duration bins of the walk's launch order, longest units first (walk.cuh k_unit_keys); 0: spatial order
@@ -288,7 +292,8 @@ extern "C" void rt_destroy(rt_ctx *ctx) {
                      &ctx->b_scratch, &ctx->b_gcounts,   &ctx->b_gcursor,   &ctx->b_cell_bin,
                      &ctx->b_omega,   &ctx->b_sigma,     &ctx->b_tau,
                      &ctx->b_pool,    &ctx->b_pool_next, &ctx->b_pool_cursor,
-                     &ctx->b_area,    &ctx->b_factor,    &ctx->b_layout,    &ctx->b_vol_alt,  &ctx->b_exc};
+                     &ctx->b_area,    &ctx->b_factor,    &ctx->b_layout,    &ctx->b_vol_alt,  &ctx->b_exc,
+                     &ctx->b_loc_xy,  &ctx->b_loc_elem,  &ctx->b_loc_knn};
     for (DevBuf *b : all) release(*b);
     for (int ph = 0; ph < 6; ++ph)
         for (int q = 0; q < 2; ++q)
@@ -1780,6 +1785,51 @@ extern "C" int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d
 }
 
 // ------------------------------------------------------------------------------------------------------
+// point location outside the walk
+// ------------------------------------------------------------------------------------------------------
+extern "C" int rt_find_elements(rt_ctx *ctx, int64_t n, const double *xy, int32_t k, int32_t *element, const int32_t **d_element) {
+    if (!ctx) return RT_ERR_ARG;
+    if (!ctx->has_mesh) return fail(ctx, RT_ERR_ARG, "rt_find_elements: upload a mesh first");
+    if (k < 1 || k > kMaxK) return fail(ctx, RT_ERR_ARG, "rt_find_elements: k = %d outside [1, RT_MAX_K = %d]", (int)k, kMaxK);
+    if (n < 0 || (n > 0 && !xy)) return fail(ctx, RT_ERR_ARG, "rt_find_elements: n = %lld points at %p", (long long)n, (const void *)xy);
+    // a NaN distance never compares less than another: the ring search would keep the first node it visits and never meet its
+    // stopping bound, i.e. scan the whole grid twice for a meaningless answer
+    for (int64_t i = 0; i < 2 * n; ++i)
+        if (!std::isfinite(xy[i]))
+            return fail(ctx, RT_ERR_ARG, "rt_find_elements: point %lld has a non-finite coordinate", (long long)(i / 2));
+    ctx->locate_knn = 0.0;
+    ctx->locate_ms = 0.0;
+    if (n > 0) {
+        CK(cudaSetDevice(ctx->device));
+        cudaStream_t st = ctx->stream;
+        CK(ensure(ctx->b_loc_xy, sizeof(double2) * (size_t)n));
+        CK(ensure(ctx->b_loc_elem, sizeof(int) * (size_t)n));
+        CK(ensure(ctx->b_loc_knn, sizeof(unsigned long long)));
+        CK(cudaMemcpyAsync(ctx->b_loc_xy.p, xy, sizeof(double2) * (size_t)n, cudaMemcpyHostToDevice, st));
+        CK(cudaMemsetAsync(ctx->b_loc_knn.p, 0, sizeof(unsigned long long), st));
+        CK(cudaEventRecord(ctx->ev2[0], st));
+        if (ctx->mixed)
+            k_find_elements<true><<<blocks_for(n, kLocateThreads), kLocateThreads, 0, st>>>(
+                ctx->m, n, (const double2 *)ctx->b_loc_xy.p, k, (int *)ctx->b_loc_elem.p, (unsigned long long *)ctx->b_loc_knn.p);
+        else
+            k_find_elements<false><<<blocks_for(n, kLocateThreads), kLocateThreads, 0, st>>>(
+                ctx->m, n, (const double2 *)ctx->b_loc_xy.p, k, (int *)ctx->b_loc_elem.p, (unsigned long long *)ctx->b_loc_knn.p);
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(ctx->ev2[1], st));
+        unsigned long long knn = 0;
+        CK(cudaMemcpyAsync(&knn, ctx->b_loc_knn.p, sizeof(knn), cudaMemcpyDeviceToHost, st));
+        if (element) CK(cudaMemcpyAsync(element, ctx->b_loc_elem.p, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, ctx->ev2[0], ctx->ev2[1]));
+        ctx->locate_knn = (double)knn;
+        ctx->locate_ms = ms;
+    }
+    if (d_element) *d_element = (const int32_t *)ctx->b_loc_elem.p;
+    return RT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------
 // volumes + NCCL
 // ------------------------------------------------------------------------------------------------------
 static int load_nccl(rt_ctx *ctx) {
@@ -1985,6 +2035,10 @@ extern "C" int rt_info(rt_ctx *ctx, const char *key, double *value) {
         *value = (double)ctx->optimistic_cancels;
     else if (k == "collectives")
         *value = (double)ctx->collectives;
+    else if (k == "locate_knn")
+        *value = ctx->locate_knn;
+    else if (k == "locate_ms")
+        *value = ctx->locate_ms;
     else
         return fail(ctx, RT_ERR_ARG, "rt_info: unknown key %s", key);
     return RT_OK;

@@ -1,7 +1,9 @@
 """Plot-friendly views of the results: the arrays the reference's Plots.jl recipes assemble (src/plot_recipes.jl), built from the
 SoA columns in one vectorised step instead of a loop over boxed Segment objects (the recipe for ``Vector{Track}`` grows three
 matrices with ``hcat`` once per segment, :50-74), plus flat NaN-separated polylines for plotting libraries that take one long
-path (SURVEY 8f-4).  Presentation only: nothing here touches the device."""
+path (SURVEY 8f-4), and a per-cell field sampled on a pixel raster for a heatmap (the recipe for ``Mesh`` draws one polygon per
+cell, which does not scale to a million cells).  Presentation only: nothing here touches the device except ``cell_raster``, which
+locates its pixels with one ``TrackGenerator.find_elements`` call."""
 from __future__ import annotations
 
 import numpy as np
@@ -73,3 +75,19 @@ def flat_mesh_edges(mesh):
     close = starts + sizes
     x[close], y[close] = xy[ids[p[:-1]], 0], xy[ids[p[:-1]], 1]
     return x[:-1], y[:-1]
+
+
+def cell_raster(tg, nx, ny, values=None):
+    """A per-cell field as an ``ny`` x ``nx`` heatmap over the bounding box: every pixel centre is located with find_element
+    (src/mesh.jl:103-146, k = 2) in one ``tg.find_elements`` call.  Returns matrices (x, y, z) of shape (ny, nx): pixel centres
+    (row j = the j-th row from the bottom) and z = ``values[e - 1]`` of the pixel's cell e, or e itself when ``values`` is None;
+    NaN where find_element returns -1."""
+    lo, hi = np.asarray(tg.mesh.bb_min, np.float64), np.asarray(tg.mesh.bb_max, np.float64)
+    xs = lo[0] + (np.arange(nx) + 0.5) * ((hi[0] - lo[0]) / nx)
+    ys = lo[1] + (np.arange(ny) + 0.5) * ((hi[1] - lo[1]) / ny)
+    x, y = np.meshgrid(xs, ys, indexing="xy")
+    ids, _ = tg.find_elements(np.stack([x.reshape(-1), y.reshape(-1)], axis=1))
+    found = ids > 0
+    z = np.full(ids.shape, np.nan)
+    z[found] = ids[found] if values is None else np.asarray(values, np.float64)[ids[found] - 1]
+    return x, y, z.reshape(ny, nx)
