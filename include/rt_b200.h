@@ -62,7 +62,16 @@ enum {
                                those of exactly the segments a full call produces (max_iter cap and failing tracks included):
                                they are summed by the count walk, which then runs one walker per track (as RT_SEG_NO_CHUNKS) */
     RT_SEG_NO_CHUNKS = 8,   /* one walker per track (no sub-track chunks) */
-    RT_SEG_SEQUENTIAL = 16  /* sequential walk kernels only (the self-verifying pipelines fall back to them by themselves) */
+    RT_SEG_SEQUENTIAL = 16, /* sequential walk kernels only (the self-verifying pipelines fall back to them by themselves) */
+    RT_SEG_EXACT_VOLUMES = 32 /* sum the volumes in the reference's order (fill_volumes, src/trackgenerator.jl:371-386): tracks in
+                               uid order, segments in walk order, one sequential `+` per segment, then / n_azim_2.  The volumes
+                               are then bit-equal to the reference's and do not depend on the run, the pipeline, the tuning
+                               knobs, the segment capacity or the number of ranks.  Every batch's (element, delta_eff*len)
+                               pairs are sorted stably by element and folded onto the running sums (about 24 bytes per segment
+                               of the largest batch on the device, RT_ERR_NOMEM if they do not fit).  Without the flag the
+                               per-element sums are atomic and their last bits vary.  RT_ERR_ARG together with
+                               RT_SEG_COUNT_ONLY or RT_SEG_NO_VOLUMES (nothing to fold).  With a communicator of more than one
+                               rank, see rt_volumes: the shard's segments must fit in one batch (RT_ERR_ARG otherwise) */
 };
 
 /* ---- context ------------------------------------------------------------------------------------- */
@@ -231,7 +240,14 @@ int rt_find_elements(rt_ctx *ctx, int64_t n, const double *xy, int32_t k, int32_
  * copies the result.  Every rank must call rt_volumes once per rt_segmentize, in the same order -- ALSO when its rt_segmentize
  * returned an error (RT_ERR_TRACK leaves valid sums; after any other error the rank joins the collective with a zero contribution
  * and raises a flag that travels with the sums): the call then returns that rank's error, and every rank that asks for the
- * volumes (host pointer) gets RT_ERR_PEER instead of silently incomplete sums.  Nobody is left waiting inside the all-reduce. */
+ * volumes (host pointer) gets RT_ERR_PEER instead of silently incomplete sums.  Nobody is left waiting inside the all-reduce.
+ * All ranks pass the same flags to rt_segmentize.  With RT_SEG_EXACT_VOLUMES the sums of a sequential fold cannot be all-reduced:
+ * rt_volumes runs a chain in rank order instead.  Rank r receives the running sums from rank r-1 (rank 0 starts from zero), folds
+ * its shard's sorted contributions onto them, and sends them to rank r+1; the last rank broadcasts the final sums and every rank
+ * normalises.  The shards must be in ascending uid order by rank (rank r's uid_begin = rank r-1's uid_end): otherwise every rank
+ * that asks for the volumes gets RT_ERR_ARG, and nobody is left waiting.  The chain's NCCL calls (ncclRecv, ncclSend,
+ * ncclBroadcast) are counted by rt_info "collectives"; with one rank it sends nothing.  A rank whose rt_segmentize failed joins the
+ * chain without contributions and with the failed-rank flag, as above (RT_ERR_PEER on its peers). */
 int rt_volumes(rt_ctx *ctx, double *volumes /* n_cells, or NULL */);
 
 /* ---- multi-GPU: one context per process/GPU, tracks sharded by uid range, mesh replicated -----------
@@ -250,7 +266,9 @@ int rt_stats(rt_ctx *ctx, double stats[8]);
  * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose
  * rt_segmentize failed: the ranks of a communicator that call rt_volumes as documented below agree on it); "rho", "band_cost"
  * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths; "locate_knn" (points that entered the k-nearest-node
- * branch of find_element) and "locate_ms" (k_find_elements alone) of the last rt_find_elements */
+ * branch of find_element) and "locate_ms" (k_find_elements alone) of the last rt_find_elements; "exact_vol_ms" (contributions,
+ * sort and fold of RT_SEG_EXACT_VOLUMES, summed over the batches of the last rt_segmentize; the chain's fold of rt_volumes is not
+ * included) */
 int rt_info(rt_ctx *ctx, const char *key, double *value);
 /* CUDA-event time (ms) of the last call's device work, by phase: 0 upload+prep, 1 trace, 2 count,
  * 3 scan, 4 fill, 5 volumes(+allreduce) */

@@ -153,7 +153,7 @@ function b200_segments(t::TrackGenerator{T}, uid::Integer) where {T}
 end
 
 """
-    b200_segmentize!(t::TrackGenerator; k=5, rtol=√eps, materialize=true)
+    b200_segmentize!(t::TrackGenerator; k=5, rtol=√eps, materialize=true, exact_volumes=false)
 
 Device version of `segmentize!` (trackgenerator.jl:357-369): walk (count + record) → scan → evaluation (+ fused `fill_volumes`).
 The records come back over the thin wire (28 bytes per segment).  With `materialize=true` every `track.segments` is refilled with
@@ -161,8 +161,13 @@ the reference's own `Segment` objects, exactly as `_segmentize_track!` leaves th
 fine for the reference's own problem sizes, seconds for 5e7 segments); with `materialize=false` they stay empty and
 `b200_segments(t, uid)` gives a lazy view instead.  For meshes whose segments do not fit host memory use `rt_segments_device` /
 the batch callback.
+With `exact_volumes=true` (`RT_SEG_EXACT_VOLUMES`) `t.volumes` are summed in `fill_volumes`' own order (tracks in uid order,
+segments in walk order) and are bit-equal to the reference's, whatever the pipeline, knobs, segment capacity or number of ranks; by
+default they are summed with atomics and their last bits vary.  With several ranks every rank passes the same flags, each shard
+must fit in one batch, and the shards must be in ascending uid order by rank (include/rt_b200.h, rt_volumes).
 """
-function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtoldefault(T), materialize::Bool=true) where {T}
+function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtoldefault(T), materialize::Bool=true,
+                          exact_volumes::Bool=false) where {T}
     @unpack tracks_by_uid, azimuthal_quadrature, volumes = t
     !isassigned(tracks_by_uid, 1) && error("Segmentation is intended after tracing. Please, " *
                                            "call `trace!` first!")
@@ -171,7 +176,8 @@ function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtolde
     rc = ccall((:rt_segmentize, LIBRT_B200), Cint,
         (Ptr{Cvoid}, Float64, Int32, Float64, Int32, Ptr{Float64}, UInt32, Ptr{Cvoid}, Ptr{Cvoid},
          Ptr{Int64}, Ptr{Int64}, Ptr{Int32}),
-        ctx, Float64(t.tiny_step), Int32(k), Float64(rtol), Int32(MAX_ITER), azimuthal_quadrature.δs, UInt32(0),
+        ctx, Float64(t.tiny_step), Int32(k), Float64(rtol), Int32(MAX_ITER), azimuthal_quadrature.δs,
+        UInt32(exact_volumes ? 32 : 0),                       # RT_SEG_EXACT_VOLUMES
         C_NULL, C_NULL, nseg, bad, st)
     if rc != 0
         # every rank of a communicator enters the all-reduce once per segmentize!, also the one that is about to throw

@@ -6,4 +6,6 @@ from .api import (  # noqa: F401
     Reflective, Segment, SegmentColumns, Track, TrackGenerator, TrackLayout, Vacuum, bc_bwd, bc_fwd, dir_next_track_bwd, dir_next_track_fwd, ell,
     find_element, nazim, nazim2, nazim4, segmentize_, trace_, RTOL_DEFAULT, MAX_ITER,
 )
-from ._lib import RTError, RT_SEG_COUNT_ONLY, RT_SEG_LITERAL, RT_SEG_NO_CHUNKS, RT_SEG_NO_VOLUMES, RT_SEG_SEQUENTIAL, build  # noqa: F401
+from ._lib import (  # noqa: F401
+    RTError, RT_SEG_COUNT_ONLY, RT_SEG_EXACT_VOLUMES, RT_SEG_LITERAL, RT_SEG_NO_CHUNKS, RT_SEG_NO_VOLUMES, RT_SEG_SEQUENTIAL, build,
+)

@@ -742,7 +742,7 @@ class SegmentBatch:
 
 
 def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flags: int = 0, max_iter: int = MAX_ITER,
-                check: bool = True, fetch_volumes: bool = True, on_batch=None) -> TrackGenerator:
+                check: bool = True, fetch_volumes: bool = True, on_batch=None, exact_volumes: bool = False) -> TrackGenerator:
     """segmentize!(tg; k, rtol): count pass -> scan -> fill pass (+ fused fill_volumes) on the device.
     ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits).  Inside it
     ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()`` and ``tg.correct_volumes()`` act
@@ -754,8 +754,16 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
     ``on_batch`` or RT_SEG_COUNT_ONLY, ``tg.volume_factors`` is None.  Batched segments are corrected by a second segmentize_
     whose ``on_batch`` calls ``tg.correct_volumes()`` for every batch: the factors come from the volumes of the call before it,
     which must have run with volumes, and the correcting call may use RT_SEG_NO_VOLUMES (its own volumes would be those of the
-    lengths before correction)."""
+    lengths before correction).
+
+    ``exact_volumes=True`` (RT_SEG_EXACT_VOLUMES) sums the volumes in the reference's order -- tracks in uid order, segments in
+    walk order -- so that they are bit-equal to fill_volumes and the same whatever the run, pipeline, knobs, segment capacity or
+    number of ranks; the default sums them with atomics, whose last bits vary.  It cannot be combined with RT_SEG_COUNT_ONLY or
+    RT_SEG_NO_VOLUMES, and with a communicator of several ranks each shard must fit in one batch and the shards must be in
+    ascending uid order by rank."""
     L = _lib.lib()
+    if exact_volumes:
+        flags |= _lib.RT_SEG_EXACT_VOLUMES
     cb = None
     if on_batch is not None:
         def _cb(bptr, _user):

@@ -20,6 +20,7 @@
 #include "march.cuh"
 #include "trace.cuh"
 #include "locate.cuh"
+#include "exact_vol.cuh"
 
 using namespace rt;
 
@@ -35,6 +36,11 @@ struct NcclApi {
     ncclResult_t (*GetUniqueId)(ncclUniqueId *) = nullptr;
     ncclResult_t (*CommInitRank)(ncclComm_t *, int, ncclUniqueId, int) = nullptr;
     ncclResult_t (*AllReduce)(const void *, void *, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*Send)(const void *, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*Recv)(void *, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*Broadcast)(const void *, void *, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*GroupStart)() = nullptr;
+    ncclResult_t (*GroupEnd)() = nullptr;
     ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
     const char *(*GetErrorString)(ncclResult_t) = nullptr;
 };
@@ -187,6 +193,18 @@ struct rt_ctx {
     bool voln_done = false;                                 // b_voln already holds the normalised volumes of the last rt_segmentize (no communicator)
     int voln_ready = -1;                                    // index of the event that marks b_voln complete (-1: main stream)
     long long collectives = 0;                              // ncclAllReduce calls issued by rt_volumes, failed-rank joins included (info)
+
+    // RT_SEG_EXACT_VOLUMES (exact_vol.cuh): the pairs of the last batch, sorted by element, and the run bounds of every element
+    bool exact = false;                // the last rt_segmentize asked for exact volumes (also when it failed: rt_volumes joins the chain)
+    bool ex_defer = false;             // ... with a communicator of several ranks: the fold of the shard waits for rt_volumes' chain
+    DevBuf b_ex_key, b_ex_val, b_ex_runs, b_ex_tmp, b_chain;  // keys / values (two of each: the sort ping-pongs), start|end, sort scratch, chain message
+    const double *ex_val = nullptr;    // sorted values of the last batch (one of the two halves of b_ex_val)
+    long long ex_n = 0;                // ... how many
+    cudaEvent_t ev_ex[2] = {nullptr, nullptr};  // stopwatch of one batch's contributions, sort and fold
+    bool ex_pending = false;           // ev_ex holds a batch not yet added to exact_vol_ms
+    double exact_vol_ms = 0.0;
+    cudaEvent_t ev_ex_free = nullptr;  // coll_stream: the chain has folded the sorted pairs (the next rt_segmentize may overwrite them)
+    bool ex_free_used = false;
 };
 
 static inline unsigned long long *d_counters(rt_ctx *c) { return (unsigned long long *)c->b_ctrl.p; }
@@ -293,7 +311,8 @@ extern "C" void rt_destroy(rt_ctx *ctx) {
                      &ctx->b_omega,   &ctx->b_sigma,     &ctx->b_tau,
                      &ctx->b_pool,    &ctx->b_pool_next, &ctx->b_pool_cursor,
                      &ctx->b_area,    &ctx->b_factor,    &ctx->b_layout,    &ctx->b_vol_alt,  &ctx->b_exc,
-                     &ctx->b_loc_xy,  &ctx->b_loc_elem,  &ctx->b_loc_knn};
+                     &ctx->b_loc_xy,  &ctx->b_loc_elem,  &ctx->b_loc_knn,
+                     &ctx->b_ex_key,  &ctx->b_ex_val,    &ctx->b_ex_runs,   &ctx->b_ex_tmp,   &ctx->b_chain};
     for (DevBuf *b : all) release(*b);
     for (int ph = 0; ph < 6; ++ph)
         for (int q = 0; q < 2; ++q)
@@ -302,7 +321,7 @@ extern "C" void rt_destroy(rt_ctx *ctx) {
         cudaStreamSynchronize(ctx->coll_stream);
         cudaStreamDestroy(ctx->coll_stream);
     }
-    for (cudaEvent_t e : {ctx->ev_fill_done, ctx->ev_vol_free[0], ctx->ev_vol_free[1]})
+    for (cudaEvent_t e : {ctx->ev_fill_done, ctx->ev_vol_free[0], ctx->ev_vol_free[1], ctx->ev_ex_free, ctx->ev_ex[0], ctx->ev_ex[1]})
         if (e) cudaEventDestroy(e);
     if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
     if (ctx->ev_aux) cudaEventDestroy(ctx->ev_aux);
@@ -887,11 +906,12 @@ static void bind_columns(const rt_ctx *ctx, WalkParams &P) {
     P.oelem = ctx->s_elem;
 }
 
-// Segment columns sized from free memory (0.92 x free / 44 bytes per segment, counting the columns held now) for `want` segments
-// (already limited by the capacity option): one batch takes what it needs if that fits, a walk in several batches everything that
-// fits.  *cap: the capacity to cut the batches with.
+// Segment columns sized from free memory (0.92 x free / 44 bytes per segment, counting the columns held now; 68 bytes and the
+// sorted pairs held now with exact volumes) for `want` segments (already limited by the capacity option): one batch takes what it
+// needs if that fits, a walk in several batches everything that fits.  *cap: the capacity to cut the batches with.
 static int size_columns(rt_ctx *ctx, long long want, bool take_all, size_t free_b, long long *cap) {
-    const long long fit = (long long)((double)(free_b + ctx->b_seg_d.bytes + ctx->b_seg_e.bytes) * 0.92 / 44.0);
+    const size_t held = ctx->b_seg_d.bytes + ctx->b_seg_e.bytes + (ctx->exact ? ctx->b_ex_key.bytes + ctx->b_ex_val.bytes : 0);
+    const long long fit = (long long)((double)(free_b + held) * 0.92 / (ctx->exact ? 68.0 : 44.0));
     *cap = take_all ? fit : std::min(want, fit);
     if (ctx->cap_cfg > 0) *cap = std::min(*cap, (long long)ctx->cap_cfg);
     return ensure_segment_buffers(ctx, *cap);
@@ -941,6 +961,9 @@ static int read_verify(rt_ctx *ctx, bool *failed) {
     return RT_OK;
 }
 
+// the accumulator the fill kernels add delta_eff*len to (none with exact volumes: exact_batch folds them)
+static double *fused_vol(const rt_ctx *ctx, const Attempt &a) { return a.want_vol && !ctx->exact ? ctx->vol_acc : nullptr; }
+
 // the resident batch may be read: after a completed rt_segmentize, or from inside its batch callback
 static bool resident_valid(const rt_ctx *ctx) { return ctx && (ctx->segmented || ctx->in_batch_cb); }
 
@@ -955,6 +978,64 @@ static int deliver_batch(rt_ctx *ctx, const Attempt &a) {
     const int stop = a.cb(&bt, a.cb_user);
     ctx->in_batch_cb = false;
     if (stop) return fail(ctx, RT_ERR_ARG, "rt_segmentize: batch callback asked to stop");
+    return RT_OK;
+}
+
+// adds the stopwatch of the last exact batch to exact_vol_ms (waits for it)
+static void exact_take_time(rt_ctx *ctx) {
+    if (!ctx->ex_pending) return;
+    float ms = 0.f;
+    if (cudaEventSynchronize(ctx->ev_ex[1]) == cudaSuccess && cudaEventElapsedTime(&ms, ctx->ev_ex[0], ctx->ev_ex[1]) == cudaSuccess)
+        ctx->exact_vol_ms += (double)ms;
+    ctx->ex_pending = false;
+}
+
+// RT_SEG_EXACT_VOLUMES (exact_vol.cuh): the pairs of the batch P describes (nseg segments, final), sorted stably by element, their
+// run bounds, and -- unless the chain of rt_volumes folds them -- the fold onto the running sums vol_acc (cleared, like the fused
+// sums, at the start of every attempt: a restarted call folds its batches again from zero).  Runs before the batch callback.
+static int exact_batch(rt_ctx *ctx, const WalkParams &P, long long nseg, Attempt &a) {
+    if (!ctx->exact) return RT_OK;
+    if (ctx->ex_defer && (P.trk_begin != 0 || P.trk_end != ctx->n_shard))
+        return fail(ctx, RT_ERR_ARG, "rt_segmentize: RT_SEG_EXACT_VOLUMES with a communicator of %d ranks needs the shard's segments in "
+                    "one batch (the rank-order chain of rt_volumes folds the whole shard); raise the segment capacity", ctx->n_ranks);
+    cudaStream_t st = ctx->stream;
+    const int nc = ctx->m.n_cells;
+    ctx->ex_n = 0;
+    if (!ctx->ev_ex[0])
+        for (cudaEvent_t &e : ctx->ev_ex) CK(cudaEventCreate(&e));
+    exact_take_time(ctx);
+    if (ctx->ex_free_used) CK(cudaStreamWaitEvent(st, ctx->ev_ex_free, 0));  // (the chain of the last rt_volumes still reads them)
+    int bits = 1;
+    while (bits < 31 && (1LL << bits) < (long long)nc) ++bits;  // ceil(log2(n_cells)) key bits
+    const size_t n = (size_t)std::max<long long>(nseg, 1);
+    if (ensure(ctx->b_ex_key, sizeof(int) * 2 * n) != cudaSuccess || ensure(ctx->b_ex_val, sizeof(double) * 2 * n) != cudaSuccess ||
+        ensure(ctx->b_ex_runs, sizeof(long long) * 2 * (size_t)nc) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: no device memory for the %lld sorted pairs of RT_SEG_EXACT_VOLUMES", nseg);
+    int *key = (int *)ctx->b_ex_key.p;
+    double *val = (double *)ctx->b_ex_val.p;
+    cub::DoubleBuffer<int> dk(key, key + n);
+    cub::DoubleBuffer<double> dv(val, val + n);
+    size_t tmp = 0;
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, dk, dv, nseg, 0, bits, st));
+    if (ensure(ctx->b_ex_tmp, tmp) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: no device memory for the sort of RT_SEG_EXACT_VOLUMES (%zu bytes)", tmp);
+    long long *start = (long long *)ctx->b_ex_runs.p, *end = start + nc;
+    CK(cudaEventRecord(ctx->ev_ex[0], st));
+    CK(cudaMemsetAsync(start, 0, sizeof(long long) * 2 * (size_t)nc, st));
+    if (nseg > 0) {
+        k_exact_contrib<<<blocks_for((P.trk_end - P.trk_begin) * 32, kExactThreads), kExactThreads, 0, st>>>(
+            P.offsets, P.trk_begin, P.trk_end, P.offset_base, ctx->t.azim, P.ang.delta_eff, P.olen, P.oelem, dk.Current(), dv.Current());
+        CK(cub::DeviceRadixSort::SortPairs(ctx->b_ex_tmp.p, tmp, dk, dv, nseg, 0, bits, st));
+        k_exact_runs<<<blocks_for(nseg, kExactThreads), kExactThreads, 0, st>>>(dk.Current(), nseg, nc, start, end);
+        if (!ctx->ex_defer)
+            k_exact_fold<<<blocks_for(nc, kExactThreads), kExactThreads, 0, st>>>(nc, start, end, dv.Current(), ctx->vol_acc);
+        a.launches += ctx->ex_defer ? 2 : 3;
+    }
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->ev_ex[1], st));
+    ctx->ex_pending = true;
+    ctx->ex_val = dv.Current();
+    ctx->ex_n = nseg;
     return RT_OK;
 }
 
@@ -1181,8 +1262,9 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         CK(cudaGetLastError());
         toc(ctx, 2);
         tic(ctx, 3);
+        // (exact volumes size their sort from the segment total on the host: never optimistic)
         const bool optimistic = !multi && !a.cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
-                                ctx->fit_gen == ctx->trace_gen && ctx->b_seg_d.p && ctx->cap > 0;
+                                ctx->fit_gen == ctx->trace_gen && ctx->b_seg_d.p && ctx->cap > 0 && !ctx->exact;
         ScanGuard guard{};
         if (optimistic) guard = ScanGuard{d_guard(ctx), base, ctx->cap, P.pool_cursor, P.pool_blocks};
         CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p + b, (long long *)ctx->b_offsets.p + b, e - b, base, guard)));
@@ -1195,7 +1277,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
             // the guard (does the batch fit the Segment columns, did the pool hold every record?) is evaluated by the scan
             P.offset_base = base;
             bind_columns(ctx, P);
-            P.vol = a.want_vol ? ctx->vol_acc : nullptr;
+            P.vol = fused_vol(ctx, a);
             tic(ctx, 4);
             launch_eval(d_guard(ctx));
             launch_track_status(ctx, P, a.rtol, d_guard(ctx), d_bad(ctx));
@@ -1228,7 +1310,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         const long long cap = ctx->cap_cfg > 0 ? std::min(ctx->cap, (long long)ctx->cap_cfg) : ctx->cap;
         P.offset_base = base;
         bind_columns(ctx, P);
-        P.vol = a.want_vol ? ctx->vol_acc : nullptr;
+        P.vol = fused_vol(ctx, a);
         const bool split = batch_total > cap;
         ctx->fit_gen = (!multi && !split) ? ctx->trace_gen : ~0ULL;  // (the next call with these tracks may skip this round trip)
         if (split) {
@@ -1259,7 +1341,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
                 a.defer_verify = true;
                 ctx->phase_ms[2] = acc[2];
                 ctx->phase_ms[3] = acc[3];
-                return RT_OK;
+                return exact_batch(ctx, P, nseg, a);  // (a failed verification restarts the call, which clears the sums again)
             }
             bool failed = false;
             int rc = read_verify(ctx, &failed);
@@ -1269,6 +1351,8 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
                 a.next = Next::Sequential;
                 return RT_OK;
             }
+            rc = exact_batch(ctx, P, nseg, a);
+            if (rc) return rc;
             rc = deliver_batch(ctx, a);
             if (rc) return rc;
         }
@@ -1338,7 +1422,7 @@ static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool 
     }
     bind_columns(ctx, P);
     P.tsum = hybrid ? (double *)ctx->b_tsum.p : nullptr;
-    P.vol = a.want_vol ? ctx->vol_acc : nullptr;
+    P.vol = fused_vol(ctx, a);
     P.counters = nullptr;
     if (ctx->opt_debug_verify_fail && hybrid) CK(cudaMemsetAsync(d_verify(ctx), 1, 1, st));
     const bool split = total > cap;
@@ -1377,6 +1461,8 @@ static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool 
                 return RT_OK;
             }
         }
+        rc = exact_batch(ctx, P, nseg, a);
+        if (rc) return rc;
         rc = deliver_batch(ctx, a);
         if (rc) return rc;
     }
@@ -1477,6 +1563,12 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
                              int32_t *bad_status) {
     if (!ctx) return RT_ERR_ARG;
     if (ctx->in_batch_cb) return fail(ctx, RT_ERR_ARG, "rt_segmentize: called from inside a batch callback");
+    // (set before anything can fail: a rank whose call failed joins the rt_volumes of this call's kind, the chain or the all-reduce)
+    ctx->exact = (flags & RT_SEG_EXACT_VOLUMES) != 0;
+    ctx->ex_defer = ctx->exact && ctx->comm && ctx->coll_stream && ctx->n_ranks > 1;
+    ctx->ex_n = 0;
+    exact_take_time(ctx);
+    ctx->exact_vol_ms = 0.0;
     // (what rt_correct_volumes may use inside this call's batch callback)
     ctx->prev_vol_valid = ctx->segmented && ctx->vol_valid && ctx->b_voln.p;
     // (whatever goes wrong below, the results of an earlier call are no longer "the last segmentize!": rt_volumes must see that)
@@ -1488,6 +1580,9 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
     if (k > kMaxK)
         return fail(ctx, RT_ERR_ARG, "rt_segmentize: k = %d exceeds RT_MAX_K = %d (the k-nearest-node fallback of find_element keeps a fixed-size candidate list)", (int)k, kMaxK);
     const bool want_vol = !(flags & RT_SEG_NO_VOLUMES);
+    if (ctx->exact && (flags & (RT_SEG_COUNT_ONLY | RT_SEG_NO_VOLUMES)))
+        return fail(ctx, RT_ERR_ARG, "rt_segmentize: RT_SEG_EXACT_VOLUMES together with %s: there are no %s to fold",
+                    (flags & RT_SEG_COUNT_ONLY) ? "RT_SEG_COUNT_ONLY" : "RT_SEG_NO_VOLUMES", (flags & RT_SEG_COUNT_ONLY) ? "segments" : "volumes");
     if (want_vol && !delta_eff) return fail(ctx, RT_ERR_ARG, "rt_segmentize: delta_eff is required unless RT_SEG_NO_VOLUMES");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
@@ -1846,7 +1941,14 @@ static int load_nccl(rt_ctx *ctx) {
     a.AllReduce = (decltype(a.AllReduce))dlsym(a.lib, "ncclAllReduce");
     a.CommDestroy = (decltype(a.CommDestroy))dlsym(a.lib, "ncclCommDestroy");
     a.GetErrorString = (decltype(a.GetErrorString))dlsym(a.lib, "ncclGetErrorString");
-    if (!a.GetUniqueId || !a.CommInitRank || !a.AllReduce || !a.CommDestroy) return fail(ctx, RT_ERR_NCCL, "NCCL symbols missing");
+    a.Send = (decltype(a.Send))dlsym(a.lib, "ncclSend");
+    a.Recv = (decltype(a.Recv))dlsym(a.lib, "ncclRecv");
+    a.Broadcast = (decltype(a.Broadcast))dlsym(a.lib, "ncclBroadcast");
+    a.GroupStart = (decltype(a.GroupStart))dlsym(a.lib, "ncclGroupStart");
+    a.GroupEnd = (decltype(a.GroupEnd))dlsym(a.lib, "ncclGroupEnd");
+    if (!a.GetUniqueId || !a.CommInitRank || !a.AllReduce || !a.CommDestroy || !a.Send || !a.Recv || !a.Broadcast || !a.GroupStart ||
+        !a.GroupEnd)
+        return fail(ctx, RT_ERR_NCCL, "NCCL symbols missing");
     return RT_OK;
 }
 
@@ -1874,11 +1976,73 @@ extern "C" int rt_comm_init(rt_ctx *ctx, int32_t n_ranks, int32_t rank, const ch
         if (cudaStreamCreateWithFlags(&ctx->coll_stream, cudaStreamNonBlocking) != cudaSuccess ||
             cudaEventCreateWithFlags(&ctx->ev_fill_done, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&ctx->ev_vol_free[0], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&ctx->ev_vol_free[1], cudaEventDisableTiming) != cudaSuccess)
+            cudaEventCreateWithFlags(&ctx->ev_vol_free[1], cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&ctx->ev_ex_free, cudaEventDisableTiming) != cudaSuccess)
             return fail(ctx, RT_ERR_CUDA, "rt_comm_init: cannot create the collective stream");
     }
     ctx->n_ranks = n_ranks;
     ctx->rank = rank;
+    return RT_OK;
+}
+
+// rt_volumes after an rt_segmentize with RT_SEG_EXACT_VOLUMES on a context with a communicator: the chain in rank order on the
+// collective stream (the message: exact_vol.cuh k_chain_stamp).  have: this rank's call succeeded (else it contributes nothing and
+// raises the failed-rank flag).  With one rank the sums were folded by rt_segmentize and nothing is sent.
+static int exact_chain(rt_ctx *ctx, bool have, double *volumes) {
+    cudaStream_t st = ctx->stream, cs = ctx->coll_stream;
+    const int nc = ctx->m.n_cells, R = ctx->n_ranks, r = ctx->rank;
+    const size_t nmsg = (size_t)nc + 3;
+    CK(ensure(ctx->b_chain, sizeof(double) * nmsg));
+    double *msg = (double *)ctx->b_chain.p, *voln = (double *)ctx->b_voln.p;
+    auto nccl = [&](const char *what, ncclResult_t rr) {
+        ctx->collectives += 1;
+        return rr == 0 ? RT_OK : fail(ctx, RT_ERR_NCCL, "%s: %s", what, ctx->nccl.GetErrorString ? ctx->nccl.GetErrorString(rr) : "?");
+    };
+    CK(cudaEventRecord(ctx->ev_fill_done, st));
+    CK(cudaStreamWaitEvent(cs, ctx->ev_fill_done, 0));
+    CK(cudaEventRecord(ctx->pev[5][0], cs));
+    int rc = RT_OK;
+    if (r > 0) {
+        rc = nccl("ncclRecv", ctx->nccl.Recv(msg, nmsg, ncclFloat64, r - 1, ctx->comm, cs));
+    } else {
+        CK(cudaMemsetAsync(msg, 0, sizeof(double) * nmsg, cs));
+        if (have) CK(cudaMemcpyAsync(msg, ctx->vol_acc, sizeof(double) * (size_t)nc, cudaMemcpyDeviceToDevice, cs));
+    }
+    if (rc) return rc;
+    if (have && ctx->ex_defer && ctx->ex_n > 0) {
+        const long long *start = (const long long *)ctx->b_ex_runs.p;
+        k_exact_fold<<<blocks_for(nc, kExactThreads), kExactThreads, 0, cs>>>(nc, start, start + nc, ctx->ex_val, msg);
+        CK(cudaEventRecord(ctx->ev_ex_free, cs));
+        ctx->ex_free_used = true;
+    }
+    k_chain_stamp<<<1, 1, 0, cs>>>(msg, nc, r > 0, (double)ctx->uid_begin, (double)(ctx->uid_begin + ctx->n_shard), have ? 0.0 : 1.0);
+    CK(cudaGetLastError());
+    if (r < R - 1) rc = nccl("ncclSend", ctx->nccl.Send(msg, nmsg, ncclFloat64, r + 1, ctx->comm, cs));
+    if (rc) return rc;
+    if (R > 1) rc = nccl("ncclBroadcast", ctx->nccl.Broadcast(msg, msg, nmsg, ncclFloat64, R - 1, ctx->comm, cs));
+    if (rc) return rc;
+    k_normalise<<<blocks_for(nc, 256), 256, 0, cs>>>(msg, voln, nc, (double)ctx->n2);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(voln + nc, msg + nc, sizeof(double), cudaMemcpyDeviceToDevice, cs));  // (the failed-rank count, as after an all-reduce)
+    CK(cudaEventRecord(ctx->pev[5][1], cs));
+    ctx->pev_dirty[5] = true;
+    if (have) {
+        CK(cudaEventRecord(ctx->ev_vol_free[ctx->vol_cur], cs));
+        ctx->ev_vol_used[ctx->vol_cur] = true;
+        ctx->voln_ready = ctx->vol_cur;
+    }
+    if (volumes || !have) CK(cudaStreamSynchronize(cs));
+    if (!have) return fail(ctx, RT_ERR_ARG, "rt_volumes: this rank's rt_segmentize failed; it joined the rank-order chain of the exact volumes without contributions and with the failed-rank flag");
+    if (volumes) {
+        double flags[2] = {0.0, 0.0};
+        CK(cudaMemcpy(volumes, voln, sizeof(double) * (size_t)nc, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(flags, msg + nc, sizeof(flags), cudaMemcpyDeviceToHost));
+        if (flags[0] != 0.0)
+            return fail(ctx, RT_ERR_PEER, "rt_volumes: rt_segmentize failed on %d rank(s) of the communicator: the volumes miss their tracks", (int)flags[0]);
+        if (flags[1] != 0.0)
+            return fail(ctx, RT_ERR_ARG, "rt_volumes: RT_SEG_EXACT_VOLUMES needs the uid shards in ascending rank order (rank r starts where "
+                        "rank r-1 ends); %d rank(s) did not, so the chained sums are not in the reference's order", (int)flags[1]);
+    }
     return RT_OK;
 }
 
@@ -1891,6 +2055,7 @@ extern "C" int rt_volumes(rt_ctx *ctx, double *volumes) {
     cudaStream_t st = ctx->stream;
     int nc = ctx->m.n_cells;
     CK(ensure(ctx->b_voln, sizeof(double) * ((size_t)nc + 1)));
+    if (coll && ctx->exact) return exact_chain(ctx, have, volumes);
     const double *src = ctx->vol_acc ? ctx->vol_acc : (const double *)ctx->b_vol.p;
     if (!have) {
         // This rank's rt_segmentize failed, but its peers are (or will be) inside the all-reduce: join it with a zero contribution
@@ -2039,6 +2204,11 @@ extern "C" int rt_info(rt_ctx *ctx, const char *key, double *value) {
         *value = ctx->locate_knn;
     else if (k == "locate_ms")
         *value = ctx->locate_ms;
+    else if (k == "exact_vol_ms") {
+        cudaSetDevice(ctx->device);
+        exact_take_time(ctx);
+        *value = ctx->exact_vol_ms;
+    }
     else
         return fail(ctx, RT_ERR_ARG, "rt_info: unknown key %s", key);
     return RT_OK;
