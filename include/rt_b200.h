@@ -63,7 +63,7 @@ enum {
                                they are summed by the count walk, which then runs one walker per track (as RT_SEG_NO_CHUNKS) */
     RT_SEG_NO_CHUNKS = 8,   /* one walker per track (no sub-track chunks) */
     RT_SEG_SEQUENTIAL = 16, /* sequential walk kernels only (the self-verifying pipelines fall back to them by themselves) */
-    RT_SEG_EXACT_VOLUMES = 32 /* sum the volumes in the reference's order (fill_volumes, src/trackgenerator.jl:371-386): tracks in
+    RT_SEG_EXACT_VOLUMES = 32, /* sum the volumes in the reference's order (fill_volumes, src/trackgenerator.jl:371-386): tracks in
                                uid order, segments in walk order, one sequential `+` per segment, then / n_azim_2.  The volumes
                                are then bit-equal to the reference's and do not depend on the run, the pipeline, the tuning
                                knobs, the segment capacity or the number of ranks.  Every batch's (element, delta_eff*len)
@@ -72,6 +72,15 @@ enum {
                                per-element sums are atomic and their last bits vary.  RT_ERR_ARG together with
                                RT_SEG_COUNT_ONLY or RT_SEG_NO_VOLUMES (nothing to fold).  With a communicator of more than one
                                rank, see rt_volumes: the shard's segments must fit in one batch (RT_ERR_ARG otherwise) */
+    RT_SEG_LENGTHS_ONLY = 64  /* write only the len and element columns (12 instead of 44 bytes per segment, 36 instead of 68 with
+                               RT_SEG_EXACT_VOLUMES): for consumers that never read p and q (optical lengths, the volume
+                               correction, a MOC sweep that keeps (len, region) per segment).  Everything else -- offsets, status,
+                               first_bad_uid, volumes, the length check, verification and fall-backs -- is computed exactly as
+                               without the flag, and len / element are the same bits.  The columns are sized at 12 bytes per
+                               segment (rt_info "segment_capacity").  The resident batch then has no p / q:
+                               rt_batch / rt_segments_device give NULL for d_px, d_py, d_qx, d_qy; rt_segments_download returns
+                               RT_ERR_ARG (copying nothing) if any of px, py, qx, qy is not NULL; rt_segments_download_compact
+                               returns RT_ERR_ARG.  No effect together with RT_SEG_COUNT_ONLY (no columns are written) */
 };
 
 /* ---- context ------------------------------------------------------------------------------------- */
@@ -143,7 +152,7 @@ typedef struct rt_batch {
     int64_t n_segments;           /* segments in this batch */
     const int64_t *d_offsets;     /* DEVICE: offsets of the shard's tracks (n_shard+1), global to the shard */
     int64_t offset_base;          /* subtract from d_offsets[uid-shard_begin] to index the arrays below */
-    const double *d_px, *d_py, *d_qx, *d_qy, *d_len; /* DEVICE SoA */
+    const double *d_px, *d_py, *d_qx, *d_qy, *d_len; /* DEVICE SoA (d_px .. d_qy are NULL with RT_SEG_LENGTHS_ONLY) */
     const int32_t *d_element;     /* DEVICE, 1-based element ids */
     void *stream;                 /* cudaStream_t the batch was produced on */
     int32_t attempt;              /* 1: the call restarted sequentially after a failed verification; drop attempt-0 batches */
@@ -157,7 +166,8 @@ int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rtol, int32_t
 /* per-track segment counts / offsets / status of the shard after rt_segmentize (host copies) */
 int rt_segment_offsets(rt_ctx *ctx, int64_t *offsets /* n_shard+1 */, int32_t *status /* n_shard or NULL */);
 /* Segment(p, q, len, element) records (src/segment.jl:23-33) of the resident batch (the whole shard when
- * it fitted), SoA, in uid order then walk order. Any pointer may be NULL.  Also valid inside the batch callback of rt_segmentize. */
+ * it fitted), SoA, in uid order then walk order. Any pointer may be NULL.  Also valid inside the batch callback of rt_segmentize.
+ * After RT_SEG_LENGTHS_ONLY only len and element exist: px, py, qx, qy must be NULL (RT_ERR_ARG otherwise, nothing copied). */
 int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double *qy, double *len,
                          int32_t *element);
 /* The same records over a thinner wire: 28 instead of 44 bytes per segment cross the bus.  Inside a track, `p` of a segment is
@@ -167,10 +177,11 @@ int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double
  * p[i] = q[i-1] and patches the listed positions: the result is bit-identical to rt_segments_download (tests/test_gpu_parity.py).
  * *n_exceptions receives the number of exceptions found; if it exceeds max_exceptions the call returns RT_ERR_NOMEM after the
  * columns have been copied, and can be repeated with larger buffers.  Column pointers may be NULL.  Also valid inside the batch
- * callback of rt_segmentize. */
+ * callback of rt_segmentize.  RT_ERR_ARG after RT_SEG_LENGTHS_ONLY (there is no q, and no p to rebuild). */
 int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy, double *len, int32_t *element, int64_t max_exceptions,
                                  int64_t *exc_index, double *exc_px, double *exc_py, int64_t *n_exceptions);
-/* device-resident view of the resident batch for on-GPU consumers (transport sweeps) */
+/* device-resident view of the resident batch for on-GPU consumers (transport sweeps); d_px .. d_qy are NULL after
+ * RT_SEG_LENGTHS_ONLY */
 int rt_segments_device(rt_ctx *ctx, rt_batch *view);
 
 /* ---- what a transport sweep consumes besides the Segment records, kept on the device (SURVEY.md 8f-1) -------------
@@ -260,7 +271,8 @@ int rt_comm_init(rt_ctx *ctx, int32_t n_ranks, int32_t rank, const char id[128])
  * stats[0..7] of the last rt_segmentize: kernel launches, fast transitions, slow (literal) iterations,
  * nearest-node queries, knn queries, count-pass ms, fill-pass ms, scan+volumes ms. */
 int rt_stats(rt_ctx *ctx, double stats[8]);
-/* named scalars: "verify_fallbacks", "n_units", "segment_capacity", "count_batches"
+/* named scalars: "verify_fallbacks", "n_units", "segment_capacity" (segments the allocated columns hold, in the layout of the last
+ * rt_segmentize), "count_batches"
  * (uid batches of the single-walk pipeline's count walk) of the last rt_segmentize; "optimistic_cancels" (calls of this context
  * whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
  * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose

@@ -141,6 +141,7 @@ function _b200_p(c::B200Columns, s::Int)
 end
 
 const _B200_COLS = IdDict{Any,Tuple{B200Columns,Vector{Int64}}}()   # per TrackGenerator: columns + offsets
+const _B200_LENS = IdDict{Any,Tuple{Vector{Float64},Vector{Int32},Vector{Int64}}}()   # ... after lengths_only=true: ℓ, element, offsets
 
 """
     b200_segments(t::TrackGenerator, uid) -> B200Segments
@@ -153,7 +154,18 @@ function b200_segments(t::TrackGenerator{T}, uid::Integer) where {T}
 end
 
 """
-    b200_segmentize!(t::TrackGenerator; k=5, rtol=√eps, materialize=true, exact_volumes=false)
+    b200_segment_lengths(t::TrackGenerator, uid) -> (ℓ, element)
+
+Views of the segment lengths and elements of track `uid` after `b200_segmentize!(t; lengths_only=true, materialize=false)`.
+"""
+function b200_segment_lengths(t::TrackGenerator, uid::Integer)
+    len, el, off = _B200_LENS[t.tracks_by_uid]
+    r = off[uid]+1:off[uid+1]
+    return view(len, r), view(el, r)
+end
+
+"""
+    b200_segmentize!(t::TrackGenerator; k=5, rtol=√eps, materialize=true, exact_volumes=false, lengths_only=false)
 
 Device version of `segmentize!` (trackgenerator.jl:357-369): walk (count + record) → scan → evaluation (+ fused `fill_volumes`).
 The records come back over the thin wire (28 bytes per segment).  With `materialize=true` every `track.segments` is refilled with
@@ -165,19 +177,24 @@ With `exact_volumes=true` (`RT_SEG_EXACT_VOLUMES`) `t.volumes` are summed in `fi
 segments in walk order) and are bit-equal to the reference's, whatever the pipeline, knobs, segment capacity or number of ranks; by
 default they are summed with atomics and their last bits vary.  With several ranks every rank passes the same flags, each shard
 must fit in one batch, and the shards must be in ascending uid order by rank (include/rt_b200.h, rt_volumes).
+With `lengths_only=true` (`RT_SEG_LENGTHS_ONLY`) the device writes and sends only `ℓ` and `element` (12 bytes per segment): for
+callers that never read `p` / `q` (optical lengths, a sweep that keeps (ℓ, region) per segment).  Every `track.segments` is left
+empty and `b200_segment_lengths(t, uid)` gives the track's `(ℓ, element)`; a `Segment` needs `p` and `q`, so it must be combined
+with `materialize=false`.
 """
 function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtoldefault(T), materialize::Bool=true,
-                          exact_volumes::Bool=false) where {T}
+                          exact_volumes::Bool=false, lengths_only::Bool=false) where {T}
     @unpack tracks_by_uid, azimuthal_quadrature, volumes = t
     !isassigned(tracks_by_uid, 1) && error("Segmentation is intended after tracing. Please, " *
                                            "call `trace!` first!")
+    lengths_only && materialize && error("b200_segmentize!: lengths_only=true has no p / q to build a `Segment` from: pass materialize=false")
     ctx = _b200_context(t)
     nseg = Ref{Int64}(0); bad = Ref{Int64}(0); st = Ref{Int32}(0)
     rc = ccall((:rt_segmentize, LIBRT_B200), Cint,
         (Ptr{Cvoid}, Float64, Int32, Float64, Int32, Ptr{Float64}, UInt32, Ptr{Cvoid}, Ptr{Cvoid},
          Ptr{Int64}, Ptr{Int64}, Ptr{Int32}),
         ctx, Float64(t.tiny_step), Int32(k), Float64(rtol), Int32(MAX_ITER), azimuthal_quadrature.δs,
-        UInt32(exact_volumes ? 32 : 0),                       # RT_SEG_EXACT_VOLUMES
+        UInt32((exact_volumes ? 32 : 0) | (lengths_only ? 64 : 0)),   # RT_SEG_EXACT_VOLUMES, RT_SEG_LENGTHS_ONLY
         C_NULL, C_NULL, nseg, bad, st)
     if rc != 0
         # every rank of a communicator enters the all-reduce once per segmentize!, also the one that is about to throw
@@ -189,6 +206,19 @@ function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtolde
     n = t.n_total_tracks; S = nseg[]
     off = Vector{Int64}(undef, n + 1)
     _b200_check(ctx, ccall((:rt_segment_offsets, LIBRT_B200), Cint, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int32}), ctx, off, C_NULL))
+    if lengths_only
+        len = Vector{Float64}(undef, S); el = Vector{Int32}(undef, S)
+        _b200_check(ctx, ccall((:rt_segments_download, LIBRT_B200), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+            ctx, C_NULL, C_NULL, C_NULL, C_NULL, len, el))
+        _B200_LENS[tracks_by_uid] = (len, el, off)
+        delete!(_B200_COLS, tracks_by_uid)
+        for uid in 1:n
+            empty!(tracks_by_uid[uid].segments)
+        end
+        _b200_check(ctx, ccall((:rt_volumes, LIBRT_B200), Cint, (Ptr{Cvoid}, Ptr{Float64}), ctx, volumes))
+        return t
+    end
     qx = Vector{Float64}(undef, S); qy = similar(qx); len = similar(qx); el = Vector{Int32}(undef, S)
     cap = 4n + S ÷ 64 + 1024
     ei = Vector{Int64}(undef, cap); ex = Vector{Float64}(undef, cap); ey = similar(ex); ne = Ref{Int64}(0)
@@ -206,6 +236,7 @@ function b200_segmentize!(t::TrackGenerator{T}; k::Int=5, rtol::Real=Base.rtolde
     o = sortperm(ei)
     cols = B200Columns(qx, qy, len, el, ei[o] .+ 1, ex[o], ey[o])   # (the ABI's indices are 0-based positions)
     _B200_COLS[tracks_by_uid] = (cols, off)
+    delete!(_B200_LENS, tracks_by_uid)
     for uid in 1:n
         segs = tracks_by_uid[uid].segments
         empty!(segs)

@@ -7,5 +7,6 @@ from .api import (  # noqa: F401
     find_element, nazim, nazim2, nazim4, segmentize_, trace_, RTOL_DEFAULT, MAX_ITER,
 )
 from ._lib import (  # noqa: F401
-    RTError, RT_SEG_COUNT_ONLY, RT_SEG_EXACT_VOLUMES, RT_SEG_LITERAL, RT_SEG_NO_CHUNKS, RT_SEG_NO_VOLUMES, RT_SEG_SEQUENTIAL, build,
+    RTError, RT_SEG_COUNT_ONLY, RT_SEG_EXACT_VOLUMES, RT_SEG_LENGTHS_ONLY, RT_SEG_LITERAL, RT_SEG_NO_CHUNKS, RT_SEG_NO_VOLUMES,
+    RT_SEG_SEQUENTIAL, build,
 )

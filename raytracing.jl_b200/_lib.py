@@ -112,6 +112,7 @@ SYMBOLS = {
 
 RT_SEG_LITERAL, RT_SEG_NO_VOLUMES, RT_SEG_COUNT_ONLY, RT_SEG_NO_CHUNKS, RT_SEG_SEQUENTIAL = 1, 2, 4, 8, 16
 RT_SEG_EXACT_VOLUMES = 32
+RT_SEG_LENGTHS_ONLY = 64
 
 _lib = None
 

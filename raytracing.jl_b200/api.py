@@ -112,16 +112,23 @@ class Segment:  # src/segment.jl:23-29
         return f"Segment(p={self.p}, q={self.q}, ell={self.ell}, element={self.element})"
 
 
+LENGTHS_ONLY_MSG = ("the segments were produced with RT_SEG_LENGTHS_ONLY (segmentize_(..., lengths_only=True)), which writes only "
+                    "len and element: there are no end points p / q")
+
+
 class SegmentColumns(Mapping):
     """The SoA columns px, py, qx, qy, len, element of the resident Segment batch.  After a COMPACT download
     (``fetch_segments(compact=True)``, rt_segments_download_compact) only qx, qy, len, element crossed the bus; ``px`` / ``py``
     are rebuilt on first use from p[i] = q[i-1] plus the exception list -- whole columns through ``cols["px"]``, or just the
-    range of one track through ``p_range`` (what ``track.segments`` uses).  Both are bit-identical to a full download."""
+    range of one track through ``p_range`` (what ``track.segments`` uses).  Both are bit-identical to a full download.
+    With ``lengths_only`` (the batch of a ``segmentize_(..., lengths_only=True)``) there are only len and element."""
 
     KEYS = ("px", "py", "qx", "qy", "len", "element")
 
-    def __init__(self, cols, exceptions=None):
+    def __init__(self, cols, exceptions=None, lengths_only=False):
         self._cols = dict(cols)
+        self.lengths_only = lengths_only
+        self._keys = ("len", "element") if lengths_only else self.KEYS
         self._exc = None
         if exceptions is not None:
             idx, ex, ey = exceptions
@@ -133,6 +140,8 @@ class SegmentColumns(Mapping):
         return self._exc is not None
 
     def __getitem__(self, key):
+        if self.lengths_only and key in self.KEYS and key not in self._keys:
+            raise KeyError(f"{key!r}: {LENGTHS_ONLY_MSG}")
         if key not in self._cols:
             if key == "len" and self._exc is not None:
                 # Segment(p, q): norm(p - q) (src/segment.jl:32) with the operations of the device code, in the same order:
@@ -151,13 +160,15 @@ class SegmentColumns(Mapping):
         return self._cols[key]
 
     def __iter__(self):
-        return iter(self.KEYS)
+        return iter(self._keys)
 
     def __len__(self):
-        return len(self.KEYS)
+        return len(self._keys)
 
     def p_range(self, lo, hi):
         """(px, py) of the segments [lo, hi) of the resident batch without rebuilding the whole columns"""
+        if self.lengths_only:
+            raise KeyError(LENGTHS_ONLY_MSG)
         if "px" in self._cols:
             return self._cols["px"][lo:hi], self._cols["py"][lo:hi]
         idx, ex, ey = self._exc
@@ -192,6 +203,8 @@ class SegmentList:
             i += n
         if not 0 <= i < n:
             raise IndexError(i)
+        if self._tg._lengths_only:
+            raise RuntimeError(f"a Segment needs p and q: {LENGTHS_ONLY_MSG} (read tg.segments['len'] / ['element'])")
         s, o = self._tg.segments, self._lo + i
         if self._p is None:
             self._p = s.p_range(self._lo, self._hi)
@@ -378,6 +391,7 @@ class TrackGenerator(TrackLayout):
         self._offsets = None
         self._resident = None
         self._in_batch = False  # inside the on_batch of segmentize_: the batch it received is resident
+        self._lengths_only = False  # the last segmentize_ wrote only len and element (RT_SEG_LENGTHS_ONLY)
         self.volume_factors = None
         self.n_segments = 0
 
@@ -477,7 +491,8 @@ class TrackGenerator(TrackLayout):
 
     @property
     def segments(self):
-        """SoA dict px, py, qx, qy, len, element of the resident batch (the whole shard when it fitted)."""
+        """SoA dict px, py, qx, qy, len, element of the resident batch (the whole shard when it fitted); len and element only
+        after ``segmentize_(..., lengths_only=True)``."""
         if self._segments is None:
             self.fetch_segments()
         return self._segments
@@ -502,13 +517,18 @@ class TrackGenerator(TrackLayout):
         positions where p is not the preceding q; ``px`` / ``py`` are rebuilt on the host on first use (SegmentColumns).
         ``compact="q"`` leaves ``len`` on the device as well (20 bytes per segment): it is rebuilt as norm(p - q) with the same
         IEEE operations (not after ``correct_volumes``, which rescales the resident lengths).
-        Inside ``on_batch`` of segmentize_ it copies the batch the callback received."""
+        Inside ``on_batch`` of segmentize_ it copies the batch the callback received.  After ``segmentize_(..., lengths_only=True)``
+        it copies len and element (12 bytes per segment); ``compact`` is then an error."""
         if not self._resident_valid():
             raise RuntimeError("call segmentize_ first")
+        if compact and self._lengths_only:
+            raise RuntimeError(f"fetch_segments(compact=...) sends q and rebuilds p: {LENGTHS_ONLY_MSG}")
         L = _lib.lib()
         n = self.resident_batch()[3]
         names = [("px", np.float64), ("py", np.float64), ("qx", np.float64), ("qy", np.float64), ("len", np.float64),
                  ("element", np.int32)]
+        if self._lengths_only:
+            names = names[4:]
         if compact:
             names = names[2:]
             if compact == "q":
@@ -525,8 +545,8 @@ class TrackGenerator(TrackLayout):
 
         out = {name: buffer(name, dt, n) for name, dt in names}
         if not compact:
-            _lib.check(self._ctx, L.rt_segments_download(self._ctx, *[_lib.ptr(out[k]) for k, _ in names]))
-            self._segments = SegmentColumns(out)
+            _lib.check(self._ctx, L.rt_segments_download(self._ctx, *[_lib.ptr(out.get(k)) for k in SegmentColumns.KEYS]))
+            self._segments = SegmentColumns(out, lengths_only=self._lengths_only)
             return self._segments
         cap = max(getattr(self, "_exc_cap", 0), 4 * (self.uid_end - self.uid_begin) + n // 64 + 1024) if max_exceptions is None else int(max_exceptions)
         for _ in range(2):
@@ -730,19 +750,22 @@ class DeviceColumn:
 
 class SegmentBatch:
     """One uid batch of Segment records as produced on the device (``rt_batch`` of include/rt_b200.h): what an on-GPU consumer
-    (a transport sweep) sees when the shard's segments do not fit in memory at once."""
+    (a transport sweep) sees when the shard's segments do not fit in memory at once.  ``px``, ``py``, ``qx``, ``qy`` are None
+    after ``segmentize_(..., lengths_only=True)``."""
 
     def __init__(self, b):
         self.uid_begin, self.uid_end, self.n_segments = int(b.uid_begin), int(b.uid_end), int(b.n_segments)
         self.offset_base, self.attempt, self.stream = int(b.offset_base), int(b.attempt), b.stream
         self.d_offsets = b.d_offsets  # device pointer: int64 offsets of the shard's tracks (n_shard + 1)
         n = self.n_segments
-        self.px, self.py, self.qx, self.qy, self.len = (DeviceColumn(p, n, "<f8") for p in (b.d_px, b.d_py, b.d_qx, b.d_qy, b.d_len))
+        self.px, self.py, self.qx, self.qy = (DeviceColumn(p, n, "<f8") if p else None for p in (b.d_px, b.d_py, b.d_qx, b.d_qy))
+        self.len = DeviceColumn(b.d_len, n, "<f8")
         self.element = DeviceColumn(b.d_element, n, "<i4")
 
 
 def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flags: int = 0, max_iter: int = MAX_ITER,
-                check: bool = True, fetch_volumes: bool = True, on_batch=None, exact_volumes: bool = False) -> TrackGenerator:
+                check: bool = True, fetch_volumes: bool = True, on_batch=None, exact_volumes: bool = False,
+                lengths_only: bool = False) -> TrackGenerator:
     """segmentize!(tg; k, rtol): count pass -> scan -> fill pass (+ fused fill_volumes) on the device.
     ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits).  Inside it
     ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()`` and ``tg.correct_volumes()`` act
@@ -760,10 +783,17 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
     walk order -- so that they are bit-equal to fill_volumes and the same whatever the run, pipeline, knobs, segment capacity or
     number of ranks; the default sums them with atomics, whose last bits vary.  It cannot be combined with RT_SEG_COUNT_ONLY or
     RT_SEG_NO_VOLUMES, and with a communicator of several ranks each shard must fit in one batch and the shards must be in
-    ascending uid order by rank."""
+    ascending uid order by rank.
+
+    ``lengths_only=True`` (RT_SEG_LENGTHS_ONLY) writes only the len and element columns, 12 instead of 44 bytes per segment, for
+    consumers that never read the end points (``optical_lengths``, ``correct_volumes``, an on-device sweep): everything else is
+    computed as without it, and len / element are the same bits.  ``tg.segments`` then has only ``len`` and ``element``,
+    ``SegmentBatch`` gives None for the end-point columns, and ``track.segments[i]`` and ``fetch_segments(compact=...)`` raise."""
     L = _lib.lib()
     if exact_volumes:
         flags |= _lib.RT_SEG_EXACT_VOLUMES
+    if lengths_only:
+        flags |= _lib.RT_SEG_LENGTHS_ONLY
     cb = None
     if on_batch is not None:
         def _cb(bptr, _user):
@@ -783,6 +813,7 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
         raise RuntimeError("Segmentation is intended after tracing. Please, call `trace!` first!")
     tg._segmented = False
     tg._segments = tg._offsets = tg._resident = None
+    tg._lengths_only = bool(flags & _lib.RT_SEG_LENGTHS_ONLY) and not flags & _lib.RT_SEG_COUNT_ONLY
     tg.volume_factors = None
     nseg, bad_uid, bad_status = C.c_int64(0), C.c_int64(0), C.c_int32(0)
     delta = tg.azimuthal_quadrature.deltas

@@ -18,6 +18,9 @@
 // iteration are contiguous (coalesced), and the per-track length sum needs one atomic per chunk.  Per segment the kernel
 // gathers ONE 32-byte sector (the EdgeRec), executes ~45 FP64 instructions (one shared reciprocal, one square root) and
 // writes 44 bytes: the HBM write stream of the Segment columns is its roofline.
+//
+// POINTS = false (RT_SEG_LENGTHS_ONLY): p and q are still evaluated in registers -- l = norm(p - q) and the verification need
+// them -- but only len and element are stored, 12 instead of 44 bytes per segment.
 #pragma once
 #include "walk.cuh"
 
@@ -55,6 +58,7 @@ __device__ __forceinline__ bool eval3_cross(const Line &trk, const Line &L, P2 &
     return par;
 }
 
+template <bool POINTS>
 __global__ void __launch_bounds__(kEval3Threads, RT_EVAL3_MIN_BLOCKS) k_eval3(const __grid_constant__ WalkParams P) {
     const unsigned FULL = 0xffffffffu;
     const DevMesh &m = P.m;
@@ -181,10 +185,12 @@ __global__ void __launch_bounds__(kEval3Threads, RT_EVAL3_MIN_BLOCKS) k_eval3(co
             const double l = sqrt(dx * dx + dy * dy);  // Segment(p, q): norm(p - q), src/segment.jl:32
             // (plain stores: an evict-first policy or st.cs on the output stream measures 1 % slower, write-through the same)
             const long long so = base + v;
-            P.opx[so] = p.x;
-            P.opy[so] = p.y;
-            P.oqx[so] = q.x;
-            P.oqy[so] = q.y;
+            if (POINTS) {
+                P.opx[so] = p.x;
+                P.opy[so] = p.y;
+                P.oqx[so] = q.x;
+                P.oqy[so] = q.y;
+            }
             P.olen[so] = l;
             P.oelem[so] = (int)cell + 1;
             if (P.vol) atomicAdd(&P.vol[cell], delta * l);  // volumes[i] += delta_s[a]*l, src/trackgenerator.jl:382
@@ -217,10 +223,12 @@ __global__ void __launch_bounds__(kEval3Threads, RT_EVAL3_MIN_BLOCKS) k_eval3(co
                 intersections(m, cell, trk, right, p, q, e_p, e_q);
                 const double l = norm2(p.x - q.x, p.y - q.y);
                 const long long so = base + v;
-                P.opx[so] = p.x;
-                P.opy[so] = p.y;
-                P.oqx[so] = q.x;
-                P.oqy[so] = q.y;
+                if (POINTS) {
+                    P.opx[so] = p.x;
+                    P.opy[so] = p.y;
+                    P.oqx[so] = q.x;
+                    P.oqy[so] = q.y;
+                }
                 P.olen[so] = l;
                 P.oelem[so] = cell + 1;
                 if (P.vol) atomicAdd(&P.vol[cell], delta * l);

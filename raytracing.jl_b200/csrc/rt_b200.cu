@@ -164,8 +164,10 @@ struct rt_ctx {
     long long cap_cfg = 0;  // user limit on resident segments (0 = as many as fit)
     long long cap = 0;      // allocated
     DevBuf b_seg_d, b_seg_e;
-    double *s_px = nullptr, *s_py = nullptr, *s_qx = nullptr, *s_qy = nullptr, *s_len = nullptr;
+    double *s_px = nullptr, *s_py = nullptr, *s_qx = nullptr, *s_qy = nullptr, *s_len = nullptr;  // (s_px .. s_qy: NULL in the lengths-only layout)
     int *s_elem = nullptr;
+    bool cols_points = false;  // the allocated columns hold px, py, qx, qy (44 bytes per segment) or only len, element (12 bytes)
+    bool lengths_only = false; // the last rt_segmentize (and its resident batch) wrote only len and element (RT_SEG_LENGTHS_ONLY)
     long long res_trk_begin = 0, res_trk_end = 0, res_off_base = 0, res_nseg = 0;  // resident batch (shard-local)
     bool vol_valid = false;
     // Inside the batch callback of rt_segmentize the resident batch is valid although the call has not finished (`segmented` is
@@ -838,21 +840,29 @@ extern "C" int rt_set_segment_capacity(rt_ctx *ctx, int64_t max_segments_residen
     return RT_OK;
 }
 
+// the allocated columns take `want` segments of the current call's layout (a lengths-only call also writes into the len and element
+// columns of the full layout; a default call needs the columns of p and q)
+static bool columns_fit(const rt_ctx *ctx, long long want) {
+    return ctx->b_seg_d.p && want <= ctx->cap && (ctx->cols_points || ctx->lengths_only);
+}
+
 static int ensure_segment_buffers(rt_ctx *ctx, long long want) {
-    if (want <= ctx->cap && ctx->b_seg_d.p) return RT_OK;
+    if (columns_fit(ctx, want)) return RT_OK;
     release(ctx->b_seg_d);
     release(ctx->b_seg_e);
     ctx->cap = 0;
+    const bool points = !ctx->lengths_only;
     size_t n = ((size_t)std::max<long long>(want, 1) + 15) & ~(size_t)15;  // every SoA column stays 32-byte aligned
-    CK(ensure(ctx->b_seg_d, sizeof(double) * 5 * n));
+    CK(ensure(ctx->b_seg_d, sizeof(double) * (points ? 5 : 1) * n));
     CK(ensure(ctx->b_seg_e, sizeof(int) * n));
     double *d = (double *)ctx->b_seg_d.p;
-    ctx->s_px = d;
-    ctx->s_py = d + n;
-    ctx->s_qx = d + 2 * n;
-    ctx->s_qy = d + 3 * n;
-    ctx->s_len = d + 4 * n;
+    ctx->s_px = points ? d : nullptr;
+    ctx->s_py = points ? d + n : nullptr;
+    ctx->s_qx = points ? d + 2 * n : nullptr;
+    ctx->s_qy = points ? d + 3 * n : nullptr;
+    ctx->s_len = points ? d + 4 * n : d;
     ctx->s_elem = (int *)ctx->b_seg_e.p;
+    ctx->cols_points = points;
     ctx->cap = (long long)n;
     return RT_OK;
 }
@@ -898,20 +908,23 @@ static void set_resident(rt_ctx *ctx, long long trk_begin, long long trk_end, lo
 
 // the Segment columns the fill / evaluation writes
 static void bind_columns(const rt_ctx *ctx, WalkParams &P) {
-    P.opx = ctx->s_px;
-    P.opy = ctx->s_py;
-    P.oqx = ctx->s_qx;
-    P.oqy = ctx->s_qy;
+    const bool points = !ctx->lengths_only;
+    P.opx = points ? ctx->s_px : nullptr;
+    P.opy = points ? ctx->s_py : nullptr;
+    P.oqx = points ? ctx->s_qx : nullptr;
+    P.oqy = points ? ctx->s_qy : nullptr;
     P.olen = ctx->s_len;
     P.oelem = ctx->s_elem;
 }
 
 // Segment columns sized from free memory (0.92 x free / 44 bytes per segment, counting the columns held now; 68 bytes and the
-// sorted pairs held now with exact volumes) for `want` segments (already limited by the capacity option): one batch takes what it
-// needs if that fits, a walk in several batches everything that fits.  *cap: the capacity to cut the batches with.
+// sorted pairs held now with exact volumes; 12 and 36 bytes with RT_SEG_LENGTHS_ONLY) for `want` segments (already limited by the
+// capacity option): one batch takes what it needs if that fits, a walk in several batches everything that fits.  *cap: the
+// capacity to cut the batches with.
 static int size_columns(rt_ctx *ctx, long long want, bool take_all, size_t free_b, long long *cap) {
     const size_t held = ctx->b_seg_d.bytes + ctx->b_seg_e.bytes + (ctx->exact ? ctx->b_ex_key.bytes + ctx->b_ex_val.bytes : 0);
-    const long long fit = (long long)((double)(free_b + held) * 0.92 / (ctx->exact ? 68.0 : 44.0));
+    const double per_segment = (ctx->lengths_only ? 12.0 : 44.0) + (ctx->exact ? 24.0 : 0.0);
+    const long long fit = (long long)((double)(free_b + held) * 0.92 / per_segment);
     *cap = take_all ? fit : std::min(want, fit);
     if (ctx->cap_cfg > 0) *cap = std::min(*cap, (long long)ctx->cap_cfg);
     return ensure_segment_buffers(ctx, *cap);
@@ -1162,7 +1175,11 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         PE.lmin = lmin_eval;
         PE.cancel = cancel;
         if (PE.ch.order) PE.ch.order = ctx->order_eval;
-        k_eval3<<<blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads), kEval3Threads, 0, st>>>(PE);
+        const unsigned blocks = blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads);
+        if (ctx->lengths_only)
+            k_eval3<false><<<blocks, kEval3Threads, 0, st>>>(PE);
+        else
+            k_eval3<true><<<blocks, kEval3Threads, 0, st>>>(PE);
     };
 
     // ---- memory plan
@@ -1264,7 +1281,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         tic(ctx, 3);
         // (exact volumes size their sort from the segment total on the host: never optimistic)
         const bool optimistic = !multi && !a.cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
-                                ctx->fit_gen == ctx->trace_gen && ctx->b_seg_d.p && ctx->cap > 0 && !ctx->exact;
+                                ctx->fit_gen == ctx->trace_gen && columns_fit(ctx, 1) && !ctx->exact;
         ScanGuard guard{};
         if (optimistic) guard = ScanGuard{d_guard(ctx), base, ctx->cap, P.pool_cursor, P.pool_blocks};
         CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p + b, (long long *)ctx->b_offsets.p + b, e - b, base, guard)));
@@ -1300,7 +1317,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         ctx->total_segments = base + batch_total;
         // ---- Segment columns: everything of this batch if it fits, else as much as fits
         const long long want = ctx->cap_cfg > 0 ? std::min(batch_total, (long long)ctx->cap_cfg) : batch_total;
-        if (want > ctx->cap || !ctx->b_seg_d.p) {
+        if (!columns_fit(ctx, want)) {
             CK(query_mem());
             long long fitted = 0;
             int rc = size_columns(ctx, want, multi, free_b, &fitted);
@@ -1440,10 +1457,15 @@ static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool 
             rc = cut_batch(ctx, P, h_off, 0, h_unit_base, b, cap, &nseg);
             if (rc) return rc;
         }
-        if (ctx->mixed)
-            k_walk<true, true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        const unsigned blocks = blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads);
+        if (ctx->mixed && ctx->lengths_only)
+            k_walk<true, true, false><<<blocks, kWalkThreads, 0, st>>>(P);
+        else if (ctx->mixed)
+            k_walk<true, true><<<blocks, kWalkThreads, 0, st>>>(P);
+        else if (ctx->lengths_only)
+            k_walk<true, false, false><<<blocks, kWalkThreads, 0, st>>>(P);
         else
-            k_walk<true><<<blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
+            k_walk<true><<<blocks, kWalkThreads, 0, st>>>(P);
         a.launches += 1;
         if (hybrid) {
             launch_track_status(ctx, P, a.rtol, nullptr, nullptr);
@@ -1597,6 +1619,8 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
     // cap, blind to an error or the track end in an earlier chunk) and the fix-up cannot take back what a dropped chunk added.
     // One walker per track stops exactly where the reference loop does.
     if ((flags & RT_SEG_COUNT_ONLY) && want_vol) flags |= RT_SEG_NO_CHUNKS;
+    // (count-only writes no columns: the flag changes nothing there)
+    ctx->lengths_only = (flags & RT_SEG_LENGTHS_ONLY) && !(flags & RT_SEG_COUNT_ONLY);
     if (!ctx->mixed && ctx->clear_tiny != tiny_step) {
         k_finalize_clear<<<blocks_for(m.n_cells, 128), 128, 0, st>>>(m, (CellRec *)ctx->b_cells.p, (HalfEdge *)ctx->b_he.p,
                                                                      (const float *)ctx->b_qual.p, (const float *)ctx->b_bdist.p,
@@ -1675,6 +1699,9 @@ extern "C" int rt_segment_offsets(rt_ctx *ctx, int64_t *offsets, int32_t *status
 
 extern "C" int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double *qy, double *len, int32_t *element) {
     if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_segments_download: call rt_segmentize first");
+    if (ctx->lengths_only && (px || py || qx || qy))
+        return fail(ctx, RT_ERR_ARG, "rt_segments_download: the resident batch was produced with RT_SEG_LENGTHS_ONLY and has no p / q "
+                    "columns (pass NULL for px, py, qx, qy)");
     CK(cudaSetDevice(ctx->device));
     size_t n = (size_t)ctx->res_nseg;
     if (n == 0) return RT_OK;
@@ -1692,6 +1719,9 @@ extern "C" int rt_segments_download(rt_ctx *ctx, double *px, double *py, double 
 extern "C" int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy, double *len, int32_t *element, int64_t max_exceptions,
                                             int64_t *exc_index, double *exc_px, double *exc_py, int64_t *n_exceptions) {
     if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: call rt_segmentize first");
+    if (ctx->lengths_only)
+        return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: the resident batch was produced with RT_SEG_LENGTHS_ONLY: "
+                    "there is no q to send and no p to rebuild (use rt_segments_download with len and element)");
     if (max_exceptions < 0 || !n_exceptions || (max_exceptions > 0 && (!exc_index || !exc_px || !exc_py)))
         return fail(ctx, RT_ERR_ARG, "rt_segments_download_compact: bad exception buffers");
     CK(cudaSetDevice(ctx->device));
@@ -1743,10 +1773,11 @@ extern "C" int rt_segments_device(rt_ctx *ctx, rt_batch *view) {
     view->n_segments = ctx->res_nseg;
     view->d_offsets = (const int64_t *)ctx->b_offsets.p;
     view->offset_base = ctx->res_off_base;
-    view->d_px = ctx->s_px;
-    view->d_py = ctx->s_py;
-    view->d_qx = ctx->s_qx;
-    view->d_qy = ctx->s_qy;
+    const bool points = !ctx->lengths_only;
+    view->d_px = points ? ctx->s_px : nullptr;
+    view->d_py = points ? ctx->s_py : nullptr;
+    view->d_qx = points ? ctx->s_qx : nullptr;
+    view->d_qy = points ? ctx->s_qy : nullptr;
     view->d_len = ctx->s_len;
     view->d_element = ctx->s_elem;
     view->stream = (void *)ctx->stream;

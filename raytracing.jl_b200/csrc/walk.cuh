@@ -446,14 +446,17 @@ __device__ RT_LITERAL_CALL void literal_until_push(const WalkParams &P, const Li
 }
 
 // ---- the walk ----------------------------------------------------------------------------------------------
-template <bool FILL, bool MIXED = false>
+// POINTS = false (RT_SEG_LENGTHS_ONLY, fill pass only): the ring stages and the flushes write len and element alone
+template <bool FILL, bool MIXED = false, bool POINTS = true>
 __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const __grid_constant__ WalkParams P) {
     const unsigned FULL = 0xffffffffu;
     const DevMesh &m = P.m;
     // fill pass: every thread stages its segments in a ring of kStage slots and writes complete, aligned groups of four as full
     // 32-byte sectors; the flushes happen at points that are uniform across the warp (every fourth fast iteration and once per
     // outer iteration), so the lanes of a warp execute them together although their output positions differ modulo 4
-    __shared__ double s_buf[FILL ? 5 * kStage * kWalkThreads : 1];
+    constexpr int kCols = POINTS ? 5 : 1;  // staged double columns: px, py, qx, qy, len / len
+    constexpr int kLen = kCols - 1;
+    __shared__ double s_buf[FILL ? kCols * kStage * kWalkThreads : 1];
     __shared__ int s_el[FILL ? kStage * kWalkThreads : 1];
     const int tid = threadIdx.x;
     long long gw = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
@@ -566,11 +569,13 @@ __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const
         if ((wpos & 3) && head <= stop) {
             for (; wpos < head; ++wpos) {
                 const int kk = (int)(wpos & (kStage - 1));
-                P.opx[wpos] = s_buf[(0 * kStage + kk) * kWalkThreads + tid];
-                P.opy[wpos] = s_buf[(1 * kStage + kk) * kWalkThreads + tid];
-                P.oqx[wpos] = s_buf[(2 * kStage + kk) * kWalkThreads + tid];
-                P.oqy[wpos] = s_buf[(3 * kStage + kk) * kWalkThreads + tid];
-                P.olen[wpos] = s_buf[(4 * kStage + kk) * kWalkThreads + tid];
+                if (POINTS) {
+                    P.opx[wpos] = s_buf[(0 * kStage + kk) * kWalkThreads + tid];
+                    P.opy[wpos] = s_buf[(1 * kStage + kk) * kWalkThreads + tid];
+                    P.oqx[wpos] = s_buf[(2 * kStage + kk) * kWalkThreads + tid];
+                    P.oqy[wpos] = s_buf[(3 * kStage + kk) * kWalkThreads + tid];
+                }
+                P.olen[wpos] = s_buf[(kLen * kStage + kk) * kWalkThreads + tid];
                 P.oelem[wpos] = s_el[kk * kWalkThreads + tid];
             }
         }
@@ -578,10 +583,11 @@ __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const
             const int k0 = (int)(wpos & (kStage - 1));
             double *dst[5] = {P.opx, P.opy, P.oqx, P.oqy, P.olen};
 #pragma unroll
-            for (int a = 0; a < 5; ++a)
-                stg256_stream(dst[a] + wpos, pol_stream, s_buf[(a * kStage + k0 + 0) * kWalkThreads + tid],
-                              s_buf[(a * kStage + k0 + 1) * kWalkThreads + tid], s_buf[(a * kStage + k0 + 2) * kWalkThreads + tid],
-                              s_buf[(a * kStage + k0 + 3) * kWalkThreads + tid]);
+            for (int a = POINTS ? 0 : 4; a < 5; ++a)
+                stg256_stream(dst[a] + wpos, pol_stream, s_buf[((a - 4 + kLen) * kStage + k0 + 0) * kWalkThreads + tid],
+                              s_buf[((a - 4 + kLen) * kStage + k0 + 1) * kWalkThreads + tid],
+                              s_buf[((a - 4 + kLen) * kStage + k0 + 2) * kWalkThreads + tid],
+                              s_buf[((a - 4 + kLen) * kStage + k0 + 3) * kWalkThreads + tid]);
             stg128_stream(P.oelem + wpos, pol_stream, s_el[(k0 + 0) * kWalkThreads + tid], s_el[(k0 + 1) * kWalkThreads + tid],
                           s_el[(k0 + 2) * kWalkThreads + tid], s_el[(k0 + 3) * kWalkThreads + tid]);
             wpos += 4;
@@ -589,11 +595,13 @@ __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const
         if (all) {
             for (; wpos < o_next; ++wpos) {
                 const int kk = (int)(wpos & (kStage - 1));
-                P.opx[wpos] = s_buf[(0 * kStage + kk) * kWalkThreads + tid];
-                P.opy[wpos] = s_buf[(1 * kStage + kk) * kWalkThreads + tid];
-                P.oqx[wpos] = s_buf[(2 * kStage + kk) * kWalkThreads + tid];
-                P.oqy[wpos] = s_buf[(3 * kStage + kk) * kWalkThreads + tid];
-                P.olen[wpos] = s_buf[(4 * kStage + kk) * kWalkThreads + tid];
+                if (POINTS) {
+                    P.opx[wpos] = s_buf[(0 * kStage + kk) * kWalkThreads + tid];
+                    P.opy[wpos] = s_buf[(1 * kStage + kk) * kWalkThreads + tid];
+                    P.oqx[wpos] = s_buf[(2 * kStage + kk) * kWalkThreads + tid];
+                    P.oqy[wpos] = s_buf[(3 * kStage + kk) * kWalkThreads + tid];
+                }
+                P.olen[wpos] = s_buf[(kLen * kStage + kk) * kWalkThreads + tid];
                 P.oelem[wpos] = s_el[kk * kWalkThreads + tid];
             }
         }
@@ -602,11 +610,13 @@ __global__ void __launch_bounds__(kWalkThreads, RT_WALK_MIN_BLOCKS) k_walk(const
     auto push = [&](int e, double ax, double ay, double bx, double by, double l) {
         if (FILL) {
             const int k = (int)((out + nseg) & (kStage - 1));
-            s_buf[(0 * kStage + k) * kWalkThreads + tid] = ax;
-            s_buf[(1 * kStage + k) * kWalkThreads + tid] = ay;
-            s_buf[(2 * kStage + k) * kWalkThreads + tid] = bx;
-            s_buf[(3 * kStage + k) * kWalkThreads + tid] = by;
-            s_buf[(4 * kStage + k) * kWalkThreads + tid] = l;
+            if (POINTS) {
+                s_buf[(0 * kStage + k) * kWalkThreads + tid] = ax;
+                s_buf[(1 * kStage + k) * kWalkThreads + tid] = ay;
+                s_buf[(2 * kStage + k) * kWalkThreads + tid] = bx;
+                s_buf[(3 * kStage + k) * kWalkThreads + tid] = by;
+            }
+            s_buf[(kLen * kStage + k) * kWalkThreads + tid] = l;
             s_el[k * kWalkThreads + tid] = e + 1;
         }
         if (P.vol) atomicAdd(&P.vol[e], P.ang.delta_eff[az] * l);  // volumes[i] += delta_s[a]*l, src/trackgenerator.jl:382
