@@ -272,9 +272,8 @@ int rt_comm_init(rt_ctx *ctx, int32_t n_ranks, int32_t rank, const char id[128])
  * nearest-node queries, knn queries, count-pass ms, fill-pass ms, scan+volumes ms. */
 int rt_stats(rt_ctx *ctx, double stats[8]);
 /* named scalars: "verify_fallbacks", "n_units", "segment_capacity" (segments the allocated columns hold, in the layout of the last
- * rt_segmentize), "count_batches"
- * (uid batches of the single-walk pipeline's count walk) of the last rt_segmentize; "optimistic_cancels" (calls of this context
- * whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
+ * rt_segmentize), "count_batches" (uid batches of the count walk of the last rt_segmentize: 0 for an empty shard, else 1 in
+ * pipelines 0 and 1, which walk the shard in one batch); "optimistic_cancels" (calls of this context whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
  * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose
  * rt_segmentize failed: the ranks of a communicator that call rt_volumes as documented below agree on it); "rho", "band_cost"
  * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths; "locate_knn" (points that entered the k-nearest-node

@@ -104,7 +104,7 @@ struct rt_ctx {
     DevBuf b_scratch, b_gcounts, b_gcursor;  // rt_mesh_upload staging (kept between uploads)
     DevBuf b_tsum;    // self-verifying pipelines: per-track length sums
     DevBuf b_pool, b_pool_next, b_pool_cursor;  // single-walk pipeline: record blocks (walk.cuh kRecBlock), chain, cursor
-    int count_batches = 0;             // single-walk pipeline: how many uid batches the count walk needed (info)
+    int count_batches = 0;             // how many uid batches the count walk needed (info; 0 for an empty shard, else 1 in pipelines 0 and 1)
     // The chunk plan (k_plan_chunks .. k_unit_scatter) depends on the tracks, the mesh density and the chunk options only: it is
     // kept between calls and rebuilt when one of them changes (plan_key), so the steady-state segmentize! needs neither its
     // kernels nor the host round trip that sizes its arrays.
@@ -118,7 +118,6 @@ struct rt_ctx {
         bool operator==(const PlanKey &o) const { return gen == o.gen && chunk_len == o.chunk_len && band == o.band && order_grid == o.order_grid && n == o.n &&
                    band_min == o.band_min && band_div == o.band_div; }
     } plan_key;
-    bool plan_has_order = false;
     int opt_debug_clear_pool = 0;      // test hook (initcheck): zero the record pool before every walk, so that the evaluation's speculative
                                        // load of a chunk's first records (issued before its count is known) never reads unwritten words
     double opt_band_cost = 28.0;       // shard planning: cost of one boundary-band cell in fast transitions (measured: cfg4 on 8 GPUs)
@@ -145,7 +144,7 @@ struct rt_ctx {
     int opt_pipeline = 3;              // 3: single walk (k_march counts AND records, k_eval3 evaluates) [default]; 0: hybrid (k_march without records
                                        // counts, geometric fill walk), 1: sequential (walk.cuh only); 3 falls back to 0 (pool exhausted) or 1, 0 falls back to 1
     int verify_fallbacks = 0;
-    int opt_debug_verify_fail = 0;     // test hook: make the verification of the two-stage pipeline fail
+    int opt_debug_verify_fail = 0;     // test hook: make the verification of pipelines 3 and 0 fail
     double tau_ms = 0.0;
     cudaEvent_t ev2[2] = {nullptr, nullptr};  // kernel stopwatch of the synchronous exports (rt_optical_lengths, rt_find_elements)
     DevBuf b_loc_xy, b_loc_elem, b_loc_knn;   // rt_find_elements: points, element ids, k-nearest branch counter
@@ -163,9 +162,7 @@ struct rt_ctx {
     long long total_segments = 0;
     long long cap_cfg = 0;  // user limit on resident segments (0 = as many as fit)
     long long cap = 0;      // allocated
-    DevBuf b_seg_d, b_seg_e;
-    double *s_px = nullptr, *s_py = nullptr, *s_qx = nullptr, *s_qy = nullptr, *s_len = nullptr;  // (s_px .. s_qy: NULL in the lengths-only layout)
-    int *s_elem = nullptr;
+    DevBuf b_seg_d, b_seg_e;   // Segment columns of `cap` segments each (seg_columns): px, py, qx, qy, len | element
     bool cols_points = false;  // the allocated columns hold px, py, qx, qy (44 bytes per segment) or only len, element (12 bytes)
     bool lengths_only = false; // the last rt_segmentize (and its resident batch) wrote only len and element (RT_SEG_LENGTHS_ONLY)
     long long res_trk_begin = 0, res_trk_end = 0, res_off_base = 0, res_nseg = 0;  // resident batch (shard-local)
@@ -855,16 +852,23 @@ static int ensure_segment_buffers(rt_ctx *ctx, long long want) {
     size_t n = ((size_t)std::max<long long>(want, 1) + 15) & ~(size_t)15;  // every SoA column stays 32-byte aligned
     CK(ensure(ctx->b_seg_d, sizeof(double) * (points ? 5 : 1) * n));
     CK(ensure(ctx->b_seg_e, sizeof(int) * n));
-    double *d = (double *)ctx->b_seg_d.p;
-    ctx->s_px = points ? d : nullptr;
-    ctx->s_py = points ? d + n : nullptr;
-    ctx->s_qx = points ? d + 2 * n : nullptr;
-    ctx->s_qy = points ? d + 3 * n : nullptr;
-    ctx->s_len = points ? d + 4 * n : d;
-    ctx->s_elem = (int *)ctx->b_seg_e.p;
     ctx->cols_points = points;
     ctx->cap = (long long)n;
     return RT_OK;
+}
+
+// The Segment columns of the current call: px .. qy are NULL when it asked for RT_SEG_LENGTHS_ONLY, also when the allocation holds
+// them, and whenever the allocation does not
+struct SegColumns {
+    double *px, *py, *qx, *qy, *len;
+    int *elem;
+};
+static SegColumns seg_columns(const rt_ctx *ctx) {
+    double *d = (double *)ctx->b_seg_d.p;
+    const size_t n = (size_t)ctx->cap;
+    const bool points = ctx->cols_points && !ctx->lengths_only;
+    return {points ? d : nullptr, points ? d + n : nullptr, points ? d + 2 * n : nullptr, points ? d + 3 * n : nullptr,
+            ctx->cols_points ? d + 4 * n : d, (int *)ctx->b_seg_e.p};
 }
 
 // fast transitions only accept chords that are certainly not dropped by isapprox(p, q) (src/track.jl:156) and long enough for
@@ -892,7 +896,6 @@ struct Attempt {
     int index;                    // rt_batch::attempt
     Next next = Next::Done;
     double launches = 0;          // kernel launches (stats[0] when this attempt is the final one)
-    bool first_bad_scan = false;  // k_first_bad finds the first failing track (the single walk's k_track_status reports it itself)
     bool defer_verify = false;    // the verification flag arrives with the final control read-back
     bool defer_total = false;     // ... and so do the segment total and the guard of the optimistic evaluation
 };
@@ -908,13 +911,13 @@ static void set_resident(rt_ctx *ctx, long long trk_begin, long long trk_end, lo
 
 // the Segment columns the fill / evaluation writes
 static void bind_columns(const rt_ctx *ctx, WalkParams &P) {
-    const bool points = !ctx->lengths_only;
-    P.opx = points ? ctx->s_px : nullptr;
-    P.opy = points ? ctx->s_py : nullptr;
-    P.oqx = points ? ctx->s_qx : nullptr;
-    P.oqy = points ? ctx->s_qy : nullptr;
-    P.olen = ctx->s_len;
-    P.oelem = ctx->s_elem;
+    const SegColumns c = seg_columns(ctx);
+    P.opx = c.px;
+    P.opy = c.py;
+    P.oqx = c.qx;
+    P.oqy = c.qy;
+    P.olen = c.len;
+    P.oelem = c.elem;
 }
 
 // Segment columns sized from free memory (0.92 x free / 44 bytes per segment, counting the columns held now; 68 bytes and the
@@ -1151,46 +1154,22 @@ static int plan_chunks(rt_ctx *ctx, WalkParams &P, uint32_t flags, double *launc
     return RT_OK;
 }
 
-// ---- single-walk pipeline (mode 3): k_march counts AND records every chunk in one walk, k_eval3 evaluates the records -------
-// The records live in a pool of kRecBlock-record blocks: block i < slots is the first block of chunk slot i of the batch, the
-// blocks behind are claimed by the walkers as they need them.  Shards whose pool would not fit next to the Segment columns are
-// processed in uid batches (whole 32-track blocks): count+record a batch, scan its offsets (carrying the running total), then
-// evaluate it -- in sub-batches when its segments exceed the resident capacity.  Next::Hybrid asks for the call to be repeated
-// with the hybrid pipeline (pool exhausted: the mesh is far denser along some chunks than the Cauchy-Crofton estimate).
-static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
-    cudaStream_t st = ctx->stream;
-    const long long n = ctx->n_shard;
-    const long long n_blocks = (n + 31) / 32;
-    const long long n_units = P.ch.n_units;
-    const size_t nn = (size_t)std::max<long long>(n, 1);
-    const int *order_all = P.ch.order;
-    CK(ensure(ctx->b_tsum, sizeof(double) * nn));  // (cleared per batch by k_seed, like the pool cursor and the volume accumulator)
-    CK(ensure(ctx->b_pool_cursor, sizeof(int)));
-    P.tsum = (double *)ctx->b_tsum.p;
-    P.pool_cursor = (int *)ctx->b_pool_cursor.p;
-    const double lmin_eval = ctx->opt_debug_verify_fail ? INFINITY : P.lmin;
-    // the evaluation of the records of the tracks and units P describes (cancel: the guard of the optimistic evaluation)
-    auto launch_eval = [&](const int *cancel) {
-        WalkParams PE = P;
-        PE.lmin = lmin_eval;
-        PE.cancel = cancel;
-        if (PE.ch.order) PE.ch.order = ctx->order_eval;
-        const unsigned blocks = blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads);
-        if (ctx->lengths_only)
-            k_eval3<false><<<blocks, kEval3Threads, 0, st>>>(PE);
-        else
-            k_eval3<true><<<blocks, kEval3Threads, 0, st>>>(PE);
-    };
+// ---- the pipelines -------------------------------------------------------------------------------------------------------------
+// Every pipeline walks the shard in uid batches of whole 32-track blocks -- seeds, count walk, per-track fix-up, offsets of the
+// batch carrying the running total -- and evaluates each batch into the Segment columns (evaluate_batch).  They differ in kernels:
+//   3 (single walk):  k_march counts AND records every chunk into the record pool (plan_pool), k_eval3 evaluates the records and
+//                     re-checks the geometric fast-path conditions, k_track_status runs the length check (src/track.jl:171-175).
+//                     A shard whose pool would not fit next to the Segment columns is walked in several batches.
+//   0 (hybrid):       k_march without a pool counts by sign tests, k_walk<true> fills and re-derives the same decisions from the
+//                     exact geometry (a fill that disagrees with the count fails the verification), k_track_status.
+//   1 (sequential):   k_walk<false> counts and k_fixup_tracks checks the lengths, k_walk<true> fills; nothing to verify.
+// Pipelines 0 and 1 walk the shard in one batch.
 
-    // ---- memory plan
-    size_t free_b = 0, total_b = 0;
-    bool have_mem = false;
-    auto query_mem = [&]() -> cudaError_t {
-        if (have_mem) return cudaSuccess;
-        have_mem = true;
-        return cudaMemGetInfo(&free_b, &total_b);
-    };
-    const long long slots_all = n_units * 32;
+// The record pool of pipeline 3: block i < slots is the first block of chunk slot i of a walk batch, the blocks behind are claimed
+// by the walkers as they need them.  Sized for every chunk slot of the shard if that fits next to the Segment columns, else for as
+// many as fit: *max_slots, the chunk slots of one walk batch.  Next::Hybrid when not even one block of 32 tracks fits.
+static int plan_pool(rt_ctx *ctx, WalkParams &P, Attempt &a, long long *max_slots_out) {
+    const long long slots_all = P.ch.n_units * 32;
     const double est_total = ctx->sum_len * crossings_per_length(ctx);
     const double extra_per_slot = est_total * ctx->opt_pool_extra / kRecBlock / (double)std::max<long long>(slots_all, 1);
     const size_t block_bytes = sizeof(int) * (kRecBlock + 1);  // records + chain entry
@@ -1200,7 +1179,8 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
     if (ctx->opt_pool_slots > 0) max_slots = std::min(max_slots, std::max<long long>(32, ctx->opt_pool_slots & ~31LL));
     const size_t pool_have = std::min<size_t>(ctx->b_pool.bytes / (sizeof(int) * kRecBlock), ctx->b_pool_next.bytes / sizeof(int));
     if ((size_t)blocks_for_slots(std::min(max_slots, slots_all)) > pool_have) {
-        CK(query_mem());
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
         const size_t avail = free_b + ctx->b_pool.bytes + ctx->b_pool_next.bytes + ctx->b_seg_d.bytes + ctx->b_seg_e.bytes;
         const size_t budget = (size_t)((double)avail * 0.15);  // ~9 pool bytes next to 44 Segment bytes per segment
         if ((size_t)blocks_for_slots(std::min(max_slots, slots_all)) * block_bytes > budget) {
@@ -1222,32 +1202,165 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
             release(ctx->b_pool_next);
             CK(ensure(ctx->b_pool, sizeof(int) * (size_t)pb * kRecBlock));
             CK(ensure(ctx->b_pool_next, sizeof(int) * (size_t)pb));
-            have_mem = false;
         }
     }
     P.pool = (int *)ctx->b_pool.p;
     P.pool_next = (int *)ctx->b_pool_next.p;
     P.pool_blocks = (int)std::min<size_t>(ctx->b_pool.bytes / (sizeof(int) * kRecBlock), ctx->b_pool_next.bytes / sizeof(int));
     if (ctx->opt_pool_extra <= 0.0) P.pool_blocks = (int)std::min<long long>(P.pool_blocks, blocks_for_slots(std::min(max_slots, slots_all)));
+    *max_slots_out = max_slots;
+    return RT_OK;
+}
 
-    const bool multi = max_slots < slots_all;
+// adds the stopwatch of phase ph to acc[ph] (the host has waited for its stop event)
+static void take_phase(rt_ctx *ctx, int ph, double *acc) {
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, ctx->pev[ph][0], ctx->pev[ph][1]) == cudaSuccess) acc[ph] += (double)ms;
+    ctx->pev_dirty[ph] = false;
+}
+
+// The evaluation of the tracks and units P describes: k_eval3 over the records in the evaluation's unit order (pipeline 3), else
+// the fill walk in the walk's order.  cancel: the guard of the optimistic evaluation.
+static void launch_eval(rt_ctx *ctx, const WalkParams &P, int mode, const int *cancel) {
+    cudaStream_t st = ctx->stream;
+    const bool points = !ctx->lengths_only;
+    WalkParams PE = P;
+    if (mode == 3) {
+        PE.lmin = ctx->opt_debug_verify_fail ? INFINITY : P.lmin;  // (test hook: no fast record passes the verification)
+        PE.cancel = cancel;
+        if (PE.ch.order) PE.ch.order = ctx->order_eval;
+        const unsigned blocks = blocks_for((PE.unit_end - PE.unit_begin) * 32 * 32, kEval3Threads);
+        if (points)
+            k_eval3<true><<<blocks, kEval3Threads, 0, st>>>(PE);
+        else
+            k_eval3<false><<<blocks, kEval3Threads, 0, st>>>(PE);
+        return;
+    }
+    PE.counters = nullptr;  // (the count walk has counted the steps)
+    const unsigned blocks = blocks_for((PE.unit_end - PE.unit_begin) * 32, kWalkThreads);
+    if (ctx->mixed && points)
+        k_walk<true, true><<<blocks, kWalkThreads, 0, st>>>(PE);
+    else if (ctx->mixed)
+        k_walk<true, true, false><<<blocks, kWalkThreads, 0, st>>>(PE);
+    else if (points)
+        k_walk<true><<<blocks, kWalkThreads, 0, st>>>(PE);
+    else
+        k_walk<true, false, false><<<blocks, kWalkThreads, 0, st>>>(PE);
+}
+
+// Evaluates the walk batch of tracks [P.trk_begin, P.trk_end) -- `base` segments before it, batch_total in it, its offsets on the
+// device -- in sub-batches that fit the resident capacity: evaluation, length check, verification, exact volumes, batch callback.
+// multi: the shard is walked in several batches.  acc: the phase times summed so far.
+static int evaluate_batch(rt_ctx *ctx, WalkParams &P, int mode, Attempt &a, long long base, long long batch_total, bool multi,
+                          std::vector<long long> &h_unit_base, double *acc) {
+    cudaStream_t st = ctx->stream;
+    const long long b = P.trk_begin, e = P.trk_end;
+    // ---- Segment columns: everything of this batch if it fits, else as much as fits
+    const long long want = ctx->cap_cfg > 0 ? std::min(batch_total, (long long)ctx->cap_cfg) : batch_total;
+    if (!columns_fit(ctx, want)) {
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        long long fitted = 0;
+        int rc = size_columns(ctx, want, multi, free_b, &fitted);
+        if (rc) return rc;
+    }
+    const long long cap = ctx->cap_cfg > 0 ? std::min(ctx->cap, (long long)ctx->cap_cfg) : ctx->cap;
+    P.offset_base = base;
+    bind_columns(ctx, P);
+    P.vol = fused_vol(ctx, a);
+    const bool split = batch_total > cap;
+    if (mode == 3) ctx->fit_gen = (!multi && !split) ? ctx->trace_gen : ~0ULL;  // (the next call with these tracks may skip this round trip)
+    std::vector<long long> h_off;
+    if (split) {  // (the cuts need the offsets of the batch and the unit ranges of its blocks)
+        if (h_unit_base.empty()) {
+            h_unit_base.resize((size_t)((ctx->n_shard + 31) / 32) + 1);
+            CK(cudaMemcpyAsync(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost, st));
+        }
+        h_off.resize((size_t)(e - b) + 1);
+        CK(cudaMemcpyAsync(h_off.data(), (long long *)ctx->b_offsets.p + b, sizeof(long long) * h_off.size(), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+    }
+    // The verification flag of a sub-batch is read before the sub-batch is handed on.  When the call is this one evaluation and
+    // nobody waits for it, the flag comes with the final read-back of the attempt instead (one host synchronisation less per call;
+    // a failed verification restarts the call, which clears the sums again).  A fill bracket the host does not wait for is read
+    // with the phase times, and spans the following sub-batches too: pipeline 1 reads no flag, so when its batch splits, its fill
+    // time also holds the exact-volume sorts and callbacks between its sub-batches (a bracket per sub-batch would need a host
+    // wait per sub-batch, which it does not have).
+    const bool verifies = mode != 1;
+    const bool read_flag = verifies && (multi || split || a.cb);
+    a.defer_verify = verifies && !read_flag;
+    for (long long sb = b; sb < e; sb = P.trk_end) {
+        long long nseg = batch_total;
+        if (split) {
+            int rc = cut_batch(ctx, P, h_off, b, h_unit_base, sb, cap, &nseg);
+            if (rc) return rc;
+        }
+        if (read_flag || sb == b) tic(ctx, 4);
+        if (nseg > 0) launch_eval(ctx, P, mode, nullptr);
+        if (verifies) launch_track_status(ctx, P, a.rtol, nullptr, d_bad(ctx));
+        a.launches += verifies ? 2 : 1;
+        CK(cudaGetLastError());
+        set_resident(ctx, P.trk_begin, P.trk_end, P.offset_base, nseg);
+        toc(ctx, 4);
+        if (read_flag) {
+            bool failed = false;
+            int rc = read_verify(ctx, &failed);
+            if (rc) return rc;
+            take_phase(ctx, 4, acc);
+            if (failed) {
+                a.next = Next::Sequential;
+                return RT_OK;
+            }
+        }
+        int rc = exact_batch(ctx, P, nseg, a);
+        if (rc) return rc;
+        rc = deliver_batch(ctx, a);
+        if (rc) return rc;
+    }
+    return RT_OK;
+}
+
+// The pipeline `mode` after the chunk plan.  Next::Hybrid: pipeline 3's record pool ran out (the mesh is far denser along some
+// chunks than the Cauchy-Crofton estimate); Next::Sequential: the verification failed.
+static int segmentize_pipeline(rt_ctx *ctx, WalkParams &P, uint32_t flags, int mode, Attempt &a) {
+    cudaStream_t st = ctx->stream;
+    const long long n = ctx->n_shard;
+    ctx->count_batches = 0;
+    if (n == 0) {  // (no k_seed clears the volume accumulator; no phase has work)
+        if (a.want_vol) CK(cudaMemsetAsync(ctx->vol_acc, 0, sizeof(double) * ((size_t)ctx->m.n_cells + 1), st));
+        ctx->total_segments = 0;
+        for (int ph = 2; ph <= 4; ++ph) {
+            ctx->phase_ms[ph] = 0.0;
+            ctx->pev_dirty[ph] = false;
+        }
+        return RT_OK;
+    }
+    const long long n_blocks = (n + 31) / 32, n_units = P.ch.n_units;
+    const bool count_only = (flags & RT_SEG_COUNT_ONLY) != 0;
+    const int *order_all = P.ch.order;
+    // (k_seed clears what a walk batch accumulates into: the pool cursor, the per-track sums and the volume accumulator)
+    CK(ensure(ctx->b_pool_cursor, sizeof(int)));
+    P.pool_cursor = (int *)ctx->b_pool_cursor.p;
+    if (mode != 1) {
+        CK(ensure(ctx->b_tsum, sizeof(double) * (size_t)n));
+        P.tsum = (double *)ctx->b_tsum.p;
+    }
+    long long max_slots = n_units * 32;  // chunk slots of one walk batch
+    if (mode == 3) {
+        int rc = plan_pool(ctx, P, a, &max_slots);
+        if (rc || a.next != Next::Done) return rc;
+    }
+    const bool multi = max_slots < n_units * 32;
     std::vector<long long> h_unit_base;
-    if (multi || ctx->cap_cfg > 0) {
+    if (multi) {
         h_unit_base.resize((size_t)n_blocks + 1);
         CK(cudaMemcpyAsync(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
     }
-    std::vector<long long> h_off;
     long long base = 0;  // segments of the batches already done
     long long B0 = 0;
-    ctx->count_batches = 0;
     // phase times are accumulated over the batches (every batch ends with a stream synchronisation anyway)
     double acc[6] = {0, 0, 0, 0, 0, 0};
-    auto take = [&](int ph) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, ctx->pev[ph][0], ctx->pev[ph][1]) == cudaSuccess) acc[ph] += (double)ms;
-        ctx->pev_dirty[ph] = false;
-    };
     while (B0 < n_blocks) {
         long long B1 = n_blocks;
         if (multi) {
@@ -1259,28 +1372,33 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         const long long u0 = multi ? h_unit_base[(size_t)B0] : 0, u1 = multi ? h_unit_base[(size_t)B1] : n_units;
         const long long slots = (u1 - u0) * 32;
         ctx->count_batches += 1;
-        // ---- seeds, count+record walk, per-track fix-up, offsets of the batch
+        // ---- seeds, count walk, per-track fix-up, offsets of the batch
         P.trk_begin = b;
         P.trk_end = e;
         P.unit_begin = u0;
         P.unit_end = u1;
         P.ch.order = multi ? nullptr : order_all;
         P.pool_slot_base = u0 * 32;
-        P.vol = nullptr;
+        P.vol = count_only && a.want_vol ? ctx->vol_acc : nullptr;  // (count-only: the count walk sums the volumes)
         P.offset_base = 0;
         P.cursor_init = (int)slots;
         P.zero_vol = (a.want_vol && B0 == 0) ? ctx->vol_acc : nullptr;  // (+1: the failed-rank flag of rt_volumes)
         P.zero_vol_n = (long long)P.m.n_cells + 1;
-        if (ctx->opt_debug_clear_pool) CK(cudaMemsetAsync(ctx->b_pool.p, 0, ctx->b_pool.bytes, st));
+        if (mode == 3 && ctx->opt_debug_clear_pool) CK(cudaMemsetAsync(ctx->b_pool.p, 0, ctx->b_pool.bytes, st));
         if (B0 > 0) tic(ctx, 2);  // (the first batch's count phase started with the chunk plan)
         k_seed<<<blocks_for(slots, 128), 128, 0, st>>>(P);
-        k_march<<<blocks_for(slots, kMarchThreads), kMarchThreads, 0, st>>>(P);
+        if (mode == 1 && ctx->mixed)
+            k_walk<false, true><<<blocks_for(slots, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        else if (mode == 1)
+            k_walk<false><<<blocks_for(slots, kWalkThreads), kWalkThreads, 0, st>>>(P);
+        else
+            k_march<<<blocks_for(slots, kMarchThreads), kMarchThreads, 0, st>>>(P);
         k_fixup_tracks<<<blocks_for(e - b, 128), 128, 0, st>>>(P);
         CK(cudaGetLastError());
         toc(ctx, 2);
         tic(ctx, 3);
         // (exact volumes size their sort from the segment total on the host: never optimistic)
-        const bool optimistic = !multi && !a.cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
+        const bool optimistic = mode == 3 && !multi && !a.cb && ctx->cap_cfg == 0 && ctx->opt_optimistic && !ctx->skip_optimistic_once &&
                                 ctx->fit_gen == ctx->trace_gen && columns_fit(ctx, 1) && !ctx->exact;
         ScanGuard guard{};
         if (optimistic) guard = ScanGuard{d_guard(ctx), base, ctx->cap, P.pool_cursor, P.pool_blocks};
@@ -1288,7 +1406,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
         toc(ctx, 3);
         a.launches += 6;
         CK(cudaMemcpyAsync(&ctx->h_pin[1], (long long *)ctx->b_offsets.p + e, sizeof(long long), cudaMemcpyDeviceToHost, st));
-        if (!optimistic) CK(cudaMemcpyAsync(&ctx->h_pin[9], P.pool_cursor, sizeof(int), cudaMemcpyDeviceToHost, st));
+        if (mode == 3 && !optimistic) CK(cudaMemcpyAsync(&ctx->h_pin[9], P.pool_cursor, sizeof(int), cudaMemcpyDeviceToHost, st));
         if (optimistic) {
             // ---- optimistic evaluation: no host round trip between the walk and the evaluation (see rt_ctx::opt_optimistic);
             // the guard (does the batch fit the Segment columns, did the pool hold every record?) is evaluated by the scan
@@ -1296,7 +1414,7 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
             bind_columns(ctx, P);
             P.vol = fused_vol(ctx, a);
             tic(ctx, 4);
-            launch_eval(d_guard(ctx));
+            launch_eval(ctx, P, mode, d_guard(ctx));
             launch_track_status(ctx, P, a.rtol, d_guard(ctx), d_bad(ctx));
             a.launches += 2;
             CK(cudaGetLastError());
@@ -1307,192 +1425,30 @@ static int segmentize_single(rt_ctx *ctx, WalkParams &P, Attempt &a) {
             return RT_OK;
         }
         CK(cudaStreamSynchronize(st));
-        take(2);
-        take(3);
+        take_phase(ctx, 2, acc);
+        take_phase(ctx, 3, acc);
         const long long batch_total = ctx->h_pin[1] - base;
-        if ((long long)*(int *)&ctx->h_pin[9] > (long long)P.pool_blocks) {  // some walker found the pool empty
+        if (mode == 3 && (long long)*(int *)&ctx->h_pin[9] > (long long)P.pool_blocks) {  // some walker found the pool empty
             a.next = Next::Hybrid;
             return RT_OK;
         }
         ctx->total_segments = base + batch_total;
-        // ---- Segment columns: everything of this batch if it fits, else as much as fits
-        const long long want = ctx->cap_cfg > 0 ? std::min(batch_total, (long long)ctx->cap_cfg) : batch_total;
-        if (!columns_fit(ctx, want)) {
-            CK(query_mem());
-            long long fitted = 0;
-            int rc = size_columns(ctx, want, multi, free_b, &fitted);
-            if (rc) return rc;
-            have_mem = false;
+        if (count_only) {  // (pipeline 1, one batch)
+            ctx->pev_dirty[4] = false;
+            break;
         }
-        const long long cap = ctx->cap_cfg > 0 ? std::min(ctx->cap, (long long)ctx->cap_cfg) : ctx->cap;
-        P.offset_base = base;
-        bind_columns(ctx, P);
-        P.vol = fused_vol(ctx, a);
-        const bool split = batch_total > cap;
-        ctx->fit_gen = (!multi && !split) ? ctx->trace_gen : ~0ULL;  // (the next call with these tracks may skip this round trip)
-        if (split) {
-            if (h_unit_base.empty()) {  // (one walk batch whose segments do not fit after all: the unit ranges are needed now)
-                h_unit_base.resize((size_t)n_blocks + 1);
-                CK(cudaMemcpyAsync(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost, st));
-            }
-            h_off.resize((size_t)(e - b) + 1);
-            CK(cudaMemcpyAsync(h_off.data(), (long long *)ctx->b_offsets.p + b, sizeof(long long) * h_off.size(), cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-        }
-        for (long long sb = b; sb < e; sb = P.trk_end) {
-            long long nseg = batch_total;
-            if (split) {
-                int rc = cut_batch(ctx, P, h_off, b, h_unit_base, sb, cap, &nseg);
-                if (rc) return rc;
-            }
-            tic(ctx, 4);
-            if (nseg > 0) launch_eval(nullptr);
-            launch_track_status(ctx, P, a.rtol, nullptr, d_bad(ctx));
-            a.launches += 2;
-            CK(cudaGetLastError());
-            set_resident(ctx, P.trk_begin, P.trk_end, P.offset_base, nseg);
-            toc(ctx, 4);
-            if (!a.cb && !multi && !split) {
-                // one batch, nobody waits for it: the verification flag is read with the final read-back of the attempt, which
-                // saves one host synchronisation per call; the fill time is collected lazily
-                a.defer_verify = true;
-                ctx->phase_ms[2] = acc[2];
-                ctx->phase_ms[3] = acc[3];
-                return exact_batch(ctx, P, nseg, a);  // (a failed verification restarts the call, which clears the sums again)
-            }
-            bool failed = false;
-            int rc = read_verify(ctx, &failed);
-            if (rc) return rc;
-            take(4);
-            if (failed) {
-                a.next = Next::Sequential;
-                return RT_OK;
-            }
-            rc = exact_batch(ctx, P, nseg, a);
-            if (rc) return rc;
-            rc = deliver_batch(ctx, a);
-            if (rc) return rc;
-        }
+        if (mode == 0 && ctx->opt_debug_verify_fail) CK(cudaMemsetAsync(d_verify(ctx), 1, 1, st));  // (test hook: the verification fails)
+        int rc = evaluate_batch(ctx, P, mode, a, base, batch_total, multi, h_unit_base, acc);
+        if (rc || a.next != Next::Done) return rc;
         base += batch_total;
         B0 = B1;
     }
-    for (int ph = 2; ph <= 4; ++ph) ctx->phase_ms[ph] = acc[ph];
+    for (int ph = 2; ph <= 4; ++ph)
+        if (!ctx->pev_dirty[ph]) ctx->phase_ms[ph] = acc[ph];  // (a bracket the host did not wait for is read with the phase times)
     return RT_OK;
 }
 
-// ---- two-pass pipelines: count -> scan -> fill (possibly in uid batches over a recycled buffer)
-//   mode 1 (sequential): k_walk<false> counts, k_walk<true> fills (walk.cuh);
-//   mode 0 (hybrid):     k_march counts by sign tests (march.cuh; no record pool, so it records nothing), k_walk<true> fills
-//                        and re-derives the same decisions from the exact geometry, k_track_status runs the length check
-//                        (src/track.jl:171-175) after the fill.  A fill that disagrees with the count fails the verification:
-//                        Next::Sequential.
-static int segmentize_two_pass(rt_ctx *ctx, WalkParams &P, uint32_t flags, bool hybrid, Attempt &a) {
-    cudaStream_t st = ctx->stream;
-    const long long n = ctx->n_shard;
-    const size_t nn = (size_t)std::max<long long>(n, 1);
-    // (+1: the failed-rank flag of rt_volumes)
-    if (a.want_vol) CK(cudaMemsetAsync(ctx->vol_acc, 0, sizeof(double) * ((size_t)ctx->m.n_cells + 1), st));
-    // ---- seeds, count pass, per-track fix-up
-    if (n > 0) {
-        const long long n_units = P.ch.n_units;
-        k_seed<<<blocks_for(n_units * 32, 128), 128, 0, st>>>(P);
-        if (hybrid) {
-            k_march<<<blocks_for(n_units * 32, kMarchThreads), kMarchThreads, 0, st>>>(P);
-        } else {
-            P.vol = (a.want_vol && (flags & RT_SEG_COUNT_ONLY)) ? ctx->vol_acc : nullptr;
-            if (ctx->mixed)
-                k_walk<false, true><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-            else
-                k_walk<false><<<blocks_for(n_units * 32, kWalkThreads), kWalkThreads, 0, st>>>(P);
-        }
-        k_fixup_tracks<<<blocks_for(n, 128), 128, 0, st>>>(P);
-        a.launches += 3;
-        a.first_bad_scan = true;
-    }
-    CK(cudaGetLastError());
-    toc(ctx, 2);
-    // ---- scan
-    tic(ctx, 3);
-    long long total = 0;
-    if (n > 0) {
-        CK((exclusive_scan<int, long long>(ctx, (const int *)ctx->b_count.p, (long long *)ctx->b_offsets.p, n)));
-        a.launches += 3;
-        CK(cudaMemcpyAsync(&ctx->h_pin[1], (long long *)ctx->b_offsets.p + n, sizeof(long long), cudaMemcpyDeviceToHost, st));
-    }
-    toc(ctx, 3);
-    CK(cudaStreamSynchronize(st));
-    if (n > 0) total = ctx->h_pin[1];
-    ctx->total_segments = total;
-    ctx->phase_ms[4] = 0.0;
-    ctx->pev_dirty[4] = false;
-    if ((flags & RT_SEG_COUNT_ONLY) || n == 0) return RT_OK;
-
-    // ---- fill pass
-    size_t free_b = 0, total_b = 0;
-    CK(cudaMemGetInfo(&free_b, &total_b));
-    long long cap = 0;
-    int rc = size_columns(ctx, ctx->cap_cfg > 0 ? std::min(total, (long long)ctx->cap_cfg) : total, false, free_b, &cap);
-    if (rc) return rc;
-    if (hybrid) {
-        CK(ensure(ctx->b_tsum, sizeof(double) * nn));
-        CK(cudaMemsetAsync(ctx->b_tsum.p, 0, sizeof(double) * nn, st));
-    }
-    bind_columns(ctx, P);
-    P.tsum = hybrid ? (double *)ctx->b_tsum.p : nullptr;
-    P.vol = fused_vol(ctx, a);
-    P.counters = nullptr;
-    if (ctx->opt_debug_verify_fail && hybrid) CK(cudaMemsetAsync(d_verify(ctx), 1, 1, st));
-    const bool split = total > cap;
-    std::vector<long long> h_off, h_unit_base;
-    if (split) {
-        h_off.resize((size_t)n + 1);
-        CK(cudaMemcpy(h_off.data(), ctx->b_offsets.p, sizeof(long long) * ((size_t)n + 1), cudaMemcpyDeviceToHost));
-        h_unit_base.resize((size_t)((n + 31) / 32) + 1);
-        CK(cudaMemcpy(h_unit_base.data(), ctx->b_unit_base.p, sizeof(long long) * h_unit_base.size(), cudaMemcpyDeviceToHost));
-    }
-    tic(ctx, 4);
-    for (long long b = 0; b < n; b = P.trk_end) {
-        long long nseg = total;
-        if (split) {
-            rc = cut_batch(ctx, P, h_off, 0, h_unit_base, b, cap, &nseg);
-            if (rc) return rc;
-        }
-        const unsigned blocks = blocks_for((P.unit_end - P.unit_begin) * 32, kWalkThreads);
-        if (ctx->mixed && ctx->lengths_only)
-            k_walk<true, true, false><<<blocks, kWalkThreads, 0, st>>>(P);
-        else if (ctx->mixed)
-            k_walk<true, true><<<blocks, kWalkThreads, 0, st>>>(P);
-        else if (ctx->lengths_only)
-            k_walk<true, false, false><<<blocks, kWalkThreads, 0, st>>>(P);
-        else
-            k_walk<true><<<blocks, kWalkThreads, 0, st>>>(P);
-        a.launches += 1;
-        if (hybrid) {
-            launch_track_status(ctx, P, a.rtol, nullptr, nullptr);
-            a.launches += 1;
-        }
-        CK(cudaGetLastError());
-        set_resident(ctx, P.trk_begin, P.trk_end, P.offset_base, nseg);
-        if (hybrid) {
-            bool failed = false;
-            rc = read_verify(ctx, &failed);
-            if (rc) return rc;
-            if (failed) {
-                a.next = Next::Sequential;
-                toc(ctx, 4);
-                return RT_OK;
-            }
-        }
-        rc = exact_batch(ctx, P, nseg, a);
-        if (rc) return rc;
-        rc = deliver_batch(ctx, a);
-        if (rc) return rc;
-    }
-    toc(ctx, 4);
-    return RT_OK;
-}
-
-// One attempt of rt_segmentize in pipeline `mode` (segmentize_single or segmentize_two_pass); a.next says whether it stands.
+// One attempt of rt_segmentize in pipeline `mode`; a.next says whether it stands.
 static int segmentize_attempt(rt_ctx *ctx, double tiny_step, int32_t k, int32_t max_iter, uint32_t flags, int mode, Attempt &a,
                               unsigned long long *bad_out) {
     cudaStream_t st = ctx->stream;
@@ -1537,7 +1493,7 @@ static int segmentize_attempt(rt_ctx *ctx, double tiny_step, int32_t k, int32_t 
         int rc = plan_chunks(ctx, P, flags, &a.launches);
         if (rc) return rc;
     }
-    int rc = mode == 3 && n > 0 ? segmentize_single(ctx, P, a) : segmentize_two_pass(ctx, P, flags, mode == 0, a);
+    int rc = segmentize_pipeline(ctx, P, flags, mode, a);
     if (rc || a.next != Next::Done) return rc;
 
     ctx->voln_done = false;
@@ -1552,7 +1508,7 @@ static int segmentize_attempt(rt_ctx *ctx, double tiny_step, int32_t k, int32_t 
         ctx->voln_done = true;
         a.launches += 1;
     }
-    if (a.first_bad_scan) {
+    if (mode == 1 && n > 0) {  // (pipeline 1 checked the lengths in k_fixup_tracks, which does not report the first failing track)
         k_first_bad<<<blocks_for(n, 256), 256, 0, st>>>((const int *)ctx->b_status.p, n, d_bad(ctx));
         a.launches += 1;
     }
@@ -1706,12 +1662,13 @@ extern "C" int rt_segments_download(rt_ctx *ctx, double *px, double *py, double 
     size_t n = (size_t)ctx->res_nseg;
     if (n == 0) return RT_OK;
     cudaStream_t st = ctx->stream;
-    if (px) CK(cudaMemcpyAsync(px, ctx->s_px, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (py) CK(cudaMemcpyAsync(py, ctx->s_py, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (qx) CK(cudaMemcpyAsync(qx, ctx->s_qx, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (qy) CK(cudaMemcpyAsync(qy, ctx->s_qy, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (len) CK(cudaMemcpyAsync(len, ctx->s_len, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    if (element) CK(cudaMemcpyAsync(element, ctx->s_elem, sizeof(int) * n, cudaMemcpyDeviceToHost, st));
+    const SegColumns c = seg_columns(ctx);
+    if (px) CK(cudaMemcpyAsync(px, c.px, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (py) CK(cudaMemcpyAsync(py, c.py, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (qx) CK(cudaMemcpyAsync(qx, c.qx, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (qy) CK(cudaMemcpyAsync(qy, c.qy, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (len) CK(cudaMemcpyAsync(len, c.len, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    if (element) CK(cudaMemcpyAsync(element, c.elem, sizeof(int) * n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return RT_OK;
 }
@@ -1729,6 +1686,7 @@ extern "C" int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy,
     *n_exceptions = 0;
     if (n == 0) return RT_OK;
     cudaStream_t st = ctx->stream;
+    const SegColumns c = seg_columns(ctx);
     // the exception list is built on a side stream (a 0.3 ms kernel over the resident columns) while the four columns that do
     // cross the bus are already on their way
     if (!ctx->aux_stream) {
@@ -1744,13 +1702,13 @@ extern "C" int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy,
     CK(cudaEventRecord(ctx->ev_aux, st));  // (the evaluation that wrote the columns)
     CK(cudaStreamWaitEvent(ax, ctx->ev_aux, 0));
     CK(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), ax));
-    k_p_exceptions<<<blocks_for(n, 256), 256, 0, ax>>>(n, ctx->s_px, ctx->s_py, ctx->s_qx, ctx->s_qy, (long long)cap, d_cnt, d_idx, d_px, d_py);
+    k_p_exceptions<<<blocks_for(n, 256), 256, 0, ax>>>(n, c.px, c.py, c.qx, c.qy, (long long)cap, d_cnt, d_idx, d_px, d_py);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(&ctx->h_pin[11], d_cnt, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ax));
-    if (qx) CK(cudaMemcpyAsync(qx, ctx->s_qx, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    if (qy) CK(cudaMemcpyAsync(qy, ctx->s_qy, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    if (len) CK(cudaMemcpyAsync(len, ctx->s_len, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
-    if (element) CK(cudaMemcpyAsync(element, ctx->s_elem, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (qx) CK(cudaMemcpyAsync(qx, c.qx, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (qy) CK(cudaMemcpyAsync(qy, c.qy, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (len) CK(cudaMemcpyAsync(len, c.len, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (element) CK(cudaMemcpyAsync(element, c.elem, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(ax));
     const long long k = ctx->h_pin[11];
     *n_exceptions = k;
@@ -1773,13 +1731,13 @@ extern "C" int rt_segments_device(rt_ctx *ctx, rt_batch *view) {
     view->n_segments = ctx->res_nseg;
     view->d_offsets = (const int64_t *)ctx->b_offsets.p;
     view->offset_base = ctx->res_off_base;
-    const bool points = !ctx->lengths_only;
-    view->d_px = points ? ctx->s_px : nullptr;
-    view->d_py = points ? ctx->s_py : nullptr;
-    view->d_qx = points ? ctx->s_qx : nullptr;
-    view->d_qy = points ? ctx->s_qy : nullptr;
-    view->d_len = ctx->s_len;
-    view->d_element = ctx->s_elem;
+    const SegColumns c = seg_columns(ctx);
+    view->d_px = c.px;
+    view->d_py = c.py;
+    view->d_qx = c.qx;
+    view->d_qy = c.qy;
+    view->d_len = c.len;
+    view->d_element = c.elem;
     view->stream = (void *)ctx->stream;
     view->attempt = 0;
     return RT_OK;
@@ -1846,9 +1804,11 @@ extern "C" int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *s
     CK(ensure(ctx->b_tau, sizeof(double) * n_tau));
     CK(cudaMemcpyAsync(ctx->b_sigma.p, sigma_t, sizeof(double) * n_sig, cudaMemcpyHostToDevice, st));
     CK(cudaEventRecord(ctx->ev2[0], st));
-    if (n_seg > 0)
-        k_tau<<<blocks_for(n_seg * n_groups, 256), 256, 0, st>>>(n_seg, n_groups, ctx->s_len, ctx->s_elem, (const double *)ctx->b_sigma.p,
-                                                               layout, (double *)ctx->b_tau.p);
+    if (n_seg > 0) {
+        const SegColumns c = seg_columns(ctx);
+        k_tau<<<blocks_for(n_seg * n_groups, 256), 256, 0, st>>>(n_seg, n_groups, c.len, c.elem, (const double *)ctx->b_sigma.p, layout,
+                                                               (double *)ctx->b_tau.p);
+    }
     CK(cudaEventRecord(ctx->ev2[1], st));
     CK(cudaGetLastError());
     if (tau_host && n_seg > 0)
@@ -1901,8 +1861,10 @@ extern "C" int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d
     if (ctx->voln_ready >= 0) CK(cudaStreamWaitEvent(st, ctx->ev_vol_free[ctx->voln_ready], 0));  // the all-reduced volumes
     CK(ensure(ctx->b_factor, sizeof(double) * (size_t)nc));
     k_volume_factors<<<blocks_for(nc, 256), 256, 0, st>>>(nc, (const double *)ctx->b_area.p, (const double *)ctx->b_voln.p, (double *)ctx->b_factor.p);
-    if (ctx->res_nseg > 0)
-        k_scale_lengths<<<blocks_for(ctx->res_nseg, 256), 256, 0, st>>>(ctx->res_nseg, ctx->s_elem, (const double *)ctx->b_factor.p, ctx->s_len);
+    if (ctx->res_nseg > 0) {
+        const SegColumns c = seg_columns(ctx);
+        k_scale_lengths<<<blocks_for(ctx->res_nseg, 256), 256, 0, st>>>(ctx->res_nseg, c.elem, (const double *)ctx->b_factor.p, c.len);
+    }
     CK(cudaGetLastError());
     if (factors) CK(cudaMemcpyAsync(factors, ctx->b_factor.p, sizeof(double) * (size_t)nc, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -266,7 +266,7 @@ __device__ __forceinline__ double bbox_dist(const DevMesh &m, double x, double y
 __global__ void __launch_bounds__(128) k_seed(const __grid_constant__ WalkParams P) {
     long long gw = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
     int lane = threadIdx.x & 31;
-    if (P.pool_cursor) {  // single-walk pipeline: clear what the walk and the evaluation of this batch accumulate into
+    if (P.pool_cursor) {  // clear what the walk and the evaluation of this batch accumulate into
         const long long gtid = blockIdx.x * (long long)blockDim.x + threadIdx.x, gsz = gridDim.x * (long long)blockDim.x;
         if (gtid == 0) *P.pool_cursor = P.cursor_init;
         if (P.tsum)

@@ -390,3 +390,4 @@ def test_empty_shard_with_a_communicator(cases, make_tg):
     rt.segmentize_(tg)
     assert tg.n_segments == 0 and tg.info("collectives") == 1
     assert np.array_equal(tg.volumes.view(np.uint64), np.zeros(case.mesh.num_cells, np.uint64))
+    assert all(tg.segments[k].shape == (0,) for k in KEYS) and tg.info("count_batches") == 0

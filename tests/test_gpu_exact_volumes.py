@@ -208,13 +208,17 @@ def test_one_rank_communicator(cases, make_tg, pipeline):
 
 
 # ---- failing tracks -----------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("pipeline", [3, 1])
+@pytest.mark.parametrize("pipeline", [3, 0, 1])
 def test_failing_tracks_contribute(cases, make_tg, pipeline):
+    """in one batch and in several: the failing tracks' segments are summed, and the first failing track is the oracle's"""
     case = cases("far")
     assert np.count_nonzero(case.otg.seg_status == 2) > 0
     tg = make_tg(case, pipeline)
-    assert_bits(exact(tg), case.ref)
-    assert np.array_equal(tg.segment_status, case.otg.seg_status)
+    for capacity in (0, case.otg.n_segments // 4 + 1):
+        set_capacity(tg, capacity)
+        assert_bits(exact(tg), case.ref)
+        assert np.array_equal(tg.segment_status, case.otg.seg_status)
+        assert (tg.first_bad_uid, tg.bad_status) == (case.otg.first_bad_uid, case.otg.bad_status)
 
 
 # ---- only the volumes change ----------------------------------------------------------------------------------------------------

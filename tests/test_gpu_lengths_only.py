@@ -260,19 +260,35 @@ def test_end_points_are_refused(cases, make_tg):
     assert_columns(tg.fetch_segments(pinned=True), case.otg)
 
 
+def assert_no_segments(tg):
+    """a count-only call leaves no resident segment: both downloads give empty columns"""
+    assert tg.resident_batch()[3] == 0
+    s = tg.fetch_segments()
+    assert all(s[k].shape == (0,) for k in ("px", "py", "qx", "qy", "len", "element"))
+    s = tg.fetch_segments(compact=True)
+    assert tg.n_exceptions == 0 and all(s[k].shape == (0,) for k in ("qx", "qy", "len", "element"))
+
+
 @pytest.mark.parametrize("pipeline", [3, 1])
 def test_count_only_ignores_the_flag(cases, make_tg, pipeline):
+    """also as the first call of a context (no Segment columns allocated yet) and after a lengths-only call (columns without p
+    and q): no segments, and nothing to refuse"""
     case = cases("jittered")
     tg = make_tg(case, pipeline)
     for flags in (COUNT | NO_VOL, COUNT):
         rt.segmentize_(tg, flags=flags, check=False)
+        assert_no_segments(tg)
         ref = (tg.n_segments, tg.segment_offsets.copy(), tg.segment_status.copy(), tg.volumes.copy())
         rt.segmentize_(tg, flags=flags | LEN_ONLY, check=False)
+        assert_no_segments(tg)
         assert tg.n_segments == ref[0] == case.otg.n_segments
         assert np.array_equal(tg.segment_offsets, ref[1]) and np.array_equal(tg.segment_status, ref[2])
         if not flags & NO_VOL:
             assert np.allclose(tg.volumes, ref[3], rtol=1e-12, atol=0.0)
             assert_volumes_close(case.ref, tg.volumes)
+    rt.segmentize_(tg, lengths_only=True, check=False)
+    rt.segmentize_(tg, flags=COUNT, check=False)
+    assert_no_segments(tg)
 
 
 # ---- size -----------------------------------------------------------------------------------------------------------------------
