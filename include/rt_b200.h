@@ -216,6 +216,30 @@ int rt_quadrature_device(rt_ctx *ctx, rt_quad_view *view, double *omega_host);
 int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
                        double *tau_host);
 
+/* ---- material regions: a transport code gives cross sections per material, not per cell -------------------------------------
+ * rt_set_regions: cell_region has n_cells values, 1-based, in [1, n_regions] (HOST): the region (material) of every cell, e.g. from
+ * the Gridap face labeling or the physical groups of a .msh file.  The map is checked on the device: a value outside [1, n_regions]
+ * returns RT_ERR_ARG (the message names the first such cell and its value) and leaves the previous map in place; n_regions < 1 is
+ * RT_ERR_ARG.  The call also orders the cells by region once (stable: ascending cell id inside a region).  NULL clears the map; a
+ * new rt_mesh_upload clears it too.
+ * rt_optical_lengths_by_region: rt_optical_lengths with sigma_t given per REGION: n_regions x n_groups (HOST, region-major),
+ * tau[s][g] = sigma_t[region(element(s))][g] * len(s).  The table crosses the bus at its own size (not n_cells x n_groups) and is
+ * read through the cache on the device.  tau is bit-equal to rt_optical_lengths with the per-cell table expanded from the
+ * per-region one.  Same layouts, buffer ownership, in-callback behaviour and rt_info "tau_ms" as rt_optical_lengths; RT_ERR_ARG
+ * without a region map for the current mesh.
+ * rt_region_volumes: per-region sums, n_regions values each; either pointer may be NULL.
+ *   traced[r]: the normalised volumes that rt_volumes returns (all-reduced or chained with a communicator): needs a completed
+ *              rt_segmentize with volumes followed by rt_volumes, and waits for the collective rt_volumes may only have enqueued;
+ *   exact[r]:  the element areas of rt_element_volumes (triangle meshes only, as rt_element_volumes).
+ * Cells are summed in ascending cell id with one plain `+` each, starting from 0.0: with RT_SEG_EXACT_VOLUMES the traced region
+ * volumes are reproducible bit for bit, like the volumes they are summed from.  RT_ERR_ARG inside a batch callback of rt_segmentize
+ * and without a region map.
+ * All three run on the context's stream and leave the resident batch, offsets, volumes, rt_stats and rt_phase_ms as they are. */
+int rt_set_regions(rt_ctx *ctx, int32_t n_regions, const int32_t *cell_region);
+int rt_optical_lengths_by_region(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
+                                 double *tau_host);
+int rt_region_volumes(rt_ctx *ctx, double *traced, double *exact);
+
 /* ---- exact element volumes and the volume correction (SURVEY 8f-2) -------------------------------------
  * rt_element_volumes: element_volume(mesh, node_ids) = 1/2*abs((x2-x1) x (x3-x1)) for every cell (src/trackgenerator.jl:402-411),
  * computed on the device; `areas` (n_cells, may be NULL) receives a copy, *d_areas (may be NULL) the device buffer.
@@ -276,7 +300,7 @@ int rt_stats(rt_ctx *ctx, double stats[8]);
  * pipelines 0 and 1, which walk the shard in one batch); "optimistic_cancels" (calls of this context whose evaluation, launched behind the walk without reading the segment total back, was cancelled by the device-side guard and
  * repeated); "collectives" (ncclAllReduce calls this context has issued in rt_volumes, including the joins of a rank whose
  * rt_segmentize failed: the ranks of a communicator that call rt_volumes as documented below agree on it); "rho", "band_cost"
- * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths; "locate_knn" (points that entered the k-nearest-node
+ * (shard planning); "tau_ms" (k_tau alone) of the last rt_optical_lengths or rt_optical_lengths_by_region; "locate_knn" (points that entered the k-nearest-node
  * branch of find_element) and "locate_ms" (k_find_elements alone) of the last rt_find_elements; "exact_vol_ms" (contributions,
  * sort and fold of RT_SEG_EXACT_VOLUMES, summed over the batches of the last rt_segmentize; the chain's fold of rt_volumes is not
  * included) */

@@ -40,6 +40,7 @@ function _b200_context(t::TrackGenerator)
     _B200_CTX[t.tracks_by_uid] = ctx
     finalizer(t.tracks_by_uid) do v
         c = pop!(_B200_CTX, v, C_NULL)
+        pop!(_B200_NREG, v, 0)
         c == C_NULL || ccall((:rt_destroy, LIBRT_B200), Cvoid, (Ptr{Cvoid},), c)
     end
     return ctx
@@ -344,3 +345,65 @@ end
 `find_element(t.mesh, x, k)` (src/mesh.jl:103-146) for one point, with the reference's return value.
 """
 b200_find_element(t::TrackGenerator, x; k::Integer=2) = b200_find_elements(t, [x]; k=k)[1]
+
+# ---- material regions (include/rt_b200.h: rt_set_regions, rt_optical_lengths_by_region, rt_region_volumes) ---------------------
+
+# regions of the map set on each context (keyed like _B200_CTX)
+const _B200_NREG = IdDict{Any,Int}()
+
+"""
+    b200_set_regions!(t::TrackGenerator, names::AbstractVector{<:AbstractString}) -> Vector{Int32}
+
+The region of every cell from the model's face labeling: the position in `names` of the first name whose
+`get_face_mask(get_face_labeling(model), name, 2)` holds the cell.  A cell in none of them is an error.  The map is checked and
+ordered by region on the device (rt_set_regions); it is what `b200_optical_lengths_by_region` and `b200_region_volumes` read.
+"""
+function b200_set_regions!(t::TrackGenerator, names::AbstractVector{<:AbstractString})
+    ctx = _b200_context(t)
+    labeling = get_face_labeling(t.mesh.model)
+    region = zeros(Int32, num_cells(t.mesh.model))
+    for (r, name) in enumerate(names)
+        mask = get_face_mask(labeling, name, 2)
+        for c in eachindex(region)
+            region[c] == 0 && mask[c] && (region[c] = Int32(r))
+        end
+    end
+    first_free = findfirst(==(0), region)
+    first_free === nothing || error("$(count(==(0), region)) cells are in none of the labels $(names); the first is cell $(first_free)")
+    _b200_check(ctx, ccall((:rt_set_regions, LIBRT_B200), Cint, (Ptr{Cvoid}, Int32, Ptr{Int32}), ctx, Int32(length(names)), region))
+    _B200_NREG[t.tracks_by_uid] = length(names)
+    return region
+end
+
+"""
+    b200_optical_lengths_by_region(t::TrackGenerator, Σr::Matrix{Float64}) -> Matrix{Float64}
+
+`τ[g, s] = Σr[g, region(element(s))] * ℓ(s)` for every resident segment, with `Σr` of size n_groups × n_regions (one column per
+name given to `b200_set_regions!`): the cross sections of the transport code's materials, which cross the bus at their own size.
+Bit-equal to `b200_optical_lengths!` with the table expanded cell by cell.  The device buffer stays resident for an on-GPU sweep.
+"""
+function b200_optical_lengths_by_region(t::TrackGenerator, Σr::Matrix{Float64})
+    ctx = _b200_context(t)
+    size(Σr, 2) == get(_B200_NREG, t.tracks_by_uid, 0) || error("Σr must have one column per region of b200_set_regions!")
+    G = size(Σr, 1)
+    S = sum(length(track.segments) for track in t.tracks_by_uid)
+    τ = Matrix{Float64}(undef, G, S)
+    dτ = Ref{Ptr{Float64}}(C_NULL)
+    _b200_check(ctx, ccall((:rt_optical_lengths_by_region, LIBRT_B200), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Float64}, Int32, Ptr{Ptr{Float64}}, Ptr{Float64}), ctx, Int32(G), Σr, Int32(0), dτ, τ))
+    return τ
+end
+
+"""
+    b200_region_volumes(t::TrackGenerator) -> (traced, exact)
+
+Per-region sums of `t.volumes` (after `b200_segmentize!`) and of the exact cell areas (`element_volume`, triangle meshes), summed on
+the device over the cells of each region in ascending id.  Comparing the two is how `δ` and `n_azim` are chosen.
+"""
+function b200_region_volumes(t::TrackGenerator)
+    ctx = _b200_context(t)
+    n = get(_B200_NREG, t.tracks_by_uid, 0)
+    traced = zeros(n); exact = zeros(n)
+    _b200_check(ctx, ccall((:rt_region_volumes, LIBRT_B200), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}), ctx, traced, exact))
+    return traced, exact
+end

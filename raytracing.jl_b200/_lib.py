@@ -95,6 +95,9 @@ SYMBOLS = {
     "rt_tracks_device": (C.c_int, [_vp, C.POINTER(rt_track_view)]),
     "rt_quadrature_device": (C.c_int, [_vp, C.POINTER(rt_quad_view), _vp]),
     "rt_optical_lengths": (C.c_int, [_vp, C.c_int32, _f64, C.c_int32, C.POINTER(_vp), _vp]),
+    "rt_set_regions": (C.c_int, [_vp, C.c_int32, _vp]),
+    "rt_optical_lengths_by_region": (C.c_int, [_vp, C.c_int32, _f64, C.c_int32, C.POINTER(_vp), _vp]),
+    "rt_region_volumes": (C.c_int, [_vp, _vp, _vp]),
     "rt_element_volumes": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
     "rt_correct_volumes": (C.c_int, [_vp, _vp, C.POINTER(_vp)]),
     "rt_find_elements": (C.c_int, [_vp, C.c_int64, _f64, C.c_int32, _vp, C.POINTER(_vp)]),

@@ -428,6 +428,7 @@ class TrackGenerator(TrackLayout):
             mesh.bb_min, mesh.bb_max = lo, hi
         self._traced = self._segmented = False
         self._track_data = self._segments = self._offsets = self._resident = None
+        self._n_regions = 0  # (rt_mesh_upload clears the region map)
 
     def device_node_cells(self):
         """The vertex->cells table as the device holds it (1-based CSR like Gridap's Table)."""
@@ -604,6 +605,55 @@ class TrackGenerator(TrackLayout):
         _lib.check(self._ctx, _lib.lib().rt_optical_lengths(self._ctx, G, sig.reshape(-1), int(layout), C.byref(d), _lib.ptr(host)))
         return host, DeviceColumn(d.value, n * G, "<f8")
 
+    # ---- material regions (a transport code's cross sections are per material) ----------------------------------------------
+    def set_regions(self, cell_region, n_regions: int | None = None):
+        """The region (material) of every cell, 1-based (``UnstructuredDiscreteModel.cell_regions``), checked and ordered on the
+        device (rt_set_regions).  ``n_regions`` defaults to the largest value.  A value outside [1, n_regions] raises and keeps the
+        previous map; ``None`` clears the map.  ``upload_mesh`` clears it too."""
+        L = _lib.lib()
+        if cell_region is None:
+            _lib.check(self._ctx, L.rt_set_regions(self._ctx, 0, None))
+            self._n_regions = 0
+            return
+        reg = np.ascontiguousarray(cell_region, dtype=np.int32).reshape(-1)
+        if reg.shape[0] != self.mesh.num_cells:
+            raise ValueError(f"cell_region has {reg.shape[0]} values for {self.mesh.num_cells} cells")
+        n = int(reg.max()) if n_regions is None else int(n_regions)
+        _lib.check(self._ctx, L.rt_set_regions(self._ctx, n, _lib.ptr(reg)))
+        self._n_regions = n
+
+    @property
+    def n_regions(self) -> int:
+        """regions of the map set with ``set_regions`` (0: none)"""
+        return getattr(self, "_n_regions", 0)
+
+    def optical_lengths_by_region(self, sigma_t, layout: int = 0, fetch: bool = True):
+        """``optical_lengths`` with the cross sections per region: tau[s][g] = sigma_t[region(element(s))][g] * len(s), ``sigma_t``
+        of shape (n_regions, n_groups).  Bit-equal to ``optical_lengths`` with the table expanded cell by cell, and the same return
+        value: (numpy copy or None, DeviceColumn).  Needs ``set_regions``; inside ``on_batch`` of segmentize_ it acts on the batch
+        the callback received."""
+        sig = np.ascontiguousarray(sigma_t, dtype=np.float64)
+        if sig.ndim != 2 or sig.shape[0] != self.n_regions:
+            raise ValueError(f"sigma_t must have shape (n_regions = {self.n_regions}, n_groups)")
+        G = sig.shape[1]
+        view = _lib.rt_batch()
+        _lib.check(self._ctx, _lib.lib().rt_segments_device(self._ctx, C.byref(view)))
+        n = int(view.n_segments)
+        host = np.zeros((n, G) if layout == 0 else (G, n)) if fetch else None
+        d = C.c_void_p()
+        _lib.check(self._ctx, _lib.lib().rt_optical_lengths_by_region(self._ctx, G, sig.reshape(-1), int(layout), C.byref(d),
+                                                                        _lib.ptr(host)))
+        return host, DeviceColumn(d.value, n * G, "<f8")
+
+    def region_volumes(self, traced: bool = True, exact: bool = True):
+        """(traced, exact): per-region sums of ``tg.volumes`` (the traced volumes of the last segmentize_, all-reduced or chained
+        with a communicator) and of ``element_volumes()`` (triangle meshes only), summed on the device over the cells of each
+        region in ascending id (rt_region_volumes) -- what δ and n_azim are chosen by.  Either may be skipped (None)."""
+        t = np.zeros(self.n_regions) if traced else None
+        e = np.zeros(self.n_regions) if exact else None
+        _lib.check(self._ctx, _lib.lib().rt_region_volumes(self._ctx, _lib.ptr(t), _lib.ptr(e)))
+        return t, e
+
     def find_elements(self, xy, k: int = 2, fetch: bool = True):
         """find_element(mesh, x, k) (src/mesh.jl:103-146) for every row of ``xy`` (n, 2) in one device call (rt_find_elements): the
         1-based cell of each point, -1 where no cell passes.  Returns (int32 ids or None, DeviceColumn); the device buffer is reused
@@ -768,8 +818,8 @@ def segmentize_(tg: TrackGenerator, k: int = 5, rtol: float = RTOL_DEFAULT, flag
                 lengths_only: bool = False) -> TrackGenerator:
     """segmentize!(tg; k, rtol): count pass -> scan -> fill pass (+ fused fill_volumes) on the device.
     ``on_batch(SegmentBatch)`` is called after every uid batch of the fill pass (one batch when everything fits).  Inside it
-    ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()`` and ``tg.correct_volumes()`` act
-    on that batch.  An exception raised by ``on_batch`` stops the call and is re-raised here -- on a TrackGenerator with a
+    ``tg.resident_batch()``, ``tg.fetch_segments()`` / ``tg.segments``, ``tg.optical_lengths()``, ``tg.optical_lengths_by_region()``
+    and ``tg.correct_volumes()`` act on that batch.  An exception raised by ``on_batch`` stops the call and is re-raised here -- on a TrackGenerator with a
     communicator only after this rank has joined the call's all-reduce of the volumes (as after any other failure), so that its
     peers are not left waiting inside it.
 

@@ -94,6 +94,10 @@ struct rt_ctx {
     DevBuf b_nch, b_blk_chunks, b_unit_base, b_unit_block, b_ch_i, b_ch_d;  // chunk plan (walk.cuh ChunkPlan)
     DevBuf b_order, b_okeys, b_ohist;  // spatial execution order of the units
     DevBuf b_omega, b_sigma, b_tau;  // sweep-facing exports (sweep.cuh)
+    // region map (rt_set_regions): the 1-based region of every cell, the cell ids sorted stably by region and the run of every
+    // region in that order (start | end); n_regions = 0: no map.  rt_mesh_upload clears it.
+    int n_regions = 0;
+    DevBuf b_region, b_reg_order, b_reg_runs, b_reg_val;
     DevBuf b_area, b_factor;         // exact element volumes, volume-correction factors (sweep.cuh)
     DevBuf b_exc;                    // compact download: exception list (sweep.cuh k_p_exceptions)
     cudaStream_t aux_stream = nullptr;  // ... built on a side stream while the columns cross the bus
@@ -167,6 +171,7 @@ struct rt_ctx {
     bool lengths_only = false; // the last rt_segmentize (and its resident batch) wrote only len and element (RT_SEG_LENGTHS_ONLY)
     long long res_trk_begin = 0, res_trk_end = 0, res_off_base = 0, res_nseg = 0;  // resident batch (shard-local)
     bool vol_valid = false;
+    bool vol_fetched = false;  // rt_volumes ran after the last rt_segmentize (what rt_region_volumes sums)
     // Inside the batch callback of rt_segmentize the resident batch is valid although the call has not finished (`segmented` is
     // false until it returns); the volume correction then uses the normalised volumes of the PREVIOUS call, which the current one
     // overwrites only after its last callback (k_normalise, rt_volumes).
@@ -311,7 +316,8 @@ extern "C" void rt_destroy(rt_ctx *ctx) {
                      &ctx->b_pool,    &ctx->b_pool_next, &ctx->b_pool_cursor,
                      &ctx->b_area,    &ctx->b_factor,    &ctx->b_layout,    &ctx->b_vol_alt,  &ctx->b_exc,
                      &ctx->b_loc_xy,  &ctx->b_loc_elem,  &ctx->b_loc_knn,
-                     &ctx->b_ex_key,  &ctx->b_ex_val,    &ctx->b_ex_runs,   &ctx->b_ex_tmp,   &ctx->b_chain};
+                     &ctx->b_ex_key,  &ctx->b_ex_val,    &ctx->b_ex_runs,   &ctx->b_ex_tmp,   &ctx->b_chain,
+                     &ctx->b_region,  &ctx->b_reg_order, &ctx->b_reg_runs,  &ctx->b_reg_val};
     for (DevBuf *b : all) release(*b);
     for (int ph = 0; ph < 6; ++ph)
         for (int q = 0; q < 2; ++q)
@@ -361,6 +367,7 @@ extern "C" int rt_mesh_upload(rt_ctx *ctx, int32_t n_nodes, const double *xy, in
     if (!ctx) return RT_ERR_ARG;
     if (n_nodes < 3 || n_cells < 1 || !xy || !cell_ptrs || !cell_data || (!node_cell_ptrs != !node_cell_data) || (!bb_min != !bb_max))
         return fail(ctx, RT_ERR_ARG, "rt_mesh_upload: null or empty mesh arrays");
+    ctx->n_regions = 0;  // (a region map describes the cells of the mesh it was set for)
     const bool dev_nc = node_cell_ptrs == nullptr;  // build the vertex -> cells table on the device
     const bool dev_bb = bb_min == nullptr;          // reduce the bounding box on the device
     bool mixed = false;
@@ -1552,6 +1559,7 @@ extern "C" int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rt
     // (whatever goes wrong below, the results of an earlier call are no longer "the last segmentize!": rt_volumes must see that)
     ctx->segmented = false;
     ctx->vol_valid = false;
+    ctx->vol_fetched = false;
     if (!ctx->traced)
         return fail(ctx, RT_ERR_NOT_TRACED, "Segmentation is intended after tracing. Please, call `trace!` first!");
     if (k < 1 || max_iter < 0) return fail(ctx, RT_ERR_ARG, "rt_segmentize: bad k / max_iter");
@@ -1792,22 +1800,27 @@ extern "C" int rt_quadrature_device(rt_ctx *ctx, rt_quad_view *v, double *omega_
     return RT_OK;
 }
 
-extern "C" int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
-                                  double *tau_host) {
-    if (!ctx || n_groups < 1 || !sigma_t || (layout != 0 && layout != 1)) return fail(ctx, RT_ERR_ARG, "rt_optical_lengths: bad arguments");
-    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_optical_lengths: call rt_segmentize first");
+// tau of the resident batch from a table of n_rows x n_groups cross sections: one row per cell, or with `region` (the device
+// region map) one row per region
+static int optical_lengths(rt_ctx *ctx, const char *fn, int32_t n_groups, const double *sigma_t, long long n_rows, const int *region,
+                           int32_t layout, const double **d_tau, double *tau_host) {
+    if (!ctx || n_groups < 1 || !sigma_t || (layout != 0 && layout != 1)) return fail(ctx, RT_ERR_ARG, "%s: bad arguments", fn);
+    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "%s: call rt_segmentize first", fn);
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const long long n_seg = ctx->res_nseg;
-    const size_t n_sig = (size_t)ctx->m.n_cells * (size_t)n_groups, n_tau = (size_t)std::max<long long>(n_seg, 1) * (size_t)n_groups;
+    const size_t n_sig = (size_t)n_rows * (size_t)n_groups, n_tau = (size_t)std::max<long long>(n_seg, 1) * (size_t)n_groups;
     CK(ensure(ctx->b_sigma, sizeof(double) * n_sig));
     CK(ensure(ctx->b_tau, sizeof(double) * n_tau));
     CK(cudaMemcpyAsync(ctx->b_sigma.p, sigma_t, sizeof(double) * n_sig, cudaMemcpyHostToDevice, st));
     CK(cudaEventRecord(ctx->ev2[0], st));
     if (n_seg > 0) {
         const SegColumns c = seg_columns(ctx);
-        k_tau<<<blocks_for(n_seg * n_groups, 256), 256, 0, st>>>(n_seg, n_groups, c.len, c.elem, (const double *)ctx->b_sigma.p, layout,
-                                                               (double *)ctx->b_tau.p);
+        const unsigned blocks = blocks_for(n_seg * n_groups, 256);
+        if (region)
+            k_tau<true><<<blocks, 256, 0, st>>>(n_seg, n_groups, c.len, c.elem, (const double *)ctx->b_sigma.p, layout, (double *)ctx->b_tau.p, region);
+        else
+            k_tau<false><<<blocks, 256, 0, st>>>(n_seg, n_groups, c.len, c.elem, (const double *)ctx->b_sigma.p, layout, (double *)ctx->b_tau.p, nullptr);
     }
     CK(cudaEventRecord(ctx->ev2[1], st));
     CK(cudaGetLastError());
@@ -1818,6 +1831,74 @@ extern "C" int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *s
     cudaEventElapsedTime(&ms, ctx->ev2[0], ctx->ev2[1]);
     ctx->tau_ms = ms;
     if (d_tau) *d_tau = (const double *)ctx->b_tau.p;
+    return RT_OK;
+}
+
+extern "C" int rt_optical_lengths(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
+                                  double *tau_host) {
+    return optical_lengths(ctx, "rt_optical_lengths", n_groups, sigma_t, ctx ? ctx->m.n_cells : 0, nullptr, layout, d_tau, tau_host);
+}
+
+extern "C" int rt_optical_lengths_by_region(rt_ctx *ctx, int32_t n_groups, const double *sigma_t, int32_t layout, const double **d_tau,
+                                            double *tau_host) {
+    if (ctx && ctx->n_regions < 1)
+        return fail(ctx, RT_ERR_ARG, "rt_optical_lengths_by_region: no region map for the current mesh (call rt_set_regions after rt_mesh_upload)");
+    return optical_lengths(ctx, "rt_optical_lengths_by_region", n_groups, sigma_t, ctx ? ctx->n_regions : 0,
+                           (const int *)(ctx ? ctx->b_region.p : nullptr), layout, d_tau, tau_host);
+}
+
+// ------------------------------------------------------------------------------------------------------
+// region map: which material every cell belongs to (a transport code's cross sections are per material, not per cell)
+// ------------------------------------------------------------------------------------------------------
+extern "C" int rt_set_regions(rt_ctx *ctx, int32_t n_regions, const int32_t *cell_region) {
+    if (!ctx) return RT_ERR_ARG;
+    if (!ctx->has_mesh) return fail(ctx, RT_ERR_ARG, "rt_set_regions: upload a mesh first");
+    if (!cell_region) {
+        ctx->n_regions = 0;
+        return RT_OK;
+    }
+    if (n_regions < 1) return fail(ctx, RT_ERR_ARG, "rt_set_regions: n_regions = %d (at least 1)", (int)n_regions);
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int nc = ctx->m.n_cells;
+    // the new map is staged and checked on the side: a rejected map leaves the previous one in place
+    struct Scratch {
+        DevBuf map, keys, cells, tmp;
+        ~Scratch() { for (DevBuf *b : {&map, &keys, &cells, &tmp}) release(*b); }
+    } sc;
+    DevBuf &map = sc.map, &keys = sc.keys, &cells = sc.cells, &tmp = sc.tmp;
+    CK(ensure(map, sizeof(int) * (size_t)nc));
+    CK(ensure(keys, sizeof(int) * 2 * (size_t)nc + sizeof(int)));
+    CK(ensure(cells, sizeof(int) * 2 * (size_t)nc));
+    int *key = (int *)keys.p, *cell = (int *)cells.p, *d_bad = key + 2 * (size_t)nc;
+    CK(cudaMemcpyAsync(map.p, cell_region, sizeof(int) * (size_t)nc, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_bad, &nc, sizeof(int), cudaMemcpyHostToDevice, st));
+    k_region_check<<<blocks_for(nc, 256), 256, 0, st>>>(nc, n_regions, (const int *)map.p, d_bad, key, cell);
+    CK(cudaGetLastError());
+    int bad = nc;
+    CK(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (bad < nc)
+        return fail(ctx, RT_ERR_ARG, "rt_set_regions: cell %d has region %d, outside [1, n_regions = %d]", bad + 1, (int)cell_region[bad],
+                    (int)n_regions);
+    // region -> cells: a stable radix sort of the cell ids by region, then the run of every region (exact_vol.cuh k_exact_runs)
+    int bits = 1;
+    while (bits < 31 && (1LL << bits) < (long long)n_regions) ++bits;
+    cub::DoubleBuffer<int> dk(key, key + nc), dc(cell, cell + nc);
+    size_t tmp_b = 0;
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_b, dk, dc, nc, 0, bits, st));
+    CK(ensure(tmp, tmp_b));
+    CK(cub::DeviceRadixSort::SortPairs(tmp.p, tmp_b, dk, dc, nc, 0, bits, st));
+    CK(ensure(ctx->b_reg_order, sizeof(int) * (size_t)nc));
+    CK(ensure(ctx->b_reg_runs, sizeof(long long) * 2 * (size_t)n_regions));
+    long long *start = (long long *)ctx->b_reg_runs.p;
+    CK(cudaMemsetAsync(start, 0, sizeof(long long) * 2 * (size_t)n_regions, st));
+    k_exact_runs<<<blocks_for(nc, kExactThreads), kExactThreads, 0, st>>>(dk.Current(), nc, n_regions, start, start + n_regions);
+    CK(cudaMemcpyAsync(ctx->b_reg_order.p, dc.Current(), sizeof(int) * (size_t)nc, cudaMemcpyDeviceToDevice, st));
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    std::swap(ctx->b_region, map);  // (the previous map is released with the scratch)
+    ctx->n_regions = n_regions;
     return RT_OK;
 }
 
@@ -1869,6 +1950,39 @@ extern "C" int rt_correct_volumes(rt_ctx *ctx, double *factors, const double **d
     if (factors) CK(cudaMemcpyAsync(factors, ctx->b_factor.p, sizeof(double) * (size_t)nc, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (d_factors) *d_factors = (const double *)ctx->b_factor.p;
+    return RT_OK;
+}
+
+// Per-region sums of the traced volumes and of the element areas: the cells of every region in ascending id, one plain `+` each
+// from 0.0 (the gather puts the values in region order, k_exact_fold continues one running sum through each region's run)
+extern "C" int rt_region_volumes(rt_ctx *ctx, double *traced, double *exact) {
+    if (!ctx) return RT_ERR_ARG;
+    if (ctx->in_batch_cb) return fail(ctx, RT_ERR_ARG, "rt_region_volumes: not inside a batch callback (the volumes of the running rt_segmentize are not complete)");
+    if (ctx->n_regions < 1) return fail(ctx, RT_ERR_ARG, "rt_region_volumes: no region map for the current mesh (call rt_set_regions after rt_mesh_upload)");
+    if (traced && !(ctx->segmented && ctx->vol_valid && ctx->vol_fetched && ctx->b_voln.p))
+        return fail(ctx, RT_ERR_ARG, "rt_region_volumes: run rt_segmentize with volumes enabled and rt_volumes first");
+    CK(cudaSetDevice(ctx->device));
+    if (exact) {
+        int rc = ensure_areas(ctx);
+        if (rc) return rc;
+    }
+    cudaStream_t st = ctx->stream;
+    const int nc = ctx->m.n_cells, nr = ctx->n_regions;
+    CK(ensure(ctx->b_reg_val, sizeof(double) * ((size_t)nc + 2 * (size_t)nr)));
+    double *val = (double *)ctx->b_reg_val.p, *acc = val + nc;
+    const long long *start = (const long long *)ctx->b_reg_runs.p, *end = start + nr;
+    if (traced && ctx->voln_ready >= 0) CK(cudaStreamWaitEvent(st, ctx->ev_vol_free[ctx->voln_ready], 0));  // the all-reduced volumes
+    CK(cudaMemsetAsync(acc, 0, sizeof(double) * 2 * (size_t)nr, st));
+    const double *src[2] = {traced ? (const double *)ctx->b_voln.p : nullptr, exact ? (const double *)ctx->b_area.p : nullptr};
+    double *out[2] = {traced, exact};
+    for (int q = 0; q < 2; ++q) {
+        if (!src[q]) continue;
+        k_region_gather<<<blocks_for(nc, 256), 256, 0, st>>>(nc, (const int *)ctx->b_reg_order.p, src[q], val);
+        k_exact_fold<<<blocks_for(nr, kExactThreads), kExactThreads, 0, st>>>(nr, start, end, val, acc + q * nr);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(out[q], acc + q * nr, sizeof(double) * (size_t)nr, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
     return RT_OK;
 }
 
@@ -2048,7 +2162,11 @@ extern "C" int rt_volumes(rt_ctx *ctx, double *volumes) {
     cudaStream_t st = ctx->stream;
     int nc = ctx->m.n_cells;
     CK(ensure(ctx->b_voln, sizeof(double) * ((size_t)nc + 1)));
-    if (coll && ctx->exact) return exact_chain(ctx, have, volumes);
+    if (coll && ctx->exact) {
+        const int rc = exact_chain(ctx, have, volumes);
+        ctx->vol_fetched = rc == RT_OK;
+        return rc;
+    }
     const double *src = ctx->vol_acc ? ctx->vol_acc : (const double *)ctx->b_vol.p;
     if (!have) {
         // This rank's rt_segmentize failed, but its peers are (or will be) inside the all-reduce: join it with a zero contribution
@@ -2102,6 +2220,7 @@ extern "C" int rt_volumes(rt_ctx *ctx, double *volumes) {
                 return fail(ctx, RT_ERR_PEER, "rt_volumes: rt_segmentize failed on %d rank(s) of the communicator: the volumes miss their tracks", (int)failed);
         }
     }
+    ctx->vol_fetched = true;
     return RT_OK;
 }
 

@@ -26,9 +26,15 @@ __global__ void k_weights(int n2, const double *phi, double *omega) {
 }
 
 // segment-major (layout 0: tau[s*G + g], the concatenation of the reference's per-segment vectors) or group-major
-// (layout 1: tau[g*S + s], unit-stride over segments for a sweep that runs one group at a time)
+// (layout 1: tau[g*S + s], unit-stride over segments for a sweep that runs one group at a time).
+// BY_REGION: sigma_t is the small n_regions x n_groups table of a transport code's materials, indexed through the region map
+// (rt_set_regions, 1-based); it stays in L1 / L2 where the per-cell table is one random HBM row per segment.  The product is the
+// same IEEE multiplication, so tau is bit-equal to the per-cell call with the table expanded cell by cell.  (`region` comes last:
+// the parameter offsets, and so the code, of the per-cell instantiation are those of the kernel before the switch.)
+template <bool BY_REGION>
 __global__ void k_tau(long long n_seg, int n_groups, const double *__restrict__ len, const int *__restrict__ element,
-                      const double *__restrict__ sigma_t /* n_cells x n_groups */, int layout, double *__restrict__ tau) {
+                      const double *__restrict__ sigma_t /* n_cells (n_regions) x n_groups */, int layout, double *__restrict__ tau,
+                      const int *__restrict__ region) {
     const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (i >= n_seg * n_groups) return;
     long long s;
@@ -40,8 +46,29 @@ __global__ void k_tau(long long n_seg, int n_groups, const double *__restrict__ 
         g = (int)(i / n_seg);
         s = i - (long long)g * n_seg;
     }
-    const int e = element[s] - 1;
+    int e = element[s] - 1;
+    if constexpr (BY_REGION) e = region[e] - 1;
     tau[i] = sigma_t[(long long)e * n_groups + g] * len[s];
+}
+
+// ---- region map (rt_set_regions, rt_region_volumes) -----------------------------------------------------------------------
+// One pass over the map: the first cell whose region is outside [1, n_regions] (atomicMin on its index; *first_bad starts at
+// n_cells), and the (region - 1, cell) pairs whose stable sort by region gives the region -> cells order.
+__global__ void k_region_check(int n_cells, int n_regions, const int *__restrict__ region, int *__restrict__ first_bad,
+                               int *__restrict__ key, int *__restrict__ cell) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n_cells) return;
+    const int r = region[c];
+    if (r < 1 || r > n_regions) atomicMin(first_bad, c);
+    key[c] = r - 1;
+    cell[c] = c;
+}
+
+// per-cell values in region order (order: the cell ids sorted stably by region), for k_exact_runs / k_exact_fold
+__global__ void k_region_gather(int n_cells, const int *__restrict__ order, const double *__restrict__ v, double *__restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_cells) return;
+    out[i] = v[order[i]];
 }
 
 // element_volume(mesh, node_ids) = 1/2 * abs((x2 - x1) x (x3 - x1))  (src/trackgenerator.jl:402-411): the exact cell areas the

@@ -65,6 +65,30 @@ class UnstructuredDiscreteModel:
     def has_quads(self) -> bool:
         return bool(np.any(self.cell_sizes == 4))
 
+    def cell_regions(self, names) -> np.ndarray:
+        """The region (material) of every cell as int32 values in [1, len(names)]: the 1-based position in ``names`` of the first
+        name whose tag contains the cell's entity (``labels``: Gridap's face labeling ``names`` / ``tags`` / ``entities_2``, or
+        the physical groups of a .msh file).  Overlapping tags go to the name listed first.  An unknown name, or a cell in none of
+        the named tags, raises ValueError.  What ``TrackGenerator.set_regions`` takes."""
+        lab = self.labels or {}
+        known, tags, ent = list(lab.get("names") or []), lab.get("tags"), lab.get("entities_2")
+        if ent is None or tags is None:
+            raise ValueError("the model carries no cell labeling (names / tags / entities_2)")
+        ent = np.asarray(ent, dtype=np.int64).reshape(-1)
+        if ent.shape[0] != self.num_cells:
+            raise ValueError(f"the labeling has {ent.shape[0]} cell entities for {self.num_cells} cells")
+        region = np.zeros(self.num_cells, dtype=np.int32)
+        for r, name in enumerate(names, start=1):
+            if name not in known:
+                raise ValueError(f"unknown label {name!r}: the model has {known}")
+            hit = (region == 0) & np.isin(ent, np.asarray(tags[known.index(name)], dtype=np.int64))
+            region[hit] = r
+        missing = np.flatnonzero(region == 0)
+        if missing.size:
+            raise ValueError(f"{missing.size} cells are in none of the tags {list(names)}; the first is cell {missing[0] + 1} "
+                             f"(entity {ent[missing[0]]})")
+        return region
+
     def triangles0(self) -> np.ndarray:
         """0-based (n_cells, 3) view of the cell table (triangles only)."""
         if self.has_quads:
@@ -91,7 +115,9 @@ def DiscreteModelFromFile(path: str) -> UnstructuredDiscreteModel:
 def GmshDiscreteModel(path: str, renumber: bool = True) -> UnstructuredDiscreteModel:
     """Reader for MSH 4.1 ASCII (``demo/pincell.msh``; reference README quick start). Keeps the 3-node
     triangles (element type 2), nodes in tag order, node ids ascending within each cell like the
-    Gridap model the reference builds from the same file."""
+    Gridap model the reference builds from the same file.  The physical groups become ``labels`` as Gridap names them: one
+    name per ``$PhysicalNames`` entry, its tag the surface entities of ``$Entities`` that carry the group, and ``entities_2`` the
+    surface entity of every triangle (cells stay in file order, whatever the node renumbering): see ``cell_regions``."""
     with open(path) as fh:
         lines = fh.read().split("\n")
     idx = {ln.strip(): i for i, ln in enumerate(lines) if ln.startswith("$")}
@@ -120,14 +146,18 @@ def GmshDiscreteModel(path: str, renumber: bool = True) -> UnstructuredDiscreteM
     i = idx["$Elements"] + 1
     nblocks = int(lines[i].split()[0])
     i += 1
-    tris = []
+    tris, tri_ent = [], []
     for _ in range(nblocks):
-        _, _, etype, nb = (int(v) for v in lines[i].split())
+        _, etag, etype, nb = (int(v) for v in lines[i].split())
         i += 1
         if etype == 2:
             for j in range(nb):
                 tris.append([int(v) for v in lines[i + j].split()[1:4]])
+            tri_ent += [etag] * nb
         i += nb
+    labels = _msh_labels(lines, idx)
+    if labels:
+        labels["entities_2"] = tri_ent
     tri_tags = np.asarray(tris, dtype=np.int64)
     tri0 = np.searchsorted(tags, tri_tags)
     if renumber:  # keep only nodes referenced by triangles, in tag order
@@ -136,7 +166,35 @@ def GmshDiscreteModel(path: str, renumber: bool = True) -> UnstructuredDiscreteM
         remap[used] = np.arange(used.size)
         tri0 = remap[tri0]
         xyz = xyz[used]
-    return UnstructuredDiscreteModel.from_triangles(xyz[:, :2], tri0, sort_nodes=True)
+    return UnstructuredDiscreteModel.from_triangles(xyz[:, :2], tri0, sort_nodes=True, labels=labels)
+
+
+def _msh_labels(lines, idx) -> dict:
+    """{names, tags} of the physical groups of an MSH 4.1 file: ``$PhysicalNames`` (dim tag "name") and, from ``$Entities``, the
+    surfaces that carry each group (a group of points or curves tags no surface).  Empty without ``$PhysicalNames``."""
+    if "$PhysicalNames" not in idx or "$Entities" not in idx:
+        return {}
+    i = idx["$PhysicalNames"] + 1
+    groups = []  # (dim, physical tag, name) in file order
+    for ln in lines[i + 1:i + 1 + int(lines[i].split()[0])]:
+        dim, tag, name = ln.split(maxsplit=2)
+        groups.append((int(dim), int(tag), name.strip().strip('"')))
+    i = idx["$Entities"] + 1
+    n_pts, n_crv, n_srf = (int(v) for v in lines[i].split()[:3])
+    surfaces = {}  # physical tag -> surface entity tags
+    # points: tag x y z nPhys phys... ; curves and surfaces: tag minX minY minZ maxX maxY maxZ nPhys phys... nBound bound...
+    for ln in lines[i + 1 + n_pts + n_crv:i + 1 + n_pts + n_crv + n_srf]:
+        v = ln.split()
+        for ph in v[8:8 + int(v[7])]:
+            surfaces.setdefault(int(ph), []).append(int(v[0]))
+    names, tags = [], []
+    for dim, tag, name in groups:
+        if name in names:  # (a name given to groups of several dimensions: one label)
+            tags[names.index(name)] += surfaces.get(tag, []) if dim == 2 else []
+            continue
+        names.append(name)
+        tags.append(list(surfaces.get(tag, [])) if dim == 2 else [])
+    return {"names": names, "tags": tags}
 
 
 def vertex_to_cells(n_nodes: int, cell_ptrs: np.ndarray, cell_data: np.ndarray):
