@@ -118,7 +118,9 @@ int rt_mesh_neighbours(rt_ctx *ctx, int32_t *cell_nbr /* 3*n_cells */);
  * phi = tg.azimuthal_quadrature.phis, sin/cos/tan of it, dx_eff/dy_eff = the local dx/dy of trace!.
  * bcs = top,bottom,right,left.  Only uids in [uid_begin, uid_end) (1-based, end exclusive) are generated
  * on this context: that is the multi-GPU shard.  n_tracks_x/y are the constructor's counts
- * (src/trackgenerator.jl:96-108). */
+ * (src/trackgenerator.jl:96-108).  A call that gets past its null-table and boundary-code checks first drops the previous trace
+ * and segments (rt_segment_offsets, the resident batch, the volumes rt_correct_volumes and rt_region_volumes use): if it then
+ * fails, the context is untraced and the delta_eff uploaded by rt_segmentize is dropped with it (rt_quadrature_device). */
 int rt_trace(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x, const int64_t *n_tracks_y,
              const double *phi, const double *sin_phi, const double *cos_phi, const double *tan_phi,
              const double *dx_eff, const double *dy_eff, const int32_t bcs[4], int64_t uid_begin,
@@ -129,7 +131,8 @@ int rt_tracks_download(rt_ctx *ctx, int64_t *azim_idx, int64_t *track_idx, doubl
                        double *len, double *abc, int8_t *bc_fwd, int8_t *bc_bwd, int8_t *dir_fwd,
                        int8_t *dir_bwd, int64_t *next_fwd_uid, int64_t *next_bwd_uid);
 /* Split [1, n_total] into n_parts contiguous uid ranges of equal total track length (bounds has
- * n_parts+1 entries, bounds[0]=1, bounds[n_parts]=n_total+1). Same tables as rt_trace. */
+ * n_parts+1 entries, bounds[0]=1, bounds[n_parts]=n_total+1). Same tables as rt_trace.  A query: it needs an uploaded mesh
+ * only, and leaves the context's trace, segments, volumes and per-angle tables as they were. */
 int rt_plan_shards(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x, const int64_t *n_tracks_y,
                    const double *phi, const double *tan_phi, const double *dx_eff, const double *dy_eff,
                    int32_t n_parts, int64_t *bounds);
@@ -159,6 +162,8 @@ typedef struct rt_batch {
 } rt_batch;
 typedef int (*rt_batch_cb)(const rt_batch *batch, void *user);
 
+/* 0: as many segments as fit in device memory.  A track is never split across batches: a capacity below the segments of one track
+ * makes rt_segmentize fail with RT_ERR_NOMEM. */
 int rt_set_segment_capacity(rt_ctx *ctx, int64_t max_segments_resident);
 int rt_segmentize(rt_ctx *ctx, double tiny_step, int32_t k, double rtol, int32_t max_iter,
                   const double *delta_eff, uint32_t flags, rt_batch_cb cb, void *cb_user,
@@ -181,7 +186,8 @@ int rt_segments_download(rt_ctx *ctx, double *px, double *py, double *qx, double
 int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy, double *len, int32_t *element, int64_t max_exceptions,
                                  int64_t *exc_index, double *exc_px, double *exc_py, int64_t *n_exceptions);
 /* device-resident view of the resident batch for on-GPU consumers (transport sweeps); d_px .. d_qy are NULL after
- * RT_SEG_LENGTHS_ONLY */
+ * RT_SEG_LENGTHS_ONLY.  Needs a resident batch, like the downloads: a completed rt_segmentize that no rt_trace, rt_mesh_upload or
+ * failed rt_segmentize has followed, or the batch callback of the running one (RT_ERR_ARG otherwise, *view untouched). */
 int rt_segments_device(rt_ctx *ctx, rt_batch *view);
 
 /* ---- what a transport sweep consumes besides the Segment records, kept on the device (SURVEY.md 8f-1) -------------
@@ -199,9 +205,10 @@ typedef struct rt_track_view {
 } rt_track_view;
 int rt_tracks_device(rt_ctx *ctx, rt_track_view *view);
 
-/* Per-angle tables on the device: phi, sin, cos (as passed to rt_trace), delta_eff (as passed to rt_segmentize, NULL before),
- * and the azimuthal weights omega of init_weights! (src/azimuthal_quad.jl:35-53), computed on the device from phi with the
- * reference's formula; omega_host (n_azim_2 doubles) receives a copy when not NULL. */
+/* Per-angle tables on the device: phi, sin, cos (as passed to rt_trace), delta_eff (as passed to rt_segmentize; NULL after every
+ * rt_trace until an rt_segmentize with volumes uploads it), and the azimuthal weights omega of init_weights!
+ * (src/azimuthal_quad.jl:35-53), computed on the device from phi with the reference's formula; omega_host (n_azim_2 doubles)
+ * receives a copy when not NULL.  Needs a traced context: RT_ERR_NOT_TRACED after rt_mesh_upload or a failed rt_trace. */
 typedef struct rt_quad_view {
     int32_t n_azim_2;
     const double *d_phi, *d_sin, *d_cos, *d_delta_eff, *d_omega;
@@ -324,9 +331,9 @@ int rt_selftest_division(rt_ctx *ctx, int64_t n_threads, uint64_t seed, int32_t 
  * "pipeline" (3: ONE sign-test walk that counts and records every chunk + one lane per segment [default]; 0: sign-test count
  * walk + geometric fill walk; 1: sequential geometric walks only.  0 and 3 verify themselves and restart in mode 1 on any
  * disagreement; 3 restarts in mode 0 when its record
- * pool runs out), "band_chunks" (0: uniform chunks also where a track
+ * pool runs out, also when one block of 32 tracks has more chunk slots than a walk batch may take), "band_chunks" (0: uniform chunks also where a track
  * runs along the bounding box), "band_min" / "band_div" (a head or tail of a track that stays inside the boundary band for more
- * than band_min regular chunk lengths [0.0625] is cut into chunks band_div times shorter than the regular ones [8]), "pool_slots" / "pool_extra" (test hooks: chunk slots per count batch, spare record blocks),
+ * than band_min regular chunk lengths [0.0625] is cut into chunks band_div times shorter than the regular ones [8]), "pool_slots" / "pool_extra" (test hooks: chunk slots per count batch -- fewer than one 32-track block needs make pipeline 3 restart in mode 0 --, spare record blocks),
  * "debug_verify_fail", "debug_clear_pool" (test hooks), "plan_cache" (0: rebuild the chunk plan in every call), "optimistic" (0: always read
  * the segment total back before the evaluation is launched) */
 int rt_set_option(rt_ctx *ctx, const char *name, double value);

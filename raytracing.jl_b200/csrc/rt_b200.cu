@@ -250,6 +250,14 @@ static void release(DevBuf &b) {
     b.bytes = 0;
 }
 
+// a buffer of one call, released on every return path
+struct ScopedBuf : DevBuf {
+    ScopedBuf() = default;
+    ScopedBuf(const ScopedBuf &) = delete;
+    ScopedBuf &operator=(const ScopedBuf &) = delete;
+    ~ScopedBuf() { release(*this); }
+};
+
 static inline unsigned blocks_for(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
 template <typename Tin, typename Tout>
@@ -576,38 +584,53 @@ extern "C" int rt_mesh_neighbours(rt_ctx *ctx, int32_t *cell_nbr) {
 // ------------------------------------------------------------------------------------------------------
 // trace!
 // ------------------------------------------------------------------------------------------------------
-static int upload_angle_tables(rt_ctx *ctx, int32_t n2, const int64_t *nx, const int64_t *ny, const double *phi,
-                               const double *sin_phi, const double *cos_phi, const double *tan_phi, const double *dxe,
-                               const double *dye) {
+// The per-angle tables on the host: doubles phi, sin, cos, tan, dxe, dye, delta (7 x n2; a NULL column and delta stay zero) and
+// int64 nx, ny, base (3 x n2 + 1; base = the uid offset of every angle)
+static int angle_tables(rt_ctx *ctx, int32_t n2, const int64_t *nx, const int64_t *ny, const double *phi, const double *sin_phi,
+                        const double *cos_phi, const double *tan_phi, const double *dxe, const double *dye, std::vector<double> &hd,
+                        std::vector<long long> &hi) {
     if (n2 < 2 || (n2 % 2) != 0) return fail(ctx, RT_ERR_ARG, "n_azim_2 must be a positive even number");
-    std::vector<double> hd(7 * (size_t)n2, 0.0);
+    hd.assign(7 * (size_t)n2, 0.0);
     const double *cols[6] = {phi, sin_phi, cos_phi, tan_phi, dxe, dye};
     for (int q = 0; q < 6; ++q)
         if (cols[q]) memcpy(&hd[(size_t)q * n2], cols[q], sizeof(double) * n2);
-    std::vector<long long> hi(3 * (size_t)n2 + 1, 0);
-    ctx->h_base.assign((size_t)n2 + 1, 0);
+    hi.assign(3 * (size_t)n2 + 1, 0);
+    long long *base = &hi[2 * (size_t)n2];
     for (int i = 0; i < n2; ++i) {
         if (nx[i] < 1 || ny[i] < 1) return fail(ctx, RT_ERR_ARG, "n_tracks_x/y must be >= 1");
         hi[i] = nx[i];
         hi[n2 + i] = ny[i];
-        ctx->h_base[i + 1] = ctx->h_base[i] + nx[i] + ny[i];
+        base[i + 1] = base[i] + nx[i] + ny[i];
     }
-    for (int i = 0; i <= n2; ++i) hi[2 * (size_t)n2 + i] = ctx->h_base[i];
-    CK(ensure(ctx->b_ang_d, sizeof(double) * hd.size()));
-    CK(ensure(ctx->b_ang_i, sizeof(long long) * hi.size()));
-    CK(cudaMemcpyAsync(ctx->b_ang_d.p, hd.data(), sizeof(double) * hd.size(), cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->b_ang_i.p, hi.data(), sizeof(long long) * hi.size(), cudaMemcpyHostToDevice, ctx->stream));
+    return RT_OK;
+}
+
+static int upload_tables(rt_ctx *ctx, const std::vector<double> &hd, const std::vector<long long> &hi, DevBuf &bd, DevBuf &bi) {
+    CK(ensure(bd, sizeof(double) * hd.size()));
+    CK(ensure(bi, sizeof(long long) * hi.size()));
+    CK(cudaMemcpyAsync(bd.p, hd.data(), sizeof(double) * hd.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(bi.p, hi.data(), sizeof(long long) * hi.size(), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+// the tables of rt_trace become the context's: what rt_quadrature_device hands out and what rt_segmentize reads
+static int upload_angle_tables(rt_ctx *ctx, int32_t n2, const int64_t *nx, const int64_t *ny, const double *phi,
+                               const double *sin_phi, const double *cos_phi, const double *tan_phi, const double *dxe,
+                               const double *dye) {
+    std::vector<double> hd;
+    std::vector<long long> hi;
+    int rc = angle_tables(ctx, n2, nx, ny, phi, sin_phi, cos_phi, tan_phi, dxe, dye, hd, hi);
+    if (rc) return rc;
+    if ((rc = upload_tables(ctx, hd, hi, ctx->b_ang_d, ctx->b_ang_i))) return rc;
+    ctx->h_base.assign(hi.begin() + 2 * (size_t)n2, hi.end());
     ctx->n2 = n2;
     ctx->h_phi.assign(phi, phi + n2);
     ctx->has_delta = false;
     return RT_OK;
 }
 
-static void fill_trace_params(rt_ctx *ctx, TraceParams &P, const int32_t bcs[4]) {
-    int n2 = ctx->n2;
-    const double *d = (const double *)ctx->b_ang_d.p;
-    const long long *li = (const long long *)ctx->b_ang_i.p;
+static void fill_trace_params(const rt_ctx *ctx, TraceParams &P, const int32_t bcs[4], int n2, const double *d, const long long *li) {
     P.n2 = n2;
     P.n4 = n2 / 2;
     P.nx = li;
@@ -636,6 +659,10 @@ extern "C" int rt_trace(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x
     for (int q = 0; q < 4; ++q)
         if (bcs[q] < 0 || bcs[q] > 2) return fail(ctx, RT_ERR_ARG, "rt_trace: bad boundary condition code");
     CK(cudaSetDevice(ctx->device));
+    // (from here on the previous trace is gone, also when this call fails: its tracks no longer match the angle tables)
+    ctx->traced = false;
+    ctx->segmented = false;
+    ctx->has_delta = false;
     int rc = upload_angle_tables(ctx, n_azim_2, n_tracks_x, n_tracks_y, phi, sin_phi, cos_phi, tan_phi, dx_eff, dy_eff);
     if (rc) return rc;
     long long n_total = ctx->h_base[n_azim_2];
@@ -645,8 +672,6 @@ extern "C" int rt_trace(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x
     long long n = uid_end - uid_begin;
     ctx->uid_begin = uid_begin;
     ctx->n_shard = n;
-    ctx->traced = false;
-    ctx->segmented = false;
     size_t nn = (size_t)std::max<long long>(n, 1);
     CK(ensure(ctx->b_trk_d, sizeof(double) * 8 * nn));
     CK(ensure(ctx->b_trk_i, sizeof(int) * nn));
@@ -675,7 +700,7 @@ extern "C" int rt_trace(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tracks_x
     t.dir_bwd = c + 3 * nn;
     CK(cudaMemsetAsync(ctx->b_err.p, 0xff, sizeof(unsigned long long), ctx->stream));
     TraceParams P;
-    fill_trace_params(ctx, P, bcs);
+    fill_trace_params(ctx, P, bcs, ctx->n2, (const double *)ctx->b_ang_d.p, (const long long *)ctx->b_ang_i.p);
     P.uid_begin = uid_begin;
     P.n = n;
     P.t = t;
@@ -793,18 +818,20 @@ extern "C" int rt_plan_shards(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tr
     if (!ctx || !ctx->has_mesh) return fail(ctx, RT_ERR_ARG, "rt_plan_shards: upload a mesh first");
     if (n_parts < 1 || !bounds || !phi || !tan_phi || !dx_eff || !dy_eff) return fail(ctx, RT_ERR_ARG, "rt_plan_shards: bad arguments");
     CK(cudaSetDevice(ctx->device));
-    int rc = upload_angle_tables(ctx, n_azim_2, n_tracks_x, n_tracks_y, phi, nullptr, nullptr, tan_phi, dx_eff, dy_eff);
+    // (a query: the tables go to buffers of this call, so that the context's trace, segments and quadrature stay as they were)
+    std::vector<double> hd;
+    std::vector<long long> hi;
+    int rc = angle_tables(ctx, n_azim_2, n_tracks_x, n_tracks_y, phi, nullptr, nullptr, tan_phi, dx_eff, dy_eff, hd, hi);
     if (rc) return rc;
-    ctx->traced = false;
-    ctx->segmented = false;
-    long long n = ctx->h_base[n_azim_2];
-    DevBuf lens, cum, db;
+    const long long n = hi.back();
+    ScopedBuf ad, ai, lens, cum, db;
+    if ((rc = upload_tables(ctx, hd, hi, ad, ai))) return rc;
     CK(ensure(lens, sizeof(double) * (size_t)n));
     CK(ensure(cum, sizeof(double) * ((size_t)n + 1)));
     CK(ensure(db, sizeof(long long) * ((size_t)n_parts + 1)));
     CK(ensure(ctx->b_err, sizeof(unsigned long long)));
     TraceParams P;
-    fill_trace_params(ctx, P, nullptr);
+    fill_trace_params(ctx, P, nullptr, n_azim_2, (const double *)ad.p, (const long long *)ai.p);
     P.uid_begin = 1;
     P.n = n;
     P.t = TrackSoA{};
@@ -819,9 +846,6 @@ extern "C" int rt_plan_shards(rt_ctx *ctx, int32_t n_azim_2, const int64_t *n_tr
     CK(cudaStreamSynchronize(ctx->stream));
     for (int r = 0; r <= n_parts; ++r) bounds[r] = hb[r];
     for (int r = 1; r <= n_parts; ++r) bounds[r] = std::max(bounds[r], bounds[r - 1]);
-    release(lens);
-    release(cum);
-    release(db);
     return RT_OK;
 }
 
@@ -990,12 +1014,13 @@ static double *fused_vol(const rt_ctx *ctx, const Attempt &a) { return a.want_vo
 // the resident batch may be read: after a completed rt_segmentize, or from inside its batch callback
 static bool resident_valid(const rt_ctx *ctx) { return ctx && (ctx->segmented || ctx->in_batch_cb); }
 
+static void batch_view(const rt_ctx *ctx, rt_batch *view);
+
 // the resident batch (rt_segments_device) to the caller's batch callback, if there is one
 static int deliver_batch(rt_ctx *ctx, const Attempt &a) {
     if (!a.cb) return RT_OK;
     rt_batch bt;
-    int rc = rt_segments_device(ctx, &bt);
-    if (rc) return rc;
+    batch_view(ctx, &bt);
     bt.attempt = a.index;
     ctx->in_batch_cb = true;  // (the resident-batch calls accept the batch while the callback runs)
     const int stop = a.cb(&bt, a.cb_user);
@@ -1373,7 +1398,10 @@ static int segmentize_pipeline(rt_ctx *ctx, WalkParams &P, uint32_t flags, int m
         if (multi) {
             const long long lim = h_unit_base[(size_t)B0] + max_slots / 32;
             B1 = (long long)(std::upper_bound(h_unit_base.begin() + B0, h_unit_base.end(), lim) - h_unit_base.begin()) - 1;
-            if (B1 <= B0) return fail(ctx, RT_ERR_NOMEM, "rt_segmentize: one block of 32 tracks needs more than the record pool");
+            if (B1 <= B0) {  // this block alone has more chunk slots than a walk batch may take: the pool cannot hold its records
+                a.next = Next::Hybrid;
+                return RT_OK;
+            }
         }
         const long long b = 32 * B0, e = std::min(32 * B1, n);
         const long long u0 = multi ? h_unit_base[(size_t)B0] : 0, u1 = multi ? h_unit_base[(size_t)B1] : n_units;
@@ -1732,8 +1760,7 @@ extern "C" int rt_segments_download_compact(rt_ctx *ctx, double *qx, double *qy,
     return RT_OK;
 }
 
-extern "C" int rt_segments_device(rt_ctx *ctx, rt_batch *view) {
-    if (!ctx || !view) return RT_ERR_ARG;
+static void batch_view(const rt_ctx *ctx, rt_batch *view) {
     view->uid_begin = ctx->uid_begin + ctx->res_trk_begin;
     view->uid_end = ctx->uid_begin + ctx->res_trk_end;
     view->n_segments = ctx->res_nseg;
@@ -1748,6 +1775,13 @@ extern "C" int rt_segments_device(rt_ctx *ctx, rt_batch *view) {
     view->d_element = c.elem;
     view->stream = (void *)ctx->stream;
     view->attempt = 0;
+}
+
+extern "C" int rt_segments_device(rt_ctx *ctx, rt_batch *view) {
+    if (!ctx || !view) return RT_ERR_ARG;
+    // (rt_trace and rt_mesh_upload leave res_* as they were: a view of them would pair the new shard with old columns)
+    if (!resident_valid(ctx)) return fail(ctx, RT_ERR_ARG, "rt_segments_device: call rt_segmentize first");
+    batch_view(ctx, view);
     return RT_OK;
 }
 
@@ -1782,7 +1816,7 @@ extern "C" int rt_tracks_device(rt_ctx *ctx, rt_track_view *v) {
 
 extern "C" int rt_quadrature_device(rt_ctx *ctx, rt_quad_view *v, double *omega_host) {
     if (!ctx || !v) return RT_ERR_ARG;
-    if (ctx->n2 < 2) return fail(ctx, RT_ERR_NOT_TRACED, "rt_quadrature_device: call rt_trace first");
+    if (!ctx->traced) return fail(ctx, RT_ERR_NOT_TRACED, "rt_quadrature_device: call rt_trace first");
     CK(cudaSetDevice(ctx->device));
     const int n2 = ctx->n2;
     CK(ensure(ctx->b_omega, sizeof(double) * (size_t)n2));
